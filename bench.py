@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- ONMF samples/s (code + surrogate + dictionary update) on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload cfg5]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload cfg5] [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[4], the one the metric is quoted on): synthetic nonnegative data,
 d=1024 (32x32 patches), k=256 atoms, global minibatch 262,144 columns sharded by columns over the N GPUs
@@ -15,6 +15,10 @@ same steps fed from pinned HOST memory through OnmfEngine.step_host (H2D of ever
 updated dictionary inside the timed region).  `roofline` describes the dominant kernel (the LARS coder,
 timed live with CUDA events on its launch stream), `cpu_baseline` the reference CPU path (numpy + sklearn
 lasso_lars, the oracle port) on a bounded column sample on this box's host cores.
+
+--dump-outputs DIR writes what the last timed step returned (its codes) and left behind (W, A, B) as .npy files.
+The pool, W0 and the minibatch indices come from fixed seeds, so two builds run with the same arguments can be
+compared array by array.
 """
 from __future__ import annotations
 
@@ -59,6 +63,22 @@ def measured_peaks():
         except Exception:
             pass
     return 6650.0, "fallback (B200_PROFILING.md)"
+
+
+DUMP_CODE_ROWS = 16384       # code rows kept by --dump-outputs: 16 MB at k=256, about 18 MB with W, A and B
+
+
+def timed_outputs(eng, codes):
+    """What a caller of the timed path holds after its last step, as host arrays: that step's codes (this rank's
+    n x k; a fixed, seeded sample of DUMP_CODE_ROWS rows in ascending order when n is larger) and the dictionary and
+    aggregates the step left behind."""
+    import torch
+    W, A, B, _ = eng.state()
+    n = codes.shape[0]
+    if n > DUMP_CODE_ROWS:
+        rows = np.sort(np.random.default_rng(0).choice(n, DUMP_CODE_ROWS, replace=False))
+        codes = codes.index_select(0, torch.from_numpy(rows).to(codes.device))
+    return {name: x.cpu().numpy() for name, x in (("codes", codes), ("W", W), ("A", A), ("B", B))}
 
 
 class ClockSampler(threading.Thread):
@@ -261,7 +281,7 @@ def run_ours(args):
             idx.copy_(idx_all[t % n_seq])
         else:
             idx = idx_all[t % n_seq]
-        eng.step_pool(pool, idx, float(t))
+        return eng.step_pool(pool, idx, float(t))
 
     # The end-to-end loops below re-run the SAME steps as the device-timed loop (the coder's work per step depends on how far
     # the dictionary has come: +4 % per 13 steps at cfg5, profiles/r2_steps.md): the state two steps before the end of the
@@ -329,7 +349,7 @@ def run_ours(args):
     ev0.record(main)
     for _ in range(K):
         t += 1
-        one_step(t)
+        codes = one_step(t)
     eng.flush()
     ev1.record(main)
     barrier()
@@ -346,6 +366,8 @@ def run_ours(args):
             for lab, t0_, t1_ in rows[:80]:
                 sys.stderr.write("  %-10s %8.3f %8.3f\n" % (lab, t0_, t1_))
     clocks = sampler.stop()
+    # copied now: the passes below step the same engine again
+    outputs = timed_outputs(eng, codes) if (args.dump_outputs and rank == 0) else None
     elapsed_ms = ev0.elapsed_time(ev1)
     launches = eng.launches - launches0
     stats = eng.read_stats()
@@ -526,6 +548,10 @@ def run_ours(args):
                 "api": "OnmfEngine.step_host(pinned float32 Xt, t, W_out_host)", "u8_storage": e2e_u8},
         "roofline": roofline, "cpu_baseline": cpu,
     }
+    if outputs is not None:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in outputs.items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
     print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()
@@ -549,7 +575,14 @@ def main():
     ap.add_argument("--timeline", action="store_true", help="print device timestamps of the step's kernels (analysis only)")
     ap.add_argument("--graph", default="auto", choices=["auto", "on", "off"],
                     help="replay the fused step as a CUDA graph (auto: the small workloads cfg1..cfg4 on one GPU)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="write the last timed step's outputs to DIR/<name>.npy (float32): codes (rank 0's rows, at most "
+                         "%d of them, a fixed seeded sample), W, A, B" % DUMP_CODE_ROWS)
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.workload == "next"):
+        ap.error("--dump-outputs needs --impl ours and a cfgN workload")
     if args.workload == "next":
         import bench_next
         return bench_next.main((["--quick"] if args.quick else []) + (["--only", args.only] if args.only else []))

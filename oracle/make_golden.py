@@ -1,8 +1,8 @@
-"""Generate tests/golden/*.npz by running the UNMODIFIED reference in this container.
+"""Generate tests/golden/*.npz by running the UNMODIFIED reference.
 
-TEST INFRASTRUCTURE ONLY.  Run once in the authoring container (needs /root/reference):
+TEST INFRASTRUCTURE ONLY.  Needs a checkout of the reference, named by ONMF_REFERENCE_ROOT:
 
-    python oracle/make_golden.py
+    ONMF_REFERENCE_ROOT=<reference checkout> python oracle/make_golden.py
 
 Every fixture holds the inputs (X or the patch tensor, W0, the minibatch index sequence,
 alpha, history...) and the per-step outputs (H, A, B, W) of the reference's own

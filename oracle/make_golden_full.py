@@ -1,5 +1,6 @@
 """Full-length reference runs for the fp32 production-mode bars (final dictionary per atom <= 1e-3, reconstruction
-error within 0.5 %).  TEST INFRASTRUCTURE ONLY; needs /root/reference (authoring container).  Takes ~15 CPU-minutes.
+error within 0.5 %).  TEST INFRASTRUCTURE ONLY; needs a reference checkout named by ONMF_REFERENCE_ROOT.  Takes ~15
+CPU-minutes.
 
     python oracle/make_golden_full.py [cfg1 cfg2 cfg3 cfg4]
 

@@ -1,9 +1,9 @@
-"""Import the UNMODIFIED reference (HanbaekLyu/ONMF_ONTF_NDL) from /root/reference.
+"""Import the UNMODIFIED reference (HanbaekLyu/ONMF_ONTF_NDL) from a checkout named by ONMF_REFERENCE_ROOT.
 
-TEST INFRASTRUCTURE ONLY.  Works only inside the authoring container (the GPU box
-has no /root/reference).  Used by `oracle/make_golden.py` to generate the committed
-fixtures under `tests/golden/` and by `tests/test_oracle_vs_reference.py` (skipped
-when the reference tree is absent).
+TEST INFRASTRUCTURE ONLY.  The reference is not part of this repository; without
+ONMF_REFERENCE_ROOT nothing here can load it.  Used by `oracle/make_golden.py` to generate
+the committed fixtures under `tests/golden/` and by `tests/test_oracle_vs_reference.py`
+(skipped when no reference checkout is named).
 
 The reference imports three modules that are not installed here and that it never
 uses arithmetically on the hot path (SURVEY.md §8c):
@@ -20,11 +20,11 @@ import types
 
 import numpy as np
 
-REFERENCE_ROOT = os.environ.get("ONMF_REFERENCE_ROOT", "/root/reference")
+REFERENCE_ROOT = os.environ.get("ONMF_REFERENCE_ROOT", "")
 
 
 def reference_available() -> bool:
-    return os.path.isfile(os.path.join(REFERENCE_ROOT, "src", "ontf.py"))
+    return bool(REFERENCE_ROOT) and os.path.isfile(os.path.join(REFERENCE_ROOT, "src", "ontf.py"))
 
 
 def _stub(name, **attrs):
@@ -44,7 +44,7 @@ def _unfold(t, mode):
 def load_reference():
     """Returns (ref_onmf_module, ref_ontf_module)."""
     if not reference_available():
-        raise RuntimeError("reference tree not present at %s" % REFERENCE_ROOT)
+        raise RuntimeError("no reference checkout: set ONMF_REFERENCE_ROOT (now %r)" % REFERENCE_ROOT)
     try:
         import matplotlib.pyplot  # noqa: F401
     except Exception:

@@ -1,7 +1,9 @@
 """The committed fixtures against the LIVE reference: regenerate a few of them with the unmodified reference
-(/root/reference, imported through oracle/ref_loader.py) and require bit-equality with what is in tests/golden/.
+(a checkout named by ONMF_REFERENCE_ROOT, imported through oracle/ref_loader.py) and require bit-equality with what
+is in tests/golden/.
 
-Runs only where the reference tree exists (the authoring container); skipped on the GPU box.  CPU only.
+The reference is not part of this repository: without ONMF_REFERENCE_ROOT these tests skip, and the fixtures they
+guard are checked by tests/test_oracle.py and tests/test_gpu_parity.py.  CPU only.
 ONMF_SLOW=1 additionally regenerates the full-length cfg1 and cfg5 runs (~1 + ~2 CPU-minutes)."""
 import os
 import warnings
@@ -12,7 +14,7 @@ import pytest
 from oracle.ref_loader import reference_available
 
 warnings.filterwarnings("ignore")
-pytestmark = pytest.mark.skipif(not reference_available(), reason="reference tree not present (GPU box)")
+pytestmark = pytest.mark.skipif(not reference_available(), reason="no reference checkout (set ONMF_REFERENCE_ROOT)")
 
 # scalars computed through BLAS reductions may differ in the last bit with the thread count
 LOOSE = {"recon": 1e-12}
