@@ -232,6 +232,36 @@ int onmf_surrogate_fused_tc(const void* Ht, int src_kind, const void* pool, int6
                             const double* w_dev, void* A, void* B, void* workspace, size_t workspace_bytes, void* stream);
 
 /* ---------------------------------------------------------------------------------------------
+ * Patch minibatches by reference: the data matrix X (d x N), d = p*p*C, of the p x p patches of ONE resident image whose
+ * top-left corners are coords[0..N), without materialising it:
+ *     X[(r*p + c)*C + ch, j] = img[y_j + r, x_j + c, ch]        (the feature order of onmf_gather_patches)
+ * A minibatch is idx[0..n) into [0, N) (NULL: columns 0..n-1).  An index outside [0, N), or a corner whose patch leaves
+ * the image, yields a NaN row and is never dereferenced.  Storage: img is ONMF_F32, ONMF_F64 (fp64 engine, index gather
+ * only) or ONMF_STORE_U8 (value = (float)stored * (float)scale).  Every product gives the same bits as the same call on
+ * the materialised pool onmf_gather_patches(img, coords) (for u8: the pool of (float)u8 * scale, or the u8 pool on the
+ * fused path) with the same idx: only the addressing differs.
+ * ------------------------------------------------------------------------------------------- */
+typedef struct {
+  const void* img;          /* (H x W x C) row-major, device */
+  int kind;                 /* ONMF_F32, ONMF_F64 or ONMF_STORE_U8 */
+  int H, W, C, p;
+  const int32_t* coords;    /* (n_coords x 2) int32 top-left corners (y, x), device */
+  int64_t n_coords;         /* N */
+  const int64_t* idx;       /* n indices into [0, n_coords), device, or NULL for 0..n-1 */
+  int64_t n;                /* minibatch size (this rank's columns) */
+  double scale;             /* ONMF_STORE_U8: value = (float)stored * (float)scale */
+} onmf_patch_minibatch;
+
+/* index gather: Xt[j, :] = patch(coords[idx[j]]) as dtype_out rows (pitch ld elements), widening u8 -> fp32.  dtype_out is the
+ * image's dtype for ONMF_F32 / ONMF_F64 images and ONMF_F32 for ONMF_STORE_U8. */
+int onmf_gather_patches_mb(const onmf_patch_minibatch* pm, int dtype_out, void* Xt, int64_t ld, void* stream);
+/* onmf_cov_fused_tc / onmf_surrogate_fused_tc with the loaders reading patches of the image (fp32 or u8 image,
+ * onmf_fused_tc_supported(k, p*p*C); ONMF_E_UNSUPPORTED when (p+32)*W*C >= 2^31).  Workspace: onmf_surrogate_fused_tc_workspace. */
+int onmf_cov_fused_tc_patches(const onmf_patch_minibatch* pm, const void* W_hi, const void* W_lo, int k, void* Ct, void* stream);
+int onmf_surrogate_fused_tc_patches(const void* Ht, const onmf_patch_minibatch* pm, int k, void* P, int blend, double w,
+                                    const double* w_dev, void* A, void* B, void* workspace, size_t workspace_bytes, void* stream);
+
+/* ---------------------------------------------------------------------------------------------
  * K5  dictionary update (one block-coordinate-descent sweep)
  * replaces: update_dict  src/ontf.py:91-115 == src/onmf.py:92-116
  *   for j in 0..k-1:  W[:,j] -= (W A[:,j] - B[j,:]^T) / (A[j,j] + 1);  W[:,j] = max(W[:,j], 0);
@@ -382,6 +412,16 @@ int onmf_step_mb(onmf_step_plan* plan, const onmf_step_buffers* b, const onmf_mi
                  int cur);
 int onmf_step_graph_mb(onmf_step_plan* plan, const onmf_step_buffers* b, const onmf_minibatch* mb, const void* codes, double w,
                        int cur);
+/* the same three forms for a patch minibatch (onmf_patch_minibatch, d = p*p*C): the fused kernels read the patches of the
+ * image in place.  Same conditions as the _mb forms (use_tc, fp32, onmf_fused_tc_supported, no track_C) and an fp32 or u8
+ * image; other engines gather the minibatch with onmf_gather_patches_mb and take the dense forms.  The graph of
+ * onmf_step_graph_patches is keyed on the image, the corners, the geometry, the storage kind and the scale as well. */
+int onmf_step_launch_patches(onmf_step_plan* plan, const onmf_step_buffers* b, const onmf_patch_minibatch* pm, const void* codes,
+                             int cur);
+int onmf_step_patches(onmf_step_plan* plan, const onmf_step_buffers* b, const onmf_patch_minibatch* pm, const void* codes,
+                      double w, int cur);
+int onmf_step_graph_patches(onmf_step_plan* plan, const onmf_step_buffers* b, const onmf_patch_minibatch* pm, const void* codes,
+                            double w, int cur);
 
 #ifdef __cplusplus
 }

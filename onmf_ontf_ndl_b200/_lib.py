@@ -96,6 +96,12 @@ SIGNATURES = {
     "onmf_step_launch_mb": (_i, [_vp, _vp, _vp, _vp, _i]),
     "onmf_step_mb": (_i, [_vp, _vp, _vp, _vp, _dbl, _i]),
     "onmf_step_graph_mb": (_i, [_vp, _vp, _vp, _vp, _dbl, _i]),
+    "onmf_gather_patches_mb": (_i, [_vp, _i, _vp, _i64, _vp]),
+    "onmf_cov_fused_tc_patches": (_i, [_vp, _vp, _vp, _i, _vp, _vp]),
+    "onmf_surrogate_fused_tc_patches": (_i, [_vp, _vp, _i, _vp, _i, _dbl, _vp, _vp, _vp, _vp, _sz, _vp]),
+    "onmf_step_launch_patches": (_i, [_vp, _vp, _vp, _vp, _i]),
+    "onmf_step_patches": (_i, [_vp, _vp, _vp, _vp, _dbl, _i]),
+    "onmf_step_graph_patches": (_i, [_vp, _vp, _vp, _vp, _dbl, _i]),
 }
 
 
@@ -129,6 +135,33 @@ def make_minibatch(pool, idx, n, scale=1.0):
     mb.n = int(n)
     mb.scale = float(scale)
     return mb
+
+
+class PatchMinibatch(ctypes.Structure):
+    """onmf_patch_minibatch (include/onmf_b200.h): the patches at corners coords[idx[0..n)] of a resident image."""
+    _fields_ = [("img", _vp), ("kind", _i), ("H", _i), ("W", _i), ("C", _i), ("p", _i), ("coords", _vp), ("n_coords", _i64),
+                ("idx", _vp), ("n", _i64), ("scale", _dbl)]
+
+
+def make_patch_minibatch(img, p, coords, idx, n, scale=1.0):
+    """img (H x W) or (H x W x C) float32 / float64 / uint8, coords (N x 2) int32, idx int64 (n) or None (0..n-1)"""
+    _req(img, "img"); _req(coords, "coords", torch.int32)
+    if idx is not None:
+        _req(idx, "idx", torch.int64)
+    if img.dim() not in (2, 3) or coords.dim() != 2 or coords.shape[1] != 2:
+        raise OnmfKernelError("img must be (H x W [x C]) and coords (N x 2)")
+    pm = PatchMinibatch()
+    pm.img = img.data_ptr()
+    pm.kind = F64 if img.dtype == torch.float64 else _store_kind(img)
+    pm.H, pm.W = img.shape[0], img.shape[1]
+    pm.C = img.shape[2] if img.dim() == 3 else 1
+    pm.p = int(p)
+    pm.coords = coords.data_ptr()
+    pm.n_coords = coords.shape[0]
+    pm.idx = idx.data_ptr() if idx is not None else None
+    pm.n = int(n)
+    pm.scale = float(scale)
+    return pm
 
 
 _lib = None
@@ -504,6 +537,43 @@ def surrogate_fused_tc(Ht, pool, idx, n, d, P, workspace, scale=1.0, blend=None,
     return P
 
 
+def gather_patches_mb(pm, out, stream=None):
+    """out (n x d, float32 / float64, rows may be pitched) = the patches of a PatchMinibatch, widening uint8 to float32"""
+    if not out.is_cuda or out.dim() != 2 or (out.shape[0] > 1 and out.stride(1) != 1):
+        raise OnmfKernelError("out must be a CUDA (n x d) tensor with unit column stride")
+    _check(load().onmf_gather_patches_mb(ctypes.byref(pm), dt(out), _ptr(out), out.stride(0) if out.shape[0] else out.shape[1],
+                                         _stream(stream)), "onmf_gather_patches_mb")
+    return out
+
+
+def cov_fused_tc_patches(pm, Whi, Wlo, Ct, stream=None):
+    """Ct (n x k) = (patch minibatch) @ W on the fused tensor-core path"""
+    _req(Whi, "Whi", torch.float32); _req(Wlo, "Wlo", torch.float32); _req(Ct, "Ct", torch.float32)
+    _check(load().onmf_cov_fused_tc_patches(ctypes.byref(pm), _ptr(Whi), _ptr(Wlo), Whi.shape[1], _ptr(Ct), _stream(stream)),
+           "onmf_cov_fused_tc_patches")
+    return Ct
+
+
+def surrogate_fused_tc_patches(Ht, pm, P, workspace, blend=None, stream=None):
+    """P (k x (k+d)) = [Ht^T Ht | Ht^T X] for a patch minibatch X; blend = (w or a device float64 tensor, A, B)"""
+    _req(Ht, "Ht", torch.float32); _req(workspace, "workspace", torch.uint8)
+    if P is not None:
+        _req(P, "P", torch.float32)
+    w, w_dev, A, B = 0.0, None, None, None
+    if blend is not None:
+        wv, A, B = blend
+        _req(A, "A", torch.float32); _req(B, "B", torch.float32)
+        if isinstance(wv, torch.Tensor):
+            _req(wv, "w_dev", torch.float64)
+            w_dev = wv
+        else:
+            w = float(wv)
+    _check(load().onmf_surrogate_fused_tc_patches(_ptr(Ht), ctypes.byref(pm), Ht.shape[1], _ptr(P), 1 if blend is not None else 0, w,
+                                                  _ptr(w_dev), _ptr(A), _ptr(B), _ptr(workspace), workspace.numel(), _stream(stream)),
+           "onmf_surrogate_fused_tc_patches")
+    return P
+
+
 # ---- batched reconstruction ---------------------------------------------------------------------
 
 def pgd_code_columns(G, Ct, alpha, sub_iter, stopping_diff, Ht, stream=None):
@@ -597,3 +667,11 @@ class StepPlan:
     def step_mb(self, bufs, mb, codes, w, cur, graph=False):
         fn = load().onmf_step_graph_mb if graph else load().onmf_step_mb
         _check(fn(self._h, ctypes.byref(bufs), ctypes.byref(mb), _ptr(codes), float(w), int(cur)), "onmf_step_mb")
+
+    def launch_patches(self, bufs, pm, codes, cur):
+        _check(load().onmf_step_launch_patches(self._h, ctypes.byref(bufs), ctypes.byref(pm), _ptr(codes), int(cur)),
+               "onmf_step_launch_patches")
+
+    def step_patches(self, bufs, pm, codes, w, cur, graph=False):
+        fn = load().onmf_step_graph_patches if graph else load().onmf_step_patches
+        _check(fn(self._h, ctypes.byref(bufs), ctypes.byref(pm), _ptr(codes), float(w), int(cur)), "onmf_step_patches")

@@ -14,9 +14,29 @@ template <typename T> __device__ __forceinline__ T nan_of();
 template <> __device__ __forceinline__ float nan_of<float>() { return __int_as_float(0x7fc00000); }
 template <> __device__ __forceinline__ double nan_of<double>() { return __longlong_as_double(0x7ff8000000000000LL); }
 
-template <typename T>
-__global__ void gather_patches_kernel(const T* __restrict__ img, int H, int Wd, int C, const int32_t* __restrict__ coords,
-                                      long long n, int p, T* __restrict__ Xt, long long ld) {
+// stored image element -> output element: a copy, or the u8 widening (float)v * scale of onmf_widen
+template <typename T> __device__ __forceinline__ T widen_to(float v, float) { return (T)v; }
+template <typename T> __device__ __forceinline__ T widen_to(double v, float) { return (T)v; }
+template <typename T> __device__ __forceinline__ T widen_to(unsigned char v, float sc) { return (T)((float)v * sc); }
+
+// corner of minibatch sample j: coords[idx[j]] (idx == nullptr: coords[j]); false -> NaN row (index outside [0, n_coords)
+// or a patch that leaves the image), never read
+__device__ __forceinline__ bool patch_corner(const int32_t* __restrict__ coords, long long n_coords, const long long* __restrict__ idx,
+                                             long long j, int H, int Wd, int p, int& a, int& b) {
+  long long s = j;
+  if (idx) {
+    s = idx[j];
+    if (s < 0 || s >= n_coords) return false;
+  }
+  a = coords[2 * s]; b = coords[2 * s + 1];
+  return !(a < 0 || b < 0 || a > H - p || b > Wd - p);
+}
+
+// S: stored image type, T: output type.  idx == nullptr: sample j is coords[j] (n_coords == n); else coords[idx[j]].
+template <typename S, typename T>
+__global__ void gather_patches_kernel(const S* __restrict__ img, int H, int Wd, int C, const int32_t* __restrict__ coords,
+                                      long long n_coords, const long long* __restrict__ idx, long long n, int p, float scale,
+                                      T* __restrict__ Xt, long long ld) {
   // one warp per (patch, patch-row): the p*C values of a patch row are contiguous in the image and in Xt
   const int lane = threadIdx.x & 31;
   const long long wid = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
@@ -25,14 +45,14 @@ __global__ void gather_patches_kernel(const T* __restrict__ img, int H, int Wd, 
   for (long long t = wid; t < n * p; t += nw) {
     const long long j = t / p;
     const int r = (int)(t - j * p);
-    const int a = coords[2 * j], b = coords[2 * j + 1];
+    int a, b;
     T* dst = Xt + (size_t)j * ld + (size_t)r * run;
-    if (a < 0 || b < 0 || a > H - p || b > Wd - p) {        // corner outside the image: never read out of bounds,
-      for (int e = lane; e < run; e += 32) dst[e] = nan_of<T>();   // poison the patch so the error is loud downstream
+    if (!patch_corner(coords, n_coords, idx, j, H, Wd, p, a, b)) {   // never read out of bounds,
+      for (int e = lane; e < run; e += 32) dst[e] = nan_of<T>();     // poison the patch so the error is loud downstream
       continue;
     }
-    const T* src = img + ((size_t)(a + r) * Wd + b) * C;
-    for (int e = lane; e < run; e += 32) dst[e] = src[e];
+    const S* src = img + ((size_t)(a + r) * Wd + b) * C;
+    for (int e = lane; e < run; e += 32) dst[e] = widen_to<T>(src[e], scale);
   }
 }
 
@@ -85,10 +105,11 @@ __global__ void __launch_bounds__(256) gather_patches_vec_kernel(const T* __rest
 // loop, so the two integer divisions and the row-crossing logic of the flat kernel (which made it issue-bound at 0.45 of the
 // HBM rate) are paid once per thread: the V source offsets relative to the patch corner are loop invariants, and a patch costs
 // one broadcast corner load, V scalar loads and one 16-byte store.  Linear thread order == output order, stores stay coalesced.
-template <typename T, int V>
-__global__ void __launch_bounds__(1024) gather_patches_tile_kernel(const T* __restrict__ img, int H, int Wd, int C,
-                                                                   const int32_t* __restrict__ coords, long long n, int p,
-                                                                   T* __restrict__ Xt, long long ld) {
+template <typename S, typename T, int V>
+__global__ void __launch_bounds__(1024) gather_patches_tile_kernel(const S* __restrict__ img, int H, int Wd, int C,
+                                                                   const int32_t* __restrict__ coords, long long n_coords,
+                                                                   const long long* __restrict__ idx, long long n, int p,
+                                                                   float scale, T* __restrict__ Xt, long long ld) {
   struct __align__(16) Vec { T v[V]; };
   const int run = p * C;
   const int e0 = threadIdx.x * V;
@@ -103,15 +124,21 @@ __global__ void __launch_bounds__(1024) gather_patches_tile_kernel(const T* __re
   }
   const long long step = (long long)gridDim.x * blockDim.y;
   for (long long j = (long long)blockIdx.x * blockDim.y + threadIdx.y; j < n; j += step) {
-    const int2 ab = __ldg(reinterpret_cast<const int2*>(coords) + j);
+    long long s = j;
+    bool ok = true;
+    if (idx) {                                          // minibatch through an index (onmf_gather_patches_mb)
+      s = idx[j];
+      ok = s >= 0 && s < n_coords;
+    }
+    const int2 ab = ok ? __ldg(reinterpret_cast<const int2*>(coords) + s) : make_int2(-1, -1);
     Vec out;
     if (ab.x < 0 || ab.y < 0 || ab.x > H - p || ab.y > Wd - p) {
 #pragma unroll
       for (int t = 0; t < V; ++t) out.v[t] = nan_of<T>();
     } else {
-      const T* src = img + ((size_t)ab.x * Wd + ab.y) * C;
+      const S* src = img + ((size_t)ab.x * Wd + ab.y) * C;
 #pragma unroll
-      for (int t = 0; t < V; ++t) out.v[t] = __ldg(src + off[t]);
+      for (int t = 0; t < V; ++t) out.v[t] = widen_to<T>(__ldg(src + off[t]), scale);
     }
     *reinterpret_cast<Vec*>(Xt + (size_t)j * ld + e0) = out;
   }
@@ -483,8 +510,8 @@ extern "C" int onmf_gather_patches(int dtype, const void* img, int H, int Wd, in
         long long gq = cdiv<long long>(n, py);
         const long long capq = (long long)num_sms() * (2048 / (dv * py)) * 4;
         const int gridq = (int)(gq > capq ? capq : gq);
-        if (dtype == ONMF_F32) gather_patches_tile_kernel<float, 4><<<gridq, block, 0, st>>>((const float*)img, H, Wd, C, coords, n, p, (float*)Xt, ld);
-        else gather_patches_tile_kernel<double, 2><<<gridq, block, 0, st>>>((const double*)img, H, Wd, C, coords, n, p, (double*)Xt, ld);
+        if (dtype == ONMF_F32) gather_patches_tile_kernel<float, float, 4><<<gridq, block, 0, st>>>((const float*)img, H, Wd, C, coords, n, nullptr, n, p, 1.f, (float*)Xt, ld);
+        else gather_patches_tile_kernel<double, double, 2><<<gridq, block, 0, st>>>((const double*)img, H, Wd, C, coords, n, nullptr, n, p, 1.f, (double*)Xt, ld);
         ONMF_LAUNCH_CHECK("gather_patches_tile_kernel");
         return ONMF_OK;
       }
@@ -507,11 +534,53 @@ extern "C" int onmf_gather_patches(int dtype, const void* img, int H, int Wd, in
   long long warps = n * p;
   int grid = (int)cdiv<long long>(warps * 32, threads);
   if (grid > 8 * num_sms()) grid = 8 * num_sms();
-  if (dtype == ONMF_F32) gather_patches_kernel<float><<<grid, threads, 0, st>>>((const float*)img, H, Wd, C, coords, n, p, (float*)Xt, ld);
-  else if (dtype == ONMF_F64) gather_patches_kernel<double><<<grid, threads, 0, st>>>((const double*)img, H, Wd, C, coords, n, p, (double*)Xt, ld);
+  if (dtype == ONMF_F32) gather_patches_kernel<float, float><<<grid, threads, 0, st>>>((const float*)img, H, Wd, C, coords, n, nullptr, n, p, 1.f, (float*)Xt, ld);
+  else if (dtype == ONMF_F64) gather_patches_kernel<double, double><<<grid, threads, 0, st>>>((const double*)img, H, Wd, C, coords, n, nullptr, n, p, 1.f, (double*)Xt, ld);
   else return fail(ONMF_E_ARG, "gather_patches: bad dtype");
   ONMF_LAUNCH_CHECK("gather_patches_kernel");
   return ONMF_OK;
+}
+
+// the same two kernels on a patch minibatch: sample j is the patch at coords[idx[j]]
+template <typename S, typename T>
+static int gather_patches_mb(const onmf_patch_minibatch* pm, T* Xt, long long ld, cudaStream_t st) {
+  const int H = pm->H, Wd = pm->W, C = pm->C, p = pm->p;
+  const long long n = pm->n, d = (long long)p * p * C;
+  const S* img = (const S*)pm->img;
+  const float sc = (float)pm->scale;
+  const long long* idx = (const long long*)pm->idx;
+  constexpr int V = 16 / sizeof(T);
+  if (d % V == 0 && ld % V == 0 && d / V <= 1024 && (reinterpret_cast<uintptr_t>(Xt) & 15) == 0 &&
+      (reinterpret_cast<uintptr_t>(pm->coords) & 7) == 0 && (long long)H * Wd * C < (1LL << 31)) {
+    const int dv = (int)(d / V);
+    int py = 256 / dv;
+    if (py < 1) py = 1;
+    dim3 block((unsigned)dv, (unsigned)py);
+    const long long gq = cdiv<long long>(n, py);
+    const long long capq = (long long)num_sms() * (2048 / (dv * py)) * 4;
+    gather_patches_tile_kernel<S, T, V><<<(int)(gq > capq ? capq : gq), block, 0, st>>>(img, H, Wd, C, pm->coords, pm->n_coords, idx,
+                                                                                       n, p, sc, Xt, ld);
+    ONMF_LAUNCH_CHECK("gather_patches_tile_kernel");
+    return ONMF_OK;
+  }
+  int grid = (int)cdiv<long long>(n * p * 32, 256);
+  if (grid > 8 * num_sms()) grid = 8 * num_sms();
+  gather_patches_kernel<S, T><<<grid, 256, 0, st>>>(img, H, Wd, C, pm->coords, pm->n_coords, idx, n, p, sc, Xt, ld);
+  ONMF_LAUNCH_CHECK("gather_patches_kernel");
+  return ONMF_OK;
+}
+
+extern "C" int onmf_gather_patches_mb(const onmf_patch_minibatch* pm, int dtype_out, void* Xt, int64_t ld, void* stream) {
+  if (!pm || !pm->img || !Xt || pm->H <= 0 || pm->W <= 0 || pm->C <= 0 || pm->p <= 0 || pm->p > pm->H || pm->p > pm->W || pm->n < 0 ||
+      pm->n_coords < 0 || (pm->n_coords > 0 && !pm->coords) || ld < (int64_t)pm->p * pm->p * pm->C)
+    return fail(ONMF_E_ARG, "gather_patches_mb: bad argument");
+  if (!pm->idx && pm->n > pm->n_coords) return fail(ONMF_E_ARG, "gather_patches_mb: idx == NULL needs n <= n_coords");
+  if (pm->n == 0) return ONMF_OK;
+  cudaStream_t st = (cudaStream_t)stream;
+  if (pm->kind == ONMF_F32 && dtype_out == ONMF_F32) return gather_patches_mb<float>(pm, (float*)Xt, ld, st);
+  if (pm->kind == ONMF_F64 && dtype_out == ONMF_F64) return gather_patches_mb<double>(pm, (double*)Xt, ld, st);
+  if (pm->kind == ONMF_STORE_U8 && dtype_out == ONMF_F32) return gather_patches_mb<unsigned char>(pm, (float*)Xt, ld, st);
+  return fail(ONMF_E_ARG, "gather_patches_mb: storage / output kind must be F32 -> F32, F64 -> F64 or STORE_U8 -> F32");
 }
 
 extern "C" int onmf_gather_rows(int dtype, const void* pool, int64_t n_pool, int d, const int64_t* idx, int64_t n, void* Xt,

@@ -133,12 +133,73 @@ __device__ __forceinline__ void split4(const float4& x, float4& h, float4& l) {
   asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(t) : "f"(x.w)); h.w = __uint_as_float(t); l.w = x.w - h.w;
 }
 
+// The loaders read the minibatch through a SOURCE VIEW:
+//   row<S>(src, rp)  -> false for a sample that must become a NaN row (never dereferenced), else rp = its base address
+//   off(e)           -> where features e .. e+3 sit relative to a row's base (a function of e alone: computed once per
+//                       k-block / item and shared by every row the thread loads)
+//   ld4<S>(rp, o)    -> the 4 values widened to fp32 (value = (float)stored * scale for the narrow formats)
 struct PoolView {
   const void* base;       // stored minibatch pool, one sample per row
   long long ld;           // row pitch in ELEMENTS of the storage type
   const long long* idx;   // minibatch row indices into the pool, or nullptr (rows 0..n-1)
   long long n_pool;       // rows in the pool (indices outside [0, n_pool) contribute NaN rows, like the K1 gather)
   float scale;            // narrow formats: value = (float)stored * scale
+
+  struct Off { long long e; };
+  __device__ __forceinline__ Off off(int e) const { return Off{e}; }
+  template <typename S>
+  __device__ __forceinline__ bool row(long long src, const void*& rp) const {
+    rp = base;
+    if (src < 0 || src >= n_pool) return false;
+    rp = reinterpret_cast<const unsigned char*>(base) + (size_t)src * (size_t)ld * sizeof(S);
+    return true;
+  }
+  template <typename S>
+  __device__ __forceinline__ float4 ld4(const void* rp, const Off& o) const { return Src<S>::ld4(rp, o.e, scale); }
+};
+
+// A minibatch of image patches by reference: sample j is the p x p (x C) patch of the HWC image whose top-left corner is
+// coords[idx[j]], feature e = (r*p + c)*C + ch  ->  image element (y + r, x + c, ch).  A row's base is its corner; the
+// offset of feature e inside a patch is r*W*C + (c*C + ch), the same for every patch.  When p*C % 4 != 0 a 4-feature
+// chunk can straddle two patch rows, so the four offsets are kept separately and the values loaded as scalars (the
+// chunk is contiguous but in general unaligned in the image when p*C % 4 == 0: scalar loads as well).  Corner bases
+// are 64-bit; intra-patch offsets are 32-bit (the host checks (p+32)*W*C < 2^31).
+struct PatchView {
+  const void* img;        // (H x W x C) row-major
+  int H, W, C, p;
+  const int* coords;      // (n_coords x 2) int32 top-left corners (y, x)
+  long long n_coords;
+  const long long* idx;   // minibatch indices into coords, or nullptr (0..n-1)
+  float scale;
+
+  struct Off { int o[4]; };
+  __device__ __forceinline__ Off off(int e) const {
+    const int run = p * C, pitch = W * C;
+    int r = e / run, c = e - r * run;
+    Off f;
+#pragma unroll
+    for (int t = 0; t < 4; ++t) {
+      f.o[t] = r * pitch + c;
+      if (++c == run) { c = 0; ++r; }
+    }
+    return f;
+  }
+  template <typename S>
+  __device__ __forceinline__ bool row(long long src, const void*& rp) const {
+    rp = img;
+    if (src < 0 || src >= n_coords) return false;
+    const int y = __ldg(coords + 2 * src), x = __ldg(coords + 2 * src + 1);
+    if (y < 0 || x < 0 || y > H - p || x > W - p) return false;          // the patch leaves the image
+    rp = reinterpret_cast<const S*>(img) + ((size_t)y * (size_t)W + (size_t)x) * (size_t)C;
+    return true;
+  }
+  template <typename S>
+  __device__ __forceinline__ float4 ld4(const void* rp, const Off& f) const {
+    const S* q = reinterpret_cast<const S*>(rp);
+    return make_float4(wide(__ldg(q + f.o[0])), wide(__ldg(q + f.o[1])), wide(__ldg(q + f.o[2])), wide(__ldg(q + f.o[3])));
+  }
+  __device__ __forceinline__ float wide(float v) const { return v; }
+  __device__ __forceinline__ float wide(unsigned char v) const { return (float)v * scale; }   // as Src<unsigned char>::ld4
 };
 
 // =====================================================================================================================
@@ -155,9 +216,9 @@ struct CovCfg {
   static constexpr uint32_t CHUNK_BYTES = BK * 128;                // MN-major B: 32-wide N chunk = 32 k-rows x 128 B
 };
 
-template <int BN, typename S>
+template <int BN, typename S, typename V>
 __global__ void __launch_bounds__(THREADS, 1)
-cov_fused_kernel(const __grid_constant__ CUtensorMap tmW_hi, const __grid_constant__ CUtensorMap tmW_lo, PoolView X, long long n,
+cov_fused_kernel(const __grid_constant__ CUtensorMap tmW_hi, const __grid_constant__ CUtensorMap tmW_lo, V X, long long n,
                  int d, int k, float* __restrict__ Ct) {
   using C = CovCfg<BN>;
   constexpr int STAGES = C::STAGES;
@@ -292,9 +353,7 @@ cov_fused_kernel(const __grid_constant__ CUtensorMap tmW_hi, const __grid_consta
         rok[i] = j < n;
         long long src = 0;
         if (rok[i]) src = X.idx ? X.idx[j] : j;
-        rnan[i] = rok[i] && (src < 0 || src >= X.n_pool);
-        if (rnan[i]) src = 0;
-        rowp[i] = reinterpret_cast<const unsigned char*>(X.base) + (size_t)src * (size_t)X.ld * sizeof(S);
+        rnan[i] = !X.template row<S>(src, rowp[i]) && rok[i];
       }
       // first k-block of this group within the tile
       int kb = (int)((NLG - (c_tile0 % NLG) + g) % NLG);
@@ -303,12 +362,13 @@ cov_fused_kernel(const __grid_constant__ CUtensorMap tmW_hi, const __grid_consta
         const int s = (int)(c % STAGES);
         const uint32_t ph = (uint32_t)((c / STAGES) & 1);
         const int e = kb * C::BK + ch * 4;             // first feature of this thread's chunk (d % 4 == 0)
+        const typename V::Off eo = X.off(e);           // shared by the thread's 4 rows
         float4 x[4];
 #pragma unroll
         for (int i = 0; i < 4; ++i) {
           x[i] = make_float4(0.f, 0.f, 0.f, 0.f);
-          if (rok[i] && e < d) x[i] = Src<S>::ld4(rowp[i], e, X.scale);
           if (rnan[i]) { const float qn = __int_as_float(0x7fc00000); x[i] = make_float4(qn, qn, qn, qn); }
+          else if (rok[i] && e < d) x[i] = X.template ld4<S>(rowp[i], eo);
         }
         mbar_wait(smem_u32(&empty_bar[s]), ph ^ 1);    // the MMAs that read this stage last time have completed
         uint8_t* a_hi = stage_ptr(s);
@@ -355,9 +415,9 @@ __device__ __forceinline__ uint32_t mn_off(int kr, int mn) {
   return (uint32_t)((mn >> 5) * SurCfg::CHUNK + (kr >> 2) * 512 + (kr & 3) * 128 + ((((mn & 31) >> 3) ^ (kr & 3)) << 5) + ((mn & 7) >> 2) * 16);
 }
 
-template <typename S>
+template <typename S, typename V>
 __global__ void __launch_bounds__(THREADS, 1)
-sur_fused_kernel(const float* __restrict__ Ht, PoolView X, long long n, int k, int d, int n_tiles, int splits, long long kb_per_split,
+sur_fused_kernel(const float* __restrict__ Ht, V X, long long n, int k, int d, int n_tiles, int splits, long long kb_per_split,
                  float* __restrict__ part) {
   using C = SurCfg;
   extern __shared__ uint8_t smem_dyn[];
@@ -496,6 +556,12 @@ sur_fused_kernel(const float* __restrict__ Ht, PoolView X, long long n, int k, i
       long long kb0, kb1; int nt;
       item_range(item, kb0, kb1, nt);
       const int n0 = nt * C::BN;                       // first column of [Ht | X] of this item
+      typename V::Off xo[4];                           // feature offsets of the thread's X columns: fixed for the item
+#pragma unroll
+      for (int p = 0; p < 4; ++p) {
+        const int col = n0 + (f0 + 16 * p) * 4;
+        xo[p] = X.off(col >= k && col < ncat ? col - k : 0);
+      }
       long long kb = kb0 + (long long)((NLG - (c0 % NLG) + g) % NLG);
       long long src_next = -1;                         // pool row of sample (kb, kr), fetched one k-block ahead
       {
@@ -514,9 +580,9 @@ sur_fused_kernel(const float* __restrict__ Ht, PoolView X, long long n, int k, i
           src_next = -1;
           if (kb + NLG < kb1 && jn < n) src_next = X.idx ? X.idx[jn] : jn;
         }
-        const bool bad = jok && (src < 0 || src >= X.n_pool);
+        const void* xrow;
+        const bool bad = !X.template row<S>(jok ? src : 0, xrow) && jok;
         const float* hrow = Ht + (size_t)(jok ? j : 0) * k;
-        const void* xrow = reinterpret_cast<const unsigned char*>(X.base) + (size_t)((jok && !bad) ? src : 0) * (size_t)X.ld * sizeof(S);
         float4 a[4], b[4];
 #pragma unroll
         for (int p = 0; p < 4; ++p) {
@@ -528,7 +594,7 @@ sur_fused_kernel(const float* __restrict__ Ht, PoolView X, long long n, int k, i
           if (jok && col < ncat) {
             if (col < k) b[p] = *reinterpret_cast<const float4*>(hrow + col);
             else if (bad) { const float qn = __int_as_float(0x7fc00000); b[p] = make_float4(qn, qn, qn, qn); }
-            else b[p] = Src<S>::ld4(xrow, col - k, X.scale);
+            else b[p] = X.template ld4<S>(xrow, xo[p]);
           }
         }
         mbar_wait(smem_u32(&empty_bar[s]), ph ^ 1);
@@ -632,9 +698,9 @@ static int check_pool(int src_kind, const void* pool, int64_t ld, int d, const c
   return ONMF_OK;
 }
 
-template <int BN, typename S>
-static int launch_cov(const CUtensorMap& mh, const CUtensorMap& ml, const PoolView& X, long long n, int d, int k, float* Ct, cudaStream_t st) {
-  auto kern = cov_fused_kernel<BN, S>;
+template <int BN, typename S, typename V>
+static int launch_cov(const CUtensorMap& mh, const CUtensorMap& ml, const V& X, long long n, int d, int k, float* Ct, cudaStream_t st) {
+  auto kern = cov_fused_kernel<BN, S, V>;
   ONMF_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CovCfg<BN>::SMEM_BYTES));
   const long long ntiles = cdiv<long long>(n, BM);
   const int grid = (int)std::min<long long>(ntiles, num_sms());
@@ -643,8 +709,8 @@ static int launch_cov(const CUtensorMap& mh, const CUtensorMap& ml, const PoolVi
   return ONMF_OK;
 }
 
-template <typename S>
-static int dispatch_cov(const CUtensorMap& mh, const CUtensorMap& ml, const PoolView& X, long long n, int d, int k, float* Ct, cudaStream_t st) {
+template <typename S, typename V>
+static int dispatch_cov(const CUtensorMap& mh, const CUtensorMap& ml, const V& X, long long n, int d, int k, float* Ct, cudaStream_t st) {
   if (k <= 64) return launch_cov<64, S>(mh, ml, X, n, d, k, Ct, st);
   if (k <= 128) return launch_cov<128, S>(mh, ml, X, n, d, k, Ct, st);
   return launch_cov<256, S>(mh, ml, X, n, d, k, Ct, st);
@@ -661,6 +727,43 @@ static void sur_plan(long long n, int k, int d, int* n_tiles, int* splits, long 
   long long per = cdiv<long long>(kb_total, s);
   s = cdiv<long long>(kb_total, per);
   *n_tiles = nt; *splits = (int)s; *kb_per_split = per;
+}
+
+template <typename S, typename V>
+static int launch_sur(const float* Ht, const V& X, long long n, int k, int d, int nt, int sp, long long per, float* part, cudaStream_t st) {
+  auto kern = sur_fused_kernel<S, V>;
+  ONMF_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SurCfg::SMEM_BYTES));
+  const int grid = (int)std::min<long long>((long long)nt * sp, num_sms());
+  kern<<<grid, THREADS, SurCfg::SMEM_BYTES, st>>>(Ht, X, n, k, d, nt, sp, per, part);
+  ONMF_LAUNCH_CHECK("sur_fused_kernel");
+  return ONMF_OK;
+}
+
+// fixed-order sum of the per-range partial tiles into P (and, blend != 0, the A / B recursion in the same pass)
+static int sur_reduce(const float* part, int nt, int sp, int mrows, int k, int d, void* P, int blend, double w, const double* w_dev,
+                      void* A, void* B, cudaStream_t st) {
+  const long long tot = (long long)k * (k + d);
+  const unsigned grid2 = (unsigned)cdiv<long long>(tot, 256);
+  if (blend) sur_reduce_kernel<true><<<grid2, 256, 0, st>>>(part, nt, sp, mrows, k, d, (float*)P, w_dev, w, (float*)A, (float*)B);
+  else sur_reduce_kernel<false><<<grid2, 256, 0, st>>>(part, nt, sp, mrows, k, d, (float*)P, nullptr, 0.0, nullptr, nullptr);
+  ONMF_LAUNCH_CHECK("sur_reduce_kernel");
+  return ONMF_OK;
+}
+
+// a patch minibatch the fused kernels can read: fp32 / u8 image, sane geometry, 32-bit intra-patch offsets
+static int check_patches(const onmf_patch_minibatch* pm, const char* who) {
+  if (!pm || !pm->img || pm->H <= 0 || pm->W <= 0 || pm->C <= 0 || pm->p <= 0 || pm->p > pm->H || pm->p > pm->W || pm->n < 0 ||
+      pm->n_coords < 0 || (pm->n_coords > 0 && !pm->coords))
+    return fail(ONMF_E_ARG, who);
+  if (pm->kind != ONMF_F32 && pm->kind != ONMF_STORE_U8)
+    return fail(ONMF_E_ARG, "fused tensor-core products: a patch minibatch's image must be ONMF_F32 or ONMF_STORE_U8");
+  if ((long long)(pm->p + 32) * pm->W * pm->C >= (1LL << 31))
+    return fail(ONMF_E_UNSUPPORTED, "fused tensor-core products: image rows too wide for 32-bit offsets inside a patch ((p+32)*W*C >= 2^31)");
+  return ONMF_OK;
+}
+
+static PatchView patch_view(const onmf_patch_minibatch* pm) {
+  return PatchView{pm->img, pm->H, pm->W, pm->C, pm->p, pm->coords, pm->n_coords, (const long long*)pm->idx, (float)pm->scale};
 }
 
 }  // namespace tcf
@@ -719,23 +822,56 @@ extern "C" int onmf_surrogate_fused_tc(const void* Ht, int src_kind, const void*
     ONMF_CUDA(cudaMemsetAsync(part, 0, (size_t)items * mrows * tcf::SurCfg::BN * sizeof(float), st));
   } else {
     tcf::PoolView X{pool, ld_pool, (const long long*)idx, n_pool, (float)scale};
-    const int grid = (int)std::min<long long>(items, num_sms());
-#define ONMF_SUR(S)                                                                                                   \
-  {                                                                                                                   \
-    auto kern = tcf::sur_fused_kernel<S>;                                                                             \
-    ONMF_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tcf::SurCfg::SMEM_BYTES)); \
-    kern<<<grid, tcf::THREADS, tcf::SurCfg::SMEM_BYTES, st>>>((const float*)Ht, X, n, k, d, nt, sp, per, part);       \
+    if (src_kind == ONMF_F32) rc = tcf::launch_sur<float>((const float*)Ht, X, n, k, d, nt, sp, per, part, st);
+    else if (src_kind == ONMF_STORE_U8) rc = tcf::launch_sur<unsigned char>((const float*)Ht, X, n, k, d, nt, sp, per, part, st);
+    else rc = tcf::launch_sur<__half>((const float*)Ht, X, n, k, d, nt, sp, per, part, st);
+    if (rc) return rc;
   }
-    if (src_kind == ONMF_F32) ONMF_SUR(float)
-    else if (src_kind == ONMF_STORE_U8) ONMF_SUR(unsigned char)
-    else ONMF_SUR(__half)
-#undef ONMF_SUR
-    ONMF_LAUNCH_CHECK("sur_fused_kernel");
+  return tcf::sur_reduce(part, nt, sp, mrows, k, d, P, blend, w, w_dev, A, B, st);
+}
+
+// ---- the same two products on a patch minibatch (PatchView loaders) ----
+extern "C" int onmf_cov_fused_tc_patches(const onmf_patch_minibatch* pm, const void* W_hi, const void* W_lo, int k, void* Ct, void* stream) {
+  int rc = tcf::check_patches(pm, "cov_fused_tc_patches: bad patch minibatch");
+  if (rc) return rc;
+  const int d = pm->p * pm->p * pm->C;
+  if (!W_hi || !W_lo || !Ct || !onmf_fused_tc_supported(k, d)) return fail(ONMF_E_ARG, "cov_fused_tc_patches: bad argument / unsupported shape");
+  if (!tcf::aligned16(W_hi) || !tcf::aligned16(W_lo) || !tcf::aligned16(Ct)) return fail(ONMF_E_ARG, "cov_fused_tc_patches: W_hi / W_lo / Ct must be 16-byte aligned");
+  if (pm->n == 0) return ONMF_OK;
+  CUtensorMap mh, ml;
+  if ((rc = tcf::make_map_mn(&mh, (const float*)W_hi, k, d, k, 32))) return rc;
+  if ((rc = tcf::make_map_mn(&ml, (const float*)W_lo, k, d, k, 32))) return rc;
+  const tcf::PatchView X = tcf::patch_view(pm);
+  cudaStream_t st = (cudaStream_t)stream;
+  if (pm->kind == ONMF_F32) return tcf::dispatch_cov<float>(mh, ml, X, pm->n, d, k, (float*)Ct, st);
+  return tcf::dispatch_cov<unsigned char>(mh, ml, X, pm->n, d, k, (float*)Ct, st);
+}
+
+extern "C" int onmf_surrogate_fused_tc_patches(const void* Ht, const onmf_patch_minibatch* pm, int k, void* P, int blend, double w,
+                                               const double* w_dev, void* A, void* B, void* workspace, size_t workspace_bytes,
+                                               void* stream) {
+  int rc = tcf::check_patches(pm, "surrogate_fused_tc_patches: bad patch minibatch");
+  if (rc) return rc;
+  const int d = pm->p * pm->p * pm->C;
+  const long long n = pm->n;
+  if (!Ht || !onmf_fused_tc_supported(k, d)) return fail(ONMF_E_ARG, "surrogate_fused_tc_patches: bad argument / unsupported shape");
+  if (!P && !blend) return fail(ONMF_E_ARG, "surrogate_fused_tc_patches: nothing to write (P == NULL and blend == 0)");
+  if (blend && (!A || !B)) return fail(ONMF_E_ARG, "surrogate_fused_tc_patches: blend needs A and B");
+  if (!tcf::aligned16(Ht)) return fail(ONMF_E_ARG, "surrogate_fused_tc_patches: Ht must be 16-byte aligned");
+  if (!workspace || workspace_bytes < onmf_surrogate_fused_tc_workspace(n, k, d)) return fail(ONMF_E_WORKSPACE, "surrogate_fused_tc_patches: workspace too small");
+  if ((uintptr_t)workspace % 16) return fail(ONMF_E_ARG, "surrogate_fused_tc_patches: workspace must be 16-byte aligned");
+  cudaStream_t st = (cudaStream_t)stream;
+  int nt, sp; long long per;
+  tcf::sur_plan(n, k, d, &nt, &sp, &per);
+  const int mrows = cdiv(k, 128) * 128;
+  float* part = (float*)workspace;
+  if (n == 0) {
+    ONMF_CUDA(cudaMemsetAsync(part, 0, (size_t)nt * sp * mrows * tcf::SurCfg::BN * sizeof(float), st));
+  } else {
+    const tcf::PatchView X = tcf::patch_view(pm);
+    if (pm->kind == ONMF_F32) rc = tcf::launch_sur<float>((const float*)Ht, X, n, k, d, nt, sp, per, part, st);
+    else rc = tcf::launch_sur<unsigned char>((const float*)Ht, X, n, k, d, nt, sp, per, part, st);
+    if (rc) return rc;
   }
-  const long long tot = (long long)k * (k + d);
-  const unsigned grid2 = (unsigned)cdiv<long long>(tot, 256);
-  if (blend) tcf::sur_reduce_kernel<true><<<grid2, 256, 0, st>>>(part, nt, sp, mrows, k, d, (float*)P, w_dev, w, (float*)A, (float*)B);
-  else tcf::sur_reduce_kernel<false><<<grid2, 256, 0, st>>>(part, nt, sp, mrows, k, d, (float*)P, nullptr, 0.0, nullptr, nullptr);
-  ONMF_LAUNCH_CHECK("sur_reduce_kernel");
-  return ONMF_OK;
+  return tcf::sur_reduce(part, nt, sp, mrows, k, d, P, blend, w, w_dev, A, B, st);
 }

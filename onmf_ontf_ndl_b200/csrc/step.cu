@@ -16,13 +16,15 @@
 // in place (gather, widening and TF32 split inside the loaders), nothing of the minibatch is ever copied or split in HBM,
 // and on a single GPU the blend is the epilogue of the partial-sum reduction:
 //   main : cov_fused(pool, idx) -> LARS -> wait(W_t) -> sur_fused(Ht, pool, idx) + reduce + blend -> record(code_t, AB_t)
+// A third kind, the patch minibatch (onmf_patch_minibatch: image + corners + indices), takes the same fused schedule with
+// the loaders reading the patches out of the image.
 #include <new>
 
 #include "common.cuh"
 
 // one instantiated CUDA graph of the whole step for a fixed (minibatch pointer, codes pointer, n, cur, buffers)
 struct StepGraph {
-  const void* Xt;             // minibatch base pointer (Xt, or the pool of a minibatch descriptor)
+  const void* Xt;             // minibatch base pointer (Xt, the pool of a minibatch descriptor, or a patch minibatch's image)
   const void* idx;            // minibatch row indices (descriptor form) or nullptr
   const void* codes;
   long long n;
@@ -140,10 +142,12 @@ static int check_buffers(const onmf_step_buffers* b, bool need_code_bufs) {
   return ONMF_OK;
 }
 
-// what one step consumes: a dense minibatch or a descriptor (exactly one of Xt / mb, or neither on the pre-split path)
+// what one step consumes: a dense minibatch, a pool descriptor or a patch minibatch (at most one of Xt / mb / pm; none on
+// the pre-split path)
 struct StepIn {
   const void* Xt;              // dense (n x d) in the engine dtype, or nullptr
   const onmf_minibatch* mb;    // descriptor (fused tensor-core path), or nullptr
+  const onmf_patch_minibatch* pm;   // patches of a resident image (fused tensor-core path), or nullptr
   const void* codes;           // externally computed codes (n x k) or nullptr
   long long n;
 };
@@ -155,7 +159,22 @@ struct Blend {
 };
 
 static bool mb_fused(const onmf_step_buffers* b, const StepIn& in) {
-  return in.mb != nullptr && b->use_tc && onmf_fused_tc_supported(b->k, b->d);
+  return (in.mb != nullptr || in.pm != nullptr) && b->use_tc && onmf_fused_tc_supported(b->k, b->d);
+}
+
+// the two fused products on whichever by-reference minibatch the step carries
+static int fused_cov(const onmf_step_buffers* b, const StepIn& in, int cur, cudaStream_t st) {
+  if (in.pm) return onmf_cov_fused_tc_patches(in.pm, b->Whi[cur], b->Wlo[cur], b->k, b->Ct, st);
+  return onmf_cov_fused_tc(in.mb->kind, in.mb->base, in.mb->n_pool, in.mb->ld, in.mb->idx, in.n, b->d, in.mb->scale, b->Whi[cur],
+                           b->Wlo[cur], b->k, b->Ct, st);
+}
+static int fused_sur(const onmf_step_buffers* b, const StepIn& in, const void* H, void* P, int blend, double w, const double* w_dev,
+                     cudaStream_t st) {
+  void* A = blend ? b->A : nullptr;
+  void* B = blend ? b->B : nullptr;
+  if (in.pm) return onmf_surrogate_fused_tc_patches(H, in.pm, b->k, P, blend, w, w_dev, A, B, b->ws_sur, b->ws_sur_bytes, st);
+  return onmf_surrogate_fused_tc(H, in.mb->kind, in.mb->base, in.mb->n_pool, in.mb->ld, in.mb->idx, in.n, b->k, b->d, in.mb->scale, P,
+                                 blend, w, w_dev, A, B, b->ws_sur, b->ws_sur_bytes, st);
 }
 
 // Enqueue one step.  captured = false: two streams ordered by the plan's events (cross-step overlap);
@@ -168,7 +187,7 @@ static int enqueue_step(onmf_step_plan* p, const onmf_step_buffers* b, const Ste
   const size_t esz = dt == ONMF_F64 ? 8 : 4;
   const long long n = in.n;
   const bool fused = mb_fused(b, in);
-  const bool presplit = (in.Xt == nullptr && in.mb == nullptr);
+  const bool presplit = (in.Xt == nullptr && in.mb == nullptr && in.pm == nullptr);
   int rc;
   const long long l0 = g_launches;
   *blended = false;
@@ -199,9 +218,7 @@ static int enqueue_step(onmf_step_plan* p, const onmf_step_buffers* b, const Ste
     }
     if (!in.codes) {
       if (!b->Ct || !b->ws_lars) return fail(ONMF_E_ARG, "step: null coder buffer");
-      if (fused)
-        rc = onmf_cov_fused_tc(in.mb->kind, in.mb->base, in.mb->n_pool, in.mb->ld, in.mb->idx, n, d, in.mb->scale, b->Whi[cur],
-                               b->Wlo[cur], k, b->Ct, main);
+      if (fused) rc = fused_cov(b, in, cur, main);
       else if (b->use_tc) rc = onmf_cov_tc(b->Xhi, b->Xlo, n, d, b->Whi[cur], b->Wlo[cur], k, b->Ct, main);
       else rc = onmf_cov(dt, in.Xt, n, d, b->W[cur], k, b->Ct, main);
       if (rc) return rc;
@@ -230,12 +247,10 @@ static int enqueue_step(onmf_step_plan* p, const onmf_step_buffers* b, const Ste
       if (fuse_blend) {
         // the blend overwrites A, B: the dictionary update (side) must have finished reading them
         ONMF_CUDA(cudaStreamWaitEvent(main, captured ? p->ev_g2 : p->ev_W, 0));
-        rc = onmf_surrogate_fused_tc(Hcodes, in.mb->kind, in.mb->base, in.mb->n_pool, in.mb->ld, in.mb->idx, n, k, d, in.mb->scale,
-                                     nullptr, 1, bl.w, bl.mode == 2 ? b->w_dev : nullptr, b->A, b->B, b->ws_sur, b->ws_sur_bytes, main);
+        rc = fused_sur(b, in, Hcodes, nullptr, 1, bl.w, bl.mode == 2 ? b->w_dev : nullptr, main);
         *blended = true;
       } else {
-        rc = onmf_surrogate_fused_tc(Hcodes, in.mb->kind, in.mb->base, in.mb->n_pool, in.mb->ld, in.mb->idx, n, k, d, in.mb->scale,
-                                     b->P[cur], 0, 0.0, nullptr, nullptr, nullptr, b->ws_sur, b->ws_sur_bytes, main);
+        rc = fused_sur(b, in, Hcodes, b->P[cur], 0, 0.0, nullptr, main);
       }
       if (rc) return rc;
     } else if (b->use_tc) {
@@ -260,13 +275,20 @@ static int check_step_in(const onmf_step_buffers* b, const StepIn& in, int cur, 
   int rc = check_buffers(b, in.n > 0);
   if (rc) return rc;
   if (in.n < 0 || (cur != 0 && cur != 1)) return fail(ONMF_E_ARG, who);
-  if (in.Xt && in.mb) return fail(ONMF_E_ARG, "step: pass either a dense minibatch or a descriptor, not both");
+  if ((in.Xt != nullptr) + (in.mb != nullptr) + (in.pm != nullptr) > 1)
+    return fail(ONMF_E_ARG, "step: pass one of a dense minibatch, a descriptor or a patch minibatch");
   if (in.mb) {
     if (in.mb->n != in.n) return fail(ONMF_E_ARG, "step: descriptor row count differs from n");
     if (!mb_fused(b, in)) return fail(ONMF_E_UNSUPPORTED, "step: a minibatch descriptor needs the fused tensor-core path (fp32, onmf_fused_tc_supported)");
     if (b->track_C) return fail(ONMF_E_UNSUPPORTED, "step: track_C needs a dense minibatch");
   }
-  const bool presplit = (in.Xt == nullptr && in.mb == nullptr);
+  if (in.pm) {
+    if (in.pm->n != in.n) return fail(ONMF_E_ARG, "step: patch minibatch size differs from n");
+    if ((long long)in.pm->p * in.pm->p * in.pm->C != b->d) return fail(ONMF_E_ARG, "step: patch minibatch p*p*C differs from d");
+    if (!mb_fused(b, in)) return fail(ONMF_E_UNSUPPORTED, "step: a patch minibatch needs the fused tensor-core path (fp32, onmf_fused_tc_supported); gather it with onmf_gather_patches_mb otherwise");
+    if (b->track_C) return fail(ONMF_E_UNSUPPORTED, "step: track_C needs a dense minibatch");
+  }
+  const bool presplit = (in.Xt == nullptr && in.mb == nullptr && in.pm == nullptr);
   if (in.n > 0 && presplit && !b->use_tc) return fail(ONMF_E_ARG, "step: Xt = NULL needs the tensor-core path");
   if (in.n > 0 && presplit && b->track_C) return fail(ONMF_E_ARG, "step: track_C needs the unsplit minibatch");
   return ONMF_OK;
@@ -305,7 +327,7 @@ static int finish_streams(onmf_step_plan* p, const onmf_step_buffers* b, double 
 extern "C" int onmf_step_launch(onmf_step_plan* p, const onmf_step_buffers* b, const void* Xt, const void* codes,
                                 int64_t n, int cur) {
   if (!p) return fail(ONMF_E_ARG, "step_launch: null plan");
-  StepIn in{Xt, nullptr, codes, n};
+  StepIn in{Xt, nullptr, nullptr, codes, n};
   int rc = check_step_in(b, in, cur, "step_launch: bad argument");
   if (rc) return rc;
   bool blended;
@@ -314,7 +336,7 @@ extern "C" int onmf_step_launch(onmf_step_plan* p, const onmf_step_buffers* b, c
 
 extern "C" int onmf_step_launch_mb(onmf_step_plan* p, const onmf_step_buffers* b, const onmf_minibatch* mb, const void* codes, int cur) {
   if (!p || !mb) return fail(ONMF_E_ARG, "step_launch_mb: null plan / descriptor");
-  StepIn in{nullptr, mb, codes, mb->n};
+  StepIn in{nullptr, mb, nullptr, codes, mb->n};
   int rc = check_step_in(b, in, cur, "step_launch_mb: bad argument");
   if (rc) return rc;
   bool blended;
@@ -338,7 +360,7 @@ static int step_streams(onmf_step_plan* p, const onmf_step_buffers* b, const Ste
 extern "C" int onmf_step(onmf_step_plan* p, const onmf_step_buffers* b, const void* Xt, const void* codes, int64_t n,
                          double w, int cur) {
   if (!p) return fail(ONMF_E_ARG, "step: null plan");
-  StepIn in{Xt, nullptr, codes, n};
+  StepIn in{Xt, nullptr, nullptr, codes, n};
   int rc = check_step_in(b, in, cur, "step: bad argument");
   if (rc) return rc;
   return step_streams(p, b, in, w, cur);
@@ -347,7 +369,7 @@ extern "C" int onmf_step(onmf_step_plan* p, const onmf_step_buffers* b, const vo
 extern "C" int onmf_step_mb(onmf_step_plan* p, const onmf_step_buffers* b, const onmf_minibatch* mb, const void* codes, double w,
                             int cur) {
   if (!p || !mb) return fail(ONMF_E_ARG, "step_mb: null plan / descriptor");
-  StepIn in{nullptr, mb, codes, mb->n};
+  StepIn in{nullptr, mb, nullptr, codes, mb->n};
   int rc = check_step_in(b, in, cur, "step_mb: bad argument");
   if (rc) return rc;
   return step_streams(p, b, in, w, cur);
@@ -363,10 +385,20 @@ extern "C" int onmf_step_mb(onmf_step_plan* p, const onmf_step_buffers* b, const
 // Graphs are cached per (minibatch pointers, codes pointer, n, cur, buffer descriptor); a key is captured the second
 // time it is seen, so one-off calls never pay for capture + instantiation.
 // ------------------------------------------------------------------------------------------------------------------
-static unsigned long long buffers_sig(const onmf_step_buffers* b, const onmf_minibatch* mb) {
+static unsigned long long buffers_sig(const onmf_step_buffers* b, const onmf_minibatch* mb, const onmf_patch_minibatch* pm) {
   unsigned long long h = 1469598103934665603ULL;
   const unsigned char* q = reinterpret_cast<const unsigned char*>(b);
   for (size_t i = 0; i < sizeof(*b); ++i) { h ^= q[i]; h *= 1099511628211ULL; }
+  if (pm) {
+    // everything a replay bakes in besides the image / index pointers of the key: corners, geometry, storage, scale
+    double sc = pm->scale;
+    unsigned long long scb;
+    memcpy(&scb, &sc, 8);
+    const unsigned long long v[9] = {0x70617463686573ull, (unsigned long long)(uintptr_t)pm->coords, (unsigned long long)pm->n_coords,
+                                     (unsigned long long)pm->kind, (unsigned long long)pm->H, (unsigned long long)pm->W,
+                                     (unsigned long long)pm->C, (unsigned long long)pm->p, scb};
+    for (int i = 0; i < 9; ++i) { h ^= v[i]; h *= 1099511628211ULL; }
+  }
   if (mb) {
     const unsigned long long v[4] = {(unsigned long long)mb->kind, (unsigned long long)mb->n_pool, (unsigned long long)mb->ld, 0ull};
     double sc = mb->scale;
@@ -382,9 +414,9 @@ static int step_graph_impl(onmf_step_plan* p, const onmf_step_buffers* b, const 
   // not expressible as this graph: the d x d aggregate (host-side w in its blend), coder timing events, multi-GPU hold
   if (!b->w_dev || b->track_C || p->tslots > 0 || b->hold_coder) return step_streams(p, b, in, w, cur);
   cudaStream_t main = (cudaStream_t)b->main_stream, side = (cudaStream_t)b->side_stream;
-  const void* base = in.mb ? in.mb->base : in.Xt;
-  const void* idx = in.mb ? (const void*)in.mb->idx : nullptr;
-  const unsigned long long sig = buffers_sig(b, in.mb);
+  const void* base = in.pm ? in.pm->img : in.mb ? in.mb->base : in.Xt;
+  const void* idx = in.pm ? (const void*)in.pm->idx : in.mb ? (const void*)in.mb->idx : nullptr;
+  const unsigned long long sig = buffers_sig(b, in.mb, in.pm);
   StepGraph* e = nullptr;
   for (int i = 0; i < STEP_GRAPHS; ++i) {
     StepGraph& g = p->graphs[i];
@@ -457,7 +489,7 @@ static int step_graph_impl(onmf_step_plan* p, const onmf_step_buffers* b, const 
 extern "C" int onmf_step_graph(onmf_step_plan* p, const onmf_step_buffers* b, const void* Xt, const void* codes, int64_t n,
                                double w, int cur) {
   if (!p) return fail(ONMF_E_ARG, "step_graph: null plan");
-  StepIn in{Xt, nullptr, codes, n};
+  StepIn in{Xt, nullptr, nullptr, codes, n};
   int rc = check_step_in(b, in, cur, "step_graph: bad argument");
   if (rc) return rc;
   return step_graph_impl(p, b, in, w, cur);
@@ -466,8 +498,37 @@ extern "C" int onmf_step_graph(onmf_step_plan* p, const onmf_step_buffers* b, co
 extern "C" int onmf_step_graph_mb(onmf_step_plan* p, const onmf_step_buffers* b, const onmf_minibatch* mb, const void* codes,
                                   double w, int cur) {
   if (!p || !mb) return fail(ONMF_E_ARG, "step_graph_mb: null plan / descriptor");
-  StepIn in{nullptr, mb, codes, mb->n};
+  StepIn in{nullptr, mb, nullptr, codes, mb->n};
   int rc = check_step_in(b, in, cur, "step_graph_mb: bad argument");
+  if (rc) return rc;
+  return step_graph_impl(p, b, in, w, cur);
+}
+
+// ---- patch minibatches --------------------------------------------------------------------------------------------
+extern "C" int onmf_step_launch_patches(onmf_step_plan* p, const onmf_step_buffers* b, const onmf_patch_minibatch* pm, const void* codes,
+                                        int cur) {
+  if (!p || !pm) return fail(ONMF_E_ARG, "step_launch_patches: null plan / patch minibatch");
+  StepIn in{nullptr, nullptr, pm, codes, pm->n};
+  int rc = check_step_in(b, in, cur, "step_launch_patches: bad argument");
+  if (rc) return rc;
+  bool blended;
+  return launch_streams(p, b, in, cur, Blend{0, 0.0}, &blended);
+}
+
+extern "C" int onmf_step_patches(onmf_step_plan* p, const onmf_step_buffers* b, const onmf_patch_minibatch* pm, const void* codes, double w,
+                                 int cur) {
+  if (!p || !pm) return fail(ONMF_E_ARG, "step_patches: null plan / patch minibatch");
+  StepIn in{nullptr, nullptr, pm, codes, pm->n};
+  int rc = check_step_in(b, in, cur, "step_patches: bad argument");
+  if (rc) return rc;
+  return step_streams(p, b, in, w, cur);
+}
+
+extern "C" int onmf_step_graph_patches(onmf_step_plan* p, const onmf_step_buffers* b, const onmf_patch_minibatch* pm, const void* codes,
+                                       double w, int cur) {
+  if (!p || !pm) return fail(ONMF_E_ARG, "step_graph_patches: null plan / patch minibatch");
+  StepIn in{nullptr, nullptr, pm, codes, pm->n};
+  int rc = check_step_in(b, in, cur, "step_graph_patches: bad argument");
   if (rc) return rc;
   return step_graph_impl(p, b, in, w, cur);
 }

@@ -241,7 +241,11 @@ class OnmfEngine:
 
     # ------------------------------------------------------------------ coding only
     def _cov_into(self, Xt, pool, idx, scale, n, W, Whi, Wlo, Ct, stream):
-        """Ct = minibatch @ W for a dense minibatch Xt or a minibatch by reference (pool, idx, scale)."""
+        """Ct = minibatch @ W for a dense minibatch Xt or a minibatch by reference (pool, idx, scale); a patch minibatch
+        by reference comes as pool = _Patches."""
+        if isinstance(pool, _Patches) and Xt is None:
+            _lib.cov_fused_tc_patches(pool.pm, Whi, Wlo, Ct, stream=stream)
+            return
         if self.fused_tc:
             src = Xt if Xt is not None else pool
             _lib.cov_fused_tc(src, idx if Xt is None else None, n, Whi, Wlo, Ct, scale=scale if Xt is None else 1.0, stream=stream)
@@ -271,6 +275,14 @@ class OnmfEngine:
             self._Xg = torch.empty(max(n, 1), self.d, dtype=self.dtype, device=self.device)
         if n:
             _lib.gather_rows(pool, idx, self._Xg[:n], stream=stream)
+        return self._Xg[:n]
+
+    def _dense_patches(self, src, idx, n, stream):
+        """materialise a patch minibatch (engines without the fused kernels, track_C): K1 index gather (+ widening)"""
+        if getattr(self, "_Xg", None) is None or self._Xg.shape[0] < n:
+            self._Xg = torch.empty(max(n, 1), self.d, dtype=self.dtype, device=self.device)
+        if n:
+            _lib.gather_patches_mb(src.minibatch(idx, n), self._Xg[:n], stream=stream)
         return self._Xg[:n]
 
     def sparse_code(self, Xt: torch.Tensor, W: Optional[torch.Tensor] = None, alpha=None, out=None):
@@ -334,6 +346,18 @@ class OnmfEngine:
         n = int(idx.shape[0] if idx is not None else (pool.shape[0] if n is None else n))
         return self._step(None, (pool, idx, float(scale)), t, codes, n)
 
+    def step_patches(self, src, idx: Optional[torch.Tensor], t: float, codes: Optional[torch.Tensor] = None):
+        """One minibatch of image patches BY REFERENCE: columns idx (int64, device; None = columns 0..N-1) of an
+        ImagePatches `src` (patches.py).  On the fused tensor-core path (fp32, k <= 256, no track_C) the covariance and
+        partial-sum kernels read the patches straight out of the image; every other engine gathers the minibatch into its
+        dense buffer first.  Same results, bit for bit, as step_pool on the materialised pool of the same patches."""
+        if src.d != self.d:
+            raise _lib.OnmfKernelError("step_patches: the patches have d = %d, the engine %d" % (src.d, self.d))
+        if src.engine_dtype != self.dtype:
+            raise _lib.OnmfKernelError("step_patches: %s image for a %s engine" % (src.dtype, self.dtype))
+        n = int(idx.shape[0]) if idx is not None else src.N
+        return self._step(None, _Patches(src, idx, n), t, codes, n)
+
     def step(self, Xt: Optional[torch.Tensor], t: float, codes: Optional[torch.Tensor] = None, n: Optional[int] = None):
         """One minibatch: Xt (n_local x d) are THIS rank's columns of the minibatch, t the step index
         (w = t^-beta).  Returns the local codes Ht (view, valid until the next call).
@@ -357,10 +381,11 @@ class OnmfEngine:
         self._reserve(max(n, 1))
         w = float(t) ** (-self.beta)
         cur = self._cur
-        pool, idx, scale = ref if ref is not None else (None, None, 1.0)
+        patches = isinstance(ref, _Patches)
+        pool, idx, scale = (ref, ref.idx, 1.0) if patches else ref if ref is not None else (None, None, 1.0)
         by_ref = ref is not None and self.fused_tc and self.fused and not self.track_C      # kernels read the pool in place
         if ref is not None and not by_ref:
-            Xt = self._dense(pool, idx, scale, n, main)
+            Xt = self._dense_patches(ref.src, idx, n, main) if patches else self._dense(pool, idx, scale, n, main)
             ref = None
         if self._raw_W and codes is None:
             # first minibatch against a raw initial dictionary (fp32 engine): code it with the FP64 coder, then run the
@@ -468,8 +493,10 @@ class OnmfEngine:
             raise _lib.OnmfKernelError("codes must be (n x k)")
         if Xt is not None and Xt.shape[1] != self.d:
             raise _lib.OnmfKernelError("Xt must be (n x d)")
-        mb = None
-        if ref is not None:
+        mb = pm = None
+        if isinstance(ref, _Patches):
+            pm = ref.pm
+        elif ref is not None:
             pool, idx, scale = ref
             if pool.shape[1] != self.d:
                 raise _lib.OnmfKernelError("pool must be (n_pool x d)")
@@ -483,7 +510,9 @@ class OnmfEngine:
             self._make_bufs()
         if self.world > 1:
             import torch.distributed as dist
-            if mb is not None:
+            if pm is not None:
+                self._plan.launch_patches(self._sb, pm, codes, cur)
+            elif mb is not None:
                 self._plan.launch_mb(self._sb, mb, codes, cur)
             else:
                 self._plan.launch(self._sb, Xt, codes, n, cur)
@@ -492,6 +521,8 @@ class OnmfEngine:
                 if self.track_C:
                     dist.all_reduce(self.P2, group=self.pg)
             self._plan.finish(self._sb, w, cur)
+        elif pm is not None:
+            self._plan.step_patches(self._sb, pm, codes, w, cur, graph=self.graph)
         elif mb is not None:
             self._plan.step_mb(self._sb, mb, codes, w, cur, graph=self.graph)
         elif self.graph:
@@ -589,3 +620,11 @@ class OnmfEngine:
         torch.cuda.synchronize(self.device)
         vals = self.stats.cpu().tolist()
         return dict(zip(_lib.STATS_FIELDS, vals))
+
+
+class _Patches:
+    """a patch minibatch by reference inside OnmfEngine._step: the ImagePatches, the index tensor and the C descriptor"""
+
+    def __init__(self, src, idx, n):
+        self.src, self.idx = src, idx
+        self.pm = src.minibatch(idx, n)

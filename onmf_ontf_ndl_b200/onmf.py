@@ -28,7 +28,12 @@ uses 0 (src/onmf.py:82-84).  All shipped drivers pass alpha=None.
 
 Extra keywords (not in the reference): precision ("fp32" | "fp64"), coder ("lasso_lars" | "pgd"),
 compat (None | "shipped_onmf"), track_C (maintain the d x d aggregate C even without full_code),
-process_group (data-parallel training over several GPUs, see Online_NTF; lasso_lars coder, subsample=True or False).
+process_group (data-parallel training over several GPUs, see Online_NTF; lasso_lars coder, subsample=True or False),
+keep_code (False: no (r x N) `code` matrix is kept or copied back; the code slot of train_dict's result is None).
+
+X may also be a patches.ImagePatches: the patches of one resident image by reference (lasso_lars coder only).  train_dict
+then trains on the patches at the drawn indices without ever writing the (d x N) matrix out, with the same results, bit for
+bit, and the same draws from the global RNG as on X = ImagePatches.to_matrix().
 """
 from __future__ import annotations
 
@@ -37,6 +42,7 @@ import torch
 
 from . import _host, _lib
 from .engine import OnmfEngine
+from .patches import ImagePatches
 from .parallel import default_group, shard_range
 
 DEBUG = False
@@ -62,7 +68,8 @@ class Online_NMF():
                  coder=None,
                  compat=None,
                  track_C=None,
-                 process_group=None):
+                 process_group=None,
+                 keep_code=True):
         self.X = X
         self.n_components = n_components
         self.batch_size = batch_size
@@ -79,13 +86,21 @@ class Online_NMF():
         self.history = history
         self.alpha = alpha
         self.beta = beta
-        self.code = np.zeros(shape=(n_components, X.shape[1]))
+        self.keep_code = bool(keep_code)
+        self.code = np.zeros(shape=(n_components, X.shape[1])) if self.keep_code else None
         if compat not in (None, "shipped_onmf"):
             raise ValueError("compat must be None or 'shipped_onmf'")
         self.compat = compat
         self.coder = coder if coder is not None else ("pgd" if compat == "shipped_onmf" else "lasso_lars")
         if self.coder not in ("lasso_lars", "pgd"):
             raise ValueError("coder must be 'lasso_lars' or 'pgd'")
+        if isinstance(X, ImagePatches):
+            if self.coder != "lasso_lars" or compat is not None:
+                raise ValueError("training on ImagePatches uses the lasso_lars coder with accumulating aggregates")
+            if precision is None:
+                precision = X.precision
+            elif _host.torch_dtype(precision) != X.engine_dtype:
+                raise ValueError("precision %r differs from the ImagePatches' %r" % (precision, X.precision))
         self.precision = precision
         self._dtype = _host.torch_dtype(precision)
         self.track_C = track_C
@@ -161,7 +176,8 @@ class Online_NMF():
     # -- training loop ---------------------------------------------------------------------------
     def train_dict(self, full_code=False):
         dev = _host.device()
-        X = np.asarray(self.X)
+        patches = isinstance(self.X, ImagePatches)
+        X = self.X if patches else np.asarray(self.X)
         d, n = X.shape
         r = self.n_components
         code = self.code
@@ -179,7 +195,7 @@ class Online_NMF():
             C0 = agg0[2] if (agg0 is not None and len(agg0) == 3) else None
         t0 = self.history
 
-        pool = _host.to_sample_major(X, self._dtype, dev)        # (n x d)
+        pool = None if patches else _host.to_sample_major(X, self._dtype, dev)        # (n x d)
         group, world, rank = default_group(self.process_group)
         if world > 1:
             if self.coder != "lasso_lars" or self.compat == "shipped_onmf":
@@ -193,7 +209,7 @@ class Online_NMF():
             C_init = eng.C.clone() if want_C else None
         m = self.batch_size if self.subsample else n
         lo, hi = shard_range(m, world, rank)
-        Xb = torch.empty(hi - lo, d, dtype=self._dtype, device=dev) if self.subsample else None
+        Xb = torch.empty(hi - lo, d, dtype=self._dtype, device=dev) if self.subsample and not patches else None
         # lasso coder: nothing but the minibatch draw touches the global RNG inside the loop, so all steps' indices are
         # drawn up front (same stream as src/onmf.py:212 step by step) and uploaded once; the PGD coder interleaves its
         # H0 = np.random.rand(r, n) draws (src/onmf.py:245-246) and keeps the per-step order.
@@ -203,8 +219,19 @@ class Online_NMF():
             if world > 1:
                 idx_all = _host.broadcast_indices(group, dev, idx_all)
             idx_dev = _host.upload_indices(idx_all[:, lo:hi], dev)
+        # ImagePatches without subsampling: every column each step (this rank's range of them)
+        cols = torch.arange(lo, hi, dtype=torch.int64, device=dev) if patches and not self.subsample and world > 1 else None
         for i in np.arange(1, self.iterations):
             idx = np.arange(n)
+            if patches:
+                # the patches at the drawn corners, read out of the image by the kernels (or gathered into the engine's buffer)
+                if self.subsample:
+                    idx = idx_all[i - 1]
+                Ht = eng.step_patches(X, idx_dev[i - 1] if self.subsample else cols, float(t0 + i))
+                self.history = np.float64(t0 + i) + 1
+                if code is not None:
+                    code[:, idx[lo:hi]] += _host.from_sample_major(Ht)
+                continue
             if self.subsample:
                 if idx_all is not None:
                     idx = idx_all[i - 1]
@@ -212,7 +239,8 @@ class Online_NMF():
                         # X_batch = X[:, idx] (src/onmf.py:213) by reference: the kernels read the pool rows in place
                         Ht = eng.step_pool(pool, idx_dev[i - 1], float(t0 + i))
                         self.history = np.float64(t0 + i) + 1
-                        code[:, idx[lo:hi]] += _host.from_sample_major(Ht)        # src/onmf.py:221 (this rank's columns)
+                        if code is not None:
+                            code[:, idx[lo:hi]] += _host.from_sample_major(Ht)    # src/onmf.py:221 (this rank's columns)
                         continue
                     _lib.gather_rows(pool, idx_dev[i - 1], Xb)
                 else:
@@ -227,7 +255,8 @@ class Online_NMF():
                 eng.reset_aggregates(A_init, B_init, C_init)
             Ht = self._step_device(eng, Xt, float(t0 + i))
             self.history = np.float64(t0 + i) + 1
-            code[:, idx[lo:hi]] += _host.from_sample_major(Ht)        # src/onmf.py:221 (this rank's columns)
+            if code is not None:
+                code[:, idx[lo:hi]] += _host.from_sample_major(Ht)    # src/onmf.py:221 (this rank's columns)
         Wd, Ad, Bd, Cd = eng.state()
         self.lars_stats = eng.read_stats()
         Wn, An, Bn = _host.to_numpy(Wd), _host.to_numpy(Ad), _host.to_numpy(Bd)

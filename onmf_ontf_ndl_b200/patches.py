@@ -69,6 +69,81 @@ def extract_random_patches(img, patch_size, num_patches, precision=None):
     return X if A.ndim == 2 else patches_to_tensor(X, A.shape[2])
 
 
+class ImagePatches:
+    """The data matrix X (d x N), d = p*p*C, of the p x p patches of ONE image at the corners `coords`, kept by reference:
+    the image and the corners live on the device and no patch is ever written out.  X[(r*p + c)*C + ch, j] =
+    img[y_j + r, x_j + c, ch] -- the feature order of gather_patches.  Pass it as `X` to Online_NMF, or to
+    OnmfEngine.step_patches with minibatch indices into [0, N).
+
+    img: (H x W) or (H x W x C) array or tensor.  uint8 keeps uint8 storage on the device (value = float32(stored) *
+    float32(scale), scale defaulting to 1/255, the drivers' `data / 255`; fp32 engine only); any other dtype is stored in
+    `precision` ("fp32" default, or "fp64").  A corner whose patch leaves the image stands for a NaN column."""
+
+    def __init__(self, img, patch_size, coords, scale=None, precision=None):
+        a = img.detach() if isinstance(img, torch.Tensor) else np.asarray(img)
+        if a.ndim not in (2, 3):
+            raise ValueError("img must be (H x W) or (H x W x C), got shape %s" % (tuple(a.shape),))
+        co = coords.detach().cpu().numpy() if isinstance(coords, torch.Tensor) else np.asarray(coords)
+        if co.ndim != 2 or co.shape[1] != 2:
+            raise ValueError("coords must be an (N x 2) array of top-left corners, got shape %s" % (tuple(co.shape),))
+        if co.size and not np.issubdtype(co.dtype, np.integer):
+            raise ValueError("coords must be integers, got %s" % co.dtype)
+        p = int(patch_size)
+        H, W = int(a.shape[0]), int(a.shape[1])
+        C = int(a.shape[2]) if a.ndim == 3 else 1
+        if p <= 0 or p > H or p > W or C <= 0:
+            raise ValueError("patch_size %d does not fit the image %s" % (p, (H, W)))
+        u8 = (a.dtype == torch.uint8) if isinstance(a, torch.Tensor) else (a.dtype == np.uint8)
+        if u8:
+            if precision is not None and _host.torch_dtype(precision) != torch.float32:
+                raise ValueError("a uint8 image is read by the fp32 engine only (precision must be fp32)")
+            self.dtype = torch.uint8
+            self.precision = "fp32"
+            self.scale = 1.0 / 255.0 if scale is None else float(scale)
+        else:
+            if scale is not None:
+                raise ValueError("scale applies to uint8 images only")
+            self.dtype = _host.torch_dtype(precision)
+            self.precision = "fp64" if self.dtype == torch.float64 else "fp32"
+            self.scale = 1.0
+        self.patch_size, self.H, self.W, self.C = p, H, W, C
+        self.d, self.N = p * p * C, int(co.shape[0])
+        dev = _host.device()
+        if isinstance(a, torch.Tensor):
+            t = a.to(dev, self.dtype if not u8 else torch.uint8)
+        else:
+            t = torch.from_numpy(np.ascontiguousarray(a if u8 else np.asarray(a, dtype=np.float64))).to(dev, self.dtype)
+        self.img = t.reshape(H, W, C).contiguous()
+        self.coords = torch.from_numpy(np.ascontiguousarray(co, dtype=np.int32).reshape(-1, 2)).to(dev)
+
+    @property
+    def shape(self):
+        return (self.d, self.N)
+
+    @property
+    def engine_dtype(self):
+        """dtype of the engine that reads these patches"""
+        return torch.float64 if self.dtype == torch.float64 else torch.float32
+
+    def minibatch(self, idx, n=None):
+        """the C descriptor (onmf_patch_minibatch) of columns idx (int64 device tensor) or, idx None, columns 0..n-1"""
+        n = int(idx.shape[0]) if idx is not None else (self.N if n is None else int(n))
+        return _lib.make_patch_minibatch(self.img, self.patch_size, self.coords, idx, n, self.scale)
+
+    def gather(self, idx=None, out=None, stream=None):
+        """sample-major device tensor (n x d) of columns idx (None: all N), in the engine's dtype"""
+        pm = self.minibatch(idx)
+        if out is None:
+            out = torch.empty(pm.n, self.d, dtype=self.engine_dtype, device=self.img.device)
+        if pm.n:
+            _lib.gather_patches_mb(pm, out, stream=stream)
+        return out
+
+    def to_matrix(self):
+        """the (d x N) numpy float64 data matrix these patches stand for (small cases and tests)"""
+        return _host.from_sample_major(self.gather())
+
+
 def patches_to_tensor(X, channels):
     """(k*k*C, N) HWC data matrix -> the reference's (k*k, C, N) patch tensor (a view, no arithmetic)."""
     d, n = X.shape
