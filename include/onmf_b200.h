@@ -267,19 +267,38 @@ int onmf_surrogate_fused_tc_patches(const void* Ht, const onmf_patch_minibatch* 
  *   for j in 0..k-1:  W[:,j] -= (W A[:,j] - B[j,:]^T) / (A[j,j] + 1);  W[:,j] = max(W[:,j], 0);
  *                     W[:,j] /= max(1, ||W[:,j]||_2)
  * W_in and W_out (d x k) may alias.  Three kernels, chosen by shape: one CTA (d <= 1024 and W, A within its shared memory),
- * one 16-CTA thread-block cluster (d*k up to ~0.9 M fp32 entries), a cooperative grid beyond that (onmf_update_dict_ws with a
+ * one thread-block cluster of up to 16 CTAs (d*k up to ~0.9 M fp32 entries), a cooperative grid beyond that (onmf_update_dict_ws with a
  * workspace).  Each is deterministic and gives bit-identical results on every GPU of a data-parallel run; the three differ from
  * one another in summation order (last bits).
  * ------------------------------------------------------------------------------------------- */
 int onmf_update_dict(int dtype, const void* W_in, const void* A, const void* B, int d, int k,
                      void* W_out, void* stream);
-/* Dictionaries that fit one 16-CTA cluster's shared memory (d*k up to ~0.9 M fp32 / 0.45 M fp64 entries: every BASELINE
+/* Dictionaries that fit one cluster's shared memory (up to 16 CTAs) (d*k up to ~0.9 M fp32 / 0.45 M fp64 entries: every BASELINE
  * config) are swept by one cluster with W resident in shared memory and need no workspace (the function returns 0).
  * Larger ones (joint unfoldings of big tensors) fall back to a cooperative grid with W in L2 and one grid-wide barrier
  * per atom; that path needs onmf_update_dict_workspace(dtype, d, k) bytes of scratch. */
 size_t onmf_update_dict_workspace(int dtype, int d, int k);
 int onmf_update_dict_ws(int dtype, const void* W_in, const void* A, const void* B, int d, int k,
                         void* W_out, void* workspace, size_t workspace_bytes, void* stream);
+/* The kernel and launch shape onmf_update_dict[_ws] uses for (dtype, d, k), the same decision the launcher makes.  Host
+ * only: launches nothing and needs no GPU (without one it assumes the B200's 227 KB of opt-in shared memory and 148 SMs).
+ * Depends on the environment switches ONMF_BCD_SMALL, ONMF_BCD_TPR, ONMF_BCD_REGW and ONMF_BCD_MBAR as the launcher does.
+ * ONMF_E_UNSUPPORTED when no kernel takes the shape. */
+#define ONMF_BCD_KIND_SMALL 0    /* bcd_small_kernel: one CTA, one thread per row, W and A in shared memory */
+#define ONMF_BCD_KIND_CLUSTER 1  /* bcd_kernel: a cluster of 1-16 CTAs, each with a row slab of W in shared memory */
+#define ONMF_BCD_KIND_GRID 2     /* bcd_global_kernel: cooperative grid, W in global memory (needs the workspace) */
+typedef struct {
+  int kind;              /* ONMF_BCD_KIND_* */
+  int ctas;              /* cluster size (CLUSTER), grid size (GRID), 1 (SMALL) */
+  int rows_per_cta;      /* rows of W each CTA owns */
+  int tpr;               /* lanes per row of W in the dot product (CLUSTER; 1 for SMALL, a warp for GRID) */
+  int ks;                /* row pitch of W in shared memory, in elements (SMALL, CLUSTER) */
+  int threads;           /* threads per CTA */
+  int regw;              /* CLUSTER: 1 when each lane keeps its share of its row of W in registers (fp32) */
+  int mbar;              /* CLUSTER: column-norm signalling, 0 barrier.cluster, 1 release-arrive, 2 st.async */
+  size_t smem;           /* dynamic shared memory per CTA, bytes */
+} onmf_bcd_plan;
+int onmf_update_dict_plan(int dtype, int d, int k, onmf_bcd_plan* out);
 
 /* ---------------------------------------------------------------------------------------------
  * secondary coder: row-wise projected gradient (shipped src/onmf.py:233-271 with r=None),

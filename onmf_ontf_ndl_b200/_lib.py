@@ -75,6 +75,7 @@ SIGNATURES = {
     "onmf_update_dict": (_i, [_i, _vp, _vp, _vp, _i, _i, _vp, _vp]),
     "onmf_update_dict_workspace": (_sz, [_i, _i, _i]),
     "onmf_update_dict_ws": (_i, [_i, _vp, _vp, _vp, _i, _i, _vp, _vp, _sz, _vp]),
+    "onmf_update_dict_plan": (_i, [_i, _i, _i, _vp]),
     "onmf_pgd_sweep": (_i, [_i, _vp, _vp, _i64, _i, _dbl, _i, _vp, _vp]),
     "onmf_pgd_sweep_rows": (_i, [_i, _vp, _vp, _i64, _i, _dbl, _i, _vp, _i, _i, _vp]),
     "onmf_surrogate_error": (_i, [_i, _vp, _vp, _vp, _vp, _vp, _i, _i, _vp, _vp]),
@@ -398,6 +399,25 @@ def axpby(a, x, b, y, stream=None):
 
 def update_dict_workspace(dtype, d, k):
     return int(load().onmf_update_dict_workspace(F64 if dtype == torch.float64 else F32, d, k))
+
+
+class BcdPlan(ctypes.Structure):
+    """onmf_bcd_plan (include/onmf_b200.h): the kernel and launch shape of the dictionary update for one (dtype, d, k)."""
+    _fields_ = [("kind", _i), ("ctas", _i), ("rows_per_cta", _i), ("tpr", _i), ("ks", _i), ("threads", _i), ("regw", _i),
+                ("mbar", _i), ("smem", _sz)]
+
+
+BCD_KINDS = ("small", "cluster", "grid")
+
+
+def update_dict_plan(dtype, d, k):
+    """what onmf_update_dict launches for this shape, as a dict (kind: "small" / "cluster" / "grid"); host only"""
+    p = BcdPlan()
+    _check(load().onmf_update_dict_plan(F64 if dtype == torch.float64 else F32, int(d), int(k), ctypes.byref(p)),
+           "onmf_update_dict_plan")
+    out = {f: int(getattr(p, f)) for f, _ in BcdPlan._fields_}
+    out["kind"] = BCD_KINDS[p.kind]
+    return out
 
 
 def update_dict(W, A, B, W_out, stream=None, workspace=None):

@@ -66,7 +66,8 @@ __device__ __forceinline__ void mbar_wait(uint32_t mbar, uint32_t parity) {
   } while (!ok);
 }
 
-// REGW (fp32, k % 4 == 0, 4 <= tpr, k <= 32 * tpr, <= 512 threads: the cfg5 class): every lane keeps its share of its row of W
+// REGW (fp32, k % 4 == 0, 4 <= tpr, k <= 32 * tpr, <= 512 threads, pitch ks a multiple of 4: e.g. 1024 x 128, not cfg5 --
+// see bcd_plan_of): every lane keeps its share of its row of W
 // -- up to eight 4-element chunks, chunk c = tl + tpr * i -- in REGISTERS next to the shared-memory slab (which stays the
 // master copy for W[row, j] reads and the final store).  The per-atom dot product then reads only the column of A from
 // shared memory, 16 bytes per load and the same address for every row of a warp (broadcast): 8 LDS.128 + 32 FFMA per lane
@@ -453,30 +454,6 @@ __global__ void __launch_bounds__(256) bcd_global_kernel(const T* __restrict__ W
 }
 
 template <typename T>
-static int update_dict_global_t(const T* Win, const T* A, const T* B, int d, int k, T* Wout, void* ws, size_t ws_bytes,
-                                cudaStream_t st) {
-  int dev = 0, coop = 0;
-  cudaGetDevice(&dev);
-  cudaDeviceGetAttribute(&coop, cudaDevAttrCooperativeLaunch, dev);
-  if (!coop) return fail(ONMF_E_UNSUPPORTED, "update_dict: dictionary too large for one cluster and no cooperative launch");
-  int nb = num_sms();
-  if (nb > d) nb = d;
-  int rpb = cdiv(d, nb);
-  nb = cdiv(d, rpb);
-  const size_t smem = ((size_t)k + rpb + 8) * sizeof(T);
-  if (smem > (size_t)max_smem_optin()) return fail(ONMF_E_UNSUPPORTED, "update_dict: dictionary too large (row slab exceeds shared memory)");
-  if (!ws || ws_bytes < 2 * (size_t)num_sms() * sizeof(double))
-    return fail(ONMF_E_WORKSPACE, "update_dict: this dictionary needs onmf_update_dict_ws with a workspace of onmf_update_dict_workspace bytes");
-  auto kern = bcd_global_kernel<T>;
-  ONMF_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  T* partials = (T*)ws;
-  void* args[] = {(void*)&Win, (void*)&A, (void*)&B, (void*)&Wout, (void*)&d, (void*)&k, (void*)&rpb, (void*)&partials};
-  ONMF_CUDA(cudaLaunchCooperativeKernel((void*)kern, dim3(nb), dim3(256), args, smem, st));
-  ++g_launches;
-  return ONMF_OK;
-}
-
-template <typename T>
 static bool cluster_fits(int d, int k) {
   const size_t smem_cap = (size_t)max_smem_optin() - 1024;
   const int rpc = cdiv(d, BCD_MAX_CLUSTER);
@@ -488,49 +465,105 @@ static bool cluster_fits(int d, int k) {
   return ((size_t)rpc * ks + 2 * (size_t)k + 32 + 2 * BCD_MAX_CLUSTER) * sizeof(T) + 32 + (size_t)k * 8 <= smem_cap;
 }
 
+// Every decision of the launcher in one host function (onmf_update_dict_plan exposes it): which kernel, cluster / grid
+// size, rows per CTA, lanes per row, slab pitch, register form, signalling form and dynamic shared memory.  Reads the
+// A/B switches ONMF_BCD_SMALL / _TPR / _REGW / _MBAR (once per process) and the device limits (the B200's 227 KB and 148
+// SMs when no device is visible).  Returns ONMF_E_UNSUPPORTED when no kernel takes the shape.
+template <typename T>
+static int bcd_plan_of(int d, int k, onmf_bcd_plan* p) {
+  *p = onmf_bcd_plan{};
+  if (bcd_small_fits<T>(d, k)) {
+    p->kind = ONMF_BCD_KIND_SMALL;
+    p->ctas = 1;
+    p->rows_per_cta = d;
+    p->tpr = 1;
+    p->ks = bcd_small_ks<T>(k);
+    p->threads = round_up(d, 32);
+    p->smem = bcd_small_smem<T>(d, k);
+    return ONMF_OK;
+  }
+  const size_t smem_cap = (size_t)max_smem_optin() - 1024;
+  if (cluster_fits<T>(d, k)) {
+    // smallest power-of-two cluster whose slabs fit; prefer <= 128 rows per CTA so several lanes share a row
+    for (int cs = 1; cs <= BCD_MAX_CLUSTER; cs *= 2) {
+      const int rpc = cdiv(d, cs);
+      int tpr = 32;
+      while (tpr > 1 && rpc * tpr > 512) tpr >>= 1;    // 512 threads per CTA: 16 warps to synchronise per atom (measured 9 % faster than 1024)
+      while (tpr > 1 && tpr * 2 > k) tpr >>= 1;
+      static const int tpr_cap = [] { const char* e = getenv("ONMF_BCD_TPR"); return e ? atoi(e) : 0; }();   // (experiments)
+      while (tpr_cap > 0 && tpr > tpr_cap) tpr >>= 1;
+      const int ks = round_up(k, 32) + (tpr < 32 ? tpr : 1);
+      const size_t smem = ((size_t)rpc * ks + 2 * (size_t)k + 32 + 2 * BCD_MAX_CLUSTER) * sizeof(T) + 32 + (size_t)k * 8;
+      const bool fits = smem <= smem_cap && rpc <= 1024;
+      if (!fits || (rpc > 128 && cs < 8)) continue;
+      p->kind = ONMF_BCD_KIND_CLUSTER;
+      p->ctas = cs;
+      p->rows_per_cta = rpc;
+      p->tpr = tpr;
+      p->ks = ks;
+      p->threads = min(round_up(rpc * tpr, 32), 1024);
+      static const int regw_on = [] { const char* e = getenv("ONMF_BCD_REGW"); return (e && atoi(e) == 0) ? 0 : 1; }();   // (A/B runs)
+      // the register form reads rows of the slab and the column of A (at rpc * ks) as 16-byte vectors: the pitch must be a
+      // multiple of 4 floats, which rules out tpr = 32 (odd pitch, chosen for conflict-free scalar reads)
+      p->regw = regw_on && sizeof(T) == 4 && k % 4 == 0 && tpr >= 4 && k <= 32 * tpr && p->threads <= 512 && ks % 4 == 0;
+      static const int use_mbar = [] { const char* e = getenv("ONMF_BCD_MBAR"); return e ? atoi(e) : 2; }();   // (A/B runs: 0 barrier.cluster, 1 release-arrive, 2 st.async [default])
+      p->mbar = use_mbar;
+      p->smem = smem;
+      return ONMF_OK;
+    }
+    // (a shape at the edge of one cluster's shared memory whose lane count at 512 threads needs a wider pitch than
+    // cluster_fits assumed: the cooperative grid below takes it)
+  }
+  int nb = num_sms();
+  if (nb > d) nb = d;
+  const int rpb = cdiv(d, nb);
+  p->kind = ONMF_BCD_KIND_GRID;
+  p->ctas = cdiv(d, rpb);
+  p->rows_per_cta = rpb;
+  p->tpr = 32;
+  p->ks = k;
+  p->threads = 256;
+  p->smem = ((size_t)k + rpb + 8) * sizeof(T);
+  if (p->smem > (size_t)max_smem_optin()) return fail(ONMF_E_UNSUPPORTED, "update_dict: dictionary too large (row slab exceeds shared memory)");
+  return ONMF_OK;
+}
+
 template <typename T>
 static int update_dict_t(const T* Win, const T* A, const T* B, int d, int k, T* Wout, void* ws, size_t ws_bytes, cudaStream_t st) {
-  if (bcd_small_fits<T>(d, k)) {
-    const size_t smem = bcd_small_smem<T>(d, k);
+  onmf_bcd_plan p;
+  int rc = bcd_plan_of<T>(d, k, &p);
+  if (rc) return rc;
+  if (p.kind == ONMF_BCD_KIND_SMALL) {
     auto kern = bcd_small_kernel<T>;
-    ONMF_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    kern<<<1, round_up(d, 32), smem, st>>>(Win, A, B, Wout, d, k, bcd_small_ks<T>(k), bcd_small_ka<T>(k));
+    ONMF_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p.smem));
+    kern<<<1, p.threads, p.smem, st>>>(Win, A, B, Wout, d, k, p.ks, bcd_small_ka<T>(k));
     ONMF_LAUNCH_CHECK("bcd_small_kernel");
     return ONMF_OK;
   }
-  if (!cluster_fits<T>(d, k)) return update_dict_global_t<T>(Win, A, B, d, k, Wout, ws, ws_bytes, st);
-  const size_t smem_cap = (size_t)max_smem_optin() - 1024;
-  // smallest power-of-two cluster whose slabs fit; prefer <= 128 rows per CTA so several lanes share a row
-  int cs = 1;
-  int rpc = 0, tpr = 1, ks = 0;
-  size_t smem = 0;
-  for (;; cs *= 2) {
-    if (cs > BCD_MAX_CLUSTER) return fail(ONMF_E_UNSUPPORTED, "update_dict: d*k too large for one 16-CTA cluster");
-    rpc = cdiv(d, cs);
-    tpr = 32;
-    while (tpr > 1 && rpc * tpr > 512) tpr >>= 1;    // 512 threads per CTA: 16 warps to synchronise per atom (measured 9 % faster than 1024)
-    while (tpr > 1 && tpr * 2 > k) tpr >>= 1;
-    {
-      static const int tpr_cap = [] { const char* e = getenv("ONMF_BCD_TPR"); return e ? atoi(e) : 0; }();   // (experiments)
-      while (tpr_cap > 0 && tpr > tpr_cap) tpr >>= 1;
-    }
-    ks = round_up(k, 32) + (tpr < 32 ? tpr : 1);
-    smem = ((size_t)rpc * ks + 2 * (size_t)k + 32 + 2 * BCD_MAX_CLUSTER) * sizeof(T) + 32 + (size_t)k * 8;
-    bool fits = smem <= smem_cap && rpc <= 1024;
-    if (fits && (rpc <= 128 || cs >= 8)) break;
-    if (fits && cs * 2 > BCD_MAX_CLUSTER) break;
+  if (p.kind == ONMF_BCD_KIND_GRID) {
+    int dev = 0, coop = 0;
+    cudaGetDevice(&dev);
+    cudaDeviceGetAttribute(&coop, cudaDevAttrCooperativeLaunch, dev);
+    if (!coop) return fail(ONMF_E_UNSUPPORTED, "update_dict: dictionary too large for one cluster and no cooperative launch");
+    if (!ws || ws_bytes < 2 * (size_t)num_sms() * sizeof(double))
+      return fail(ONMF_E_WORKSPACE, "update_dict: this dictionary needs onmf_update_dict_ws with a workspace of onmf_update_dict_workspace bytes");
+    auto kern = bcd_global_kernel<T>;
+    ONMF_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p.smem));
+    T* partials = (T*)ws;
+    int rpb = p.rows_per_cta;
+    void* args[] = {(void*)&Win, (void*)&A, (void*)&B, (void*)&Wout, (void*)&d, (void*)&k, (void*)&rpb, (void*)&partials};
+    ONMF_CUDA(cudaLaunchCooperativeKernel((void*)kern, dim3(p.ctas), dim3(p.threads), args, p.smem, st));
+    ++g_launches;
+    return ONMF_OK;
   }
-  int threads = round_up(rpc * tpr, 32);
-  if (threads > 1024) threads = 1024;
-  static const int regw_on = [] { const char* e = getenv("ONMF_BCD_REGW"); return (e && atoi(e) == 0) ? 0 : 1; }();   // (A/B runs)
-  const bool regw = regw_on && sizeof(T) == 4 && k % 4 == 0 && tpr >= 4 && k <= 32 * tpr && threads <= 512;
-  auto kern = regw ? bcd_kernel<T, sizeof(T) == 4> : bcd_kernel<T, false>;
-  ONMF_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  const int cs = p.ctas;
+  auto kern = p.regw ? bcd_kernel<T, sizeof(T) == 4> : bcd_kernel<T, false>;
+  ONMF_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p.smem));
   if (cs > 8) ONMF_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeNonPortableClusterSizeAllowed, 1));
   cudaLaunchConfig_t cfg = {};
   cfg.gridDim = dim3(cs);
-  cfg.blockDim = dim3(threads);
-  cfg.dynamicSmemBytes = smem;
+  cfg.blockDim = dim3(p.threads);
+  cfg.dynamicSmemBytes = p.smem;
   cfg.stream = st;
   cudaLaunchAttribute attr[1];
   attr[0].id = cudaLaunchAttributeClusterDimension;
@@ -539,8 +572,7 @@ static int update_dict_t(const T* Win, const T* A, const T* B, int d, int k, T* 
   attr[0].val.clusterDim.z = 1;
   cfg.attrs = attr;
   cfg.numAttrs = 1;
-  static const int use_mbar = [] { const char* e = getenv("ONMF_BCD_MBAR"); return e ? atoi(e) : 2; }();   // (A/B runs: 0 barrier.cluster, 1 release-arrive, 2 st.async [default])
-  ONMF_CUDA(cudaLaunchKernelEx(&cfg, kern, Win, A, B, Wout, d, k, rpc, ks, tpr, use_mbar));
+  ONMF_CUDA(cudaLaunchKernelEx(&cfg, kern, Win, A, B, Wout, d, k, p.rows_per_cta, p.ks, p.tpr, p.mbar));
   ++g_launches;
   return ONMF_OK;
 }
@@ -550,8 +582,15 @@ static int update_dict_t(const T* Win, const T* A, const T* B, int d, int k, T* 
 extern "C" size_t onmf_update_dict_workspace(int dtype, int d, int k) {
   using namespace onmf;
   if (d <= 0 || k <= 0) return 0;
-  const bool fits = dtype == ONMF_F64 ? cluster_fits<double>(d, k) : cluster_fits<float>(d, k);
-  return fits ? 0 : 2 * (size_t)num_sms() * sizeof(double);
+  onmf_bcd_plan p;
+  const int rc = dtype == ONMF_F64 ? bcd_plan_of<double>(d, k, &p) : bcd_plan_of<float>(d, k, &p);
+  return (rc == ONMF_OK && p.kind == ONMF_BCD_KIND_GRID) ? 2 * (size_t)num_sms() * sizeof(double) : 0;
+}
+
+extern "C" int onmf_update_dict_plan(int dtype, int d, int k, onmf_bcd_plan* out) {
+  using namespace onmf;
+  if (!out || d <= 0 || k <= 0 || (dtype != ONMF_F32 && dtype != ONMF_F64)) return fail(ONMF_E_ARG, "update_dict_plan: bad argument");
+  return dtype == ONMF_F64 ? bcd_plan_of<double>(d, k, out) : bcd_plan_of<float>(d, k, out);
 }
 
 extern "C" int onmf_update_dict_ws(int dtype, const void* W_in, const void* A, const void* B, int d, int k, void* W_out,
