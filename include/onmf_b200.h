@@ -324,9 +324,20 @@ int onmf_pgd_sweep_rows(int dtype, const void* G, const void* Ct, int64_t n, int
 int onmf_pgd_code_columns(int dtype, const void* G, const void* Ct, int64_t n, int k, double alpha, int sub_iter,
                           double stopping_diff, void* Ht, void* stream);
 /* overlap-averaged canvas (H x W x C) from the reconstructions R ((ny*nx) x ldr) of the p x p patches whose top-left
- * corners lie on the grid (gy*stride, gx*stride); count (H x W, may be NULL) receives the overlap counts */
+ * corners lie on the grid (gy*stride, gx*stride); count (H x W, may be NULL) receives the overlap counts.  Each pixel sums
+ * its covering patches in ascending grid order j = gy*nx + gx; pixels no patch covers get 0 and count 0.  The whole-grid
+ * call of onmf_patch_grid_accumulate. */
 int onmf_patch_grid_mean(int dtype, const void* R, int64_t ldr, int ny, int nx, int p, int stride, int C, int H,
                          int W, void* canvas, void* count, void* stream);
+/* the same mean, built from consecutive ranges of grid patches: this call adds the patches j0 <= j < j1, row j - j0 of R
+ * being the reconstruction of grid patch j.  Calls over consecutive ranges that cover [0, ny*nx), in order, give the same
+ * canvas and count bits as one onmf_patch_grid_mean call, with no memset: a pixel whose first covering patch lies in the
+ * range starts from 0, every other one continues the running sum the earlier call left in the canvas; the call holding
+ * the pixel's last covering patch divides by the count and writes it.  An uncovered pixel (y, x) is written (0, count
+ * 0) by the call holding patch min(y / stride, ny - 1) * nx + min(x / stride, nx - 1).  A call touches only canvas rows
+ * gy(j0)*stride .. gy(j1-1)*stride + p and the uncovered pixels it owns. */
+int onmf_patch_grid_accumulate(int dtype, const void* R, int64_t ldr, int ny, int nx, int p, int stride, int C, int H,
+                               int W, int64_t j0, int64_t j1, void* canvas, void* count, void* stream);
 
 /* NDL motif-adjacency patches (SURVEY.md §8f.4): Xt[j, q*kk + r] = has_edge(emb[j, q], emb[j, r]) for a CSR graph with
  * sorted neighbour lists -- replaces the k*k python has_edge loop network_reconstruction_nx.py:302-305 for a batch of

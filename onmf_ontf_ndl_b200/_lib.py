@@ -81,6 +81,7 @@ SIGNATURES = {
     "onmf_surrogate_error": (_i, [_i, _vp, _vp, _vp, _vp, _vp, _i, _i, _vp, _vp]),
     "onmf_pgd_code_columns": (_i, [_i, _vp, _vp, _i64, _i, _dbl, _i, _dbl, _vp, _vp]),
     "onmf_patch_grid_mean": (_i, [_i, _vp, _i64, _i, _i, _i, _i, _i, _i, _i, _vp, _vp, _vp]),
+    "onmf_patch_grid_accumulate": (_i, [_i, _vp, _i64, _i, _i, _i, _i, _i, _i, _i, _i64, _i64, _vp, _vp, _vp]),
     "onmf_motif_patches": (_i, [_i, _vp, _vp, _i, _vp, _i64, _i, _vp, _vp]),
     "onmf_edge_scatter_add": (_i, [_i, _vp, _i64, _vp, _i64, _i, _vp, _vp, _vp, _i64, _vp, _vp]),
     "onmf_step_plan_create": (_i, [ctypes.POINTER(_vp), _i]),
@@ -611,6 +612,26 @@ def patch_grid_mean(R, ny, nx, p, stride, C, H, W, canvas, count=None, stream=No
     _check(load().onmf_patch_grid_mean(dt(R), _ptr(R), R.stride(0), ny, nx, p, stride, C, H, W, _ptr(canvas), _ptr(count),
                                        _stream(stream)), "onmf_patch_grid_mean")
     return canvas
+
+
+def patch_grid_accumulate(R, j0, j1, ny, nx, p, stride, C, H, W, canvas, count=None, stream=None):
+    """add grid patches j0 <= j < j1 (reconstructions R[j - j0]) to the overlap mean; consecutive ranges covering the grid,
+    in order, give the bits of one patch_grid_mean call (include/onmf_b200.h)"""
+    _req(R, "R"); _req(canvas, "canvas", R.dtype)
+    if count is not None:
+        _req(count, "count", R.dtype)
+    _check(load().onmf_patch_grid_accumulate(dt(R), _ptr(R), R.stride(0), ny, nx, p, stride, C, H, W, int(j0), int(j1),
+                                             _ptr(canvas), _ptr(count), _stream(stream)), "onmf_patch_grid_accumulate")
+    return canvas
+
+
+def coder_band_floor(device=None):
+    """Fewest columns per band when a coder call is split into bands that must give the bits of one call.  The coders pick a
+    kernel variant from the number of columns n, and the variants agree only to rounding: the LARS coder takes its
+    one-column-per-warp fast tier for k <= 32 when n <= 24 x SMs and for k <= 64 when n <= 48 x SMs (csrc/lars.cu
+    launch_class, FAST_SMALL_WARPS), onmf_pgd_code_columns one thread per sample for k <= 32 when n >= 16 x SMs
+    (csrc/gather.cu).  Bands of more than 48 x SMs columns fall on the same side of all three as any larger call."""
+    return 48 * torch.cuda.get_device_properties(device).multi_processor_count + 1
 
 
 def motif_patches(rowptr, colidx, emb, out, stream=None):

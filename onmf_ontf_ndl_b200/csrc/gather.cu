@@ -403,16 +403,23 @@ __global__ void __launch_bounds__(128) pgd_columns_tps_kernel(const T* __restric
 
 // Overlap-averaged canvas from per-patch reconstructions (the running mean of image_reconstruction.py:389-392 and
 // sklearn's reconstruct_from_patches_2d): patches of size p x p (x C channels) with top-left corners on the grid
-// (gy*stride, gx*stride), gy < ny, gx < nx, stored row-major as R[(gy*nx + gx), (r*p + c)*C + ch].
-// Gather form: one thread per canvas element sums the covering patches in fixed order -> deterministic, no atomics.
+// (gy*stride, gx*stride), gy < ny, gx < nx, grid patch j = gy*nx + gx.  One call adds the patches j0 <= j < j1, whose
+// reconstructions are the rows R[(j - j0), (r*p + c)*C + ch].
+// Gather form: one thread per canvas element sums its covering patches in ascending j -> deterministic, no atomics, and
+// consecutive ranges give the bits of one call over [0, ny*nx): a pixel whose first covering patch is in the range starts
+// from 0, any other continues the running sum an earlier call left in the canvas.  The covering patches of pixel (y, x)
+// are the rectangle gy_lo..gy_hi x gx_lo..gx_hi; its last patch own = gy_hi*nx + gx_hi also names the owner of a pixel
+// no patch covers (gy_hi = min(y / stride, ny - 1), likewise gx_hi), and only the call that holds `own` writes the final
+// value (sum / count, or 0 and count 0) and the count.  Threads cover the canvas rows from y0 on that the range touches.
 template <typename T>
-__global__ void patch_grid_mean_kernel(const T* __restrict__ R, long long ldr, int ny, int nx, int p, int stride, int C, int Hh,
-                                       int Ww, T* __restrict__ canvas, T* __restrict__ count) {
+__global__ void patch_grid_accumulate_kernel(const T* __restrict__ R, long long ldr, int ny, int nx, int p, int stride, int C,
+                                             int Ww, long long j0, long long j1, int y0, long long tot, T* __restrict__ canvas,
+                                             T* __restrict__ count) {
   long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-  long long tot = (long long)Hh * Ww * C;
   if (idx >= tot) return;
   const int ch = (int)(idx % C);
-  const long long pix = idx / C;
+  const long long pix = idx / C + (long long)y0 * Ww;
+  const long long out = pix * C + ch;
   const int x = (int)(pix % Ww), y = (int)(pix / Ww);
   // grid rows gy with gy*stride <= y < gy*stride + p
   int gy_hi = y / stride;
@@ -423,20 +430,39 @@ __global__ void patch_grid_mean_kernel(const T* __restrict__ R, long long ldr, i
   if (gx_hi > nx - 1) gx_hi = nx - 1;
   int gx_lo = (x - p + stride) / stride;
   if (x - p + 1 <= 0) gx_lo = 0;
-  T acc = T(0);
-  int cnt = 0;
-  for (int gy = gy_lo; gy <= gy_hi; ++gy) {
+  const long long own = (long long)gy_hi * nx + gx_hi;
+  const bool owns = own >= j0 && own < j1;
+  if (gy_lo > gy_hi || gx_lo > gx_hi) {       // no patch covers this pixel (below / right of the grid, or stride > p)
+    if (owns) {
+      canvas[out] = T(0);
+      if (count != nullptr && ch == 0) count[pix] = T(0);
+    }
+    return;
+  }
+  const long long first = (long long)gy_lo * nx + gx_lo;
+  if (first >= j1 || own < j0) return;        // no covering patch in this range
+  T acc = first >= j0 ? T(0) : canvas[out];
+  int gy_a = gy_lo, gy_b = gy_hi;
+  if (gy_a < j0 / nx) gy_a = (int)(j0 / nx);
+  if (gy_b > (j1 - 1) / nx) gy_b = (int)((j1 - 1) / nx);
+  for (int gy = gy_a; gy <= gy_b; ++gy) {
+    const long long row = (long long)gy * nx;
     const int r = y - gy * stride;
-    if (r < 0 || r >= p) continue;
-    for (int gx = gx_lo; gx <= gx_hi; ++gx) {
+    int gx_a = gx_lo, gx_b = gx_hi;
+    if (row + gx_a < j0) gx_a = (int)(j0 - row);
+    if (row + gx_b >= j1) gx_b = (int)(j1 - 1 - row);
+    for (int gx = gx_a; gx <= gx_b; ++gx) {
       const int c = x - gx * stride;
-      if (c < 0 || c >= p) continue;
-      acc += R[(size_t)((long long)gy * nx + gx) * ldr + ((size_t)r * p + c) * C + ch];
-      ++cnt;
+      acc += R[(size_t)(row + gx - j0) * ldr + ((size_t)r * p + c) * C + ch];
     }
   }
-  canvas[idx] = cnt > 0 ? acc / T(cnt) : T(0);
-  if (count != nullptr && ch == 0) count[pix] = T(cnt);
+  if (owns) {
+    const int cnt = (gy_hi - gy_lo + 1) * (gx_hi - gx_lo + 1);
+    canvas[out] = acc / T(cnt);
+    if (count != nullptr && ch == 0) count[pix] = T(cnt);
+  } else {
+    canvas[out] = acc;
+  }
 }
 
 template <typename T>
@@ -685,18 +711,37 @@ extern "C" int onmf_pgd_code_columns(int dtype, const void* G, const void* Ct, i
   return ONMF_OK;
 }
 
+extern "C" int onmf_patch_grid_accumulate(int dtype, const void* R, int64_t ldr, int ny, int nx, int p, int stride, int C, int H,
+                                          int W, int64_t j0, int64_t j1, void* canvas, void* count, void* stream) {
+  if (!R || !canvas || ny <= 0 || nx <= 0 || p <= 0 || stride <= 0 || C <= 0 || H <= 0 || W <= 0 || ldr < (int64_t)p * p * C ||
+      j0 < 0 || j1 <= j0 || j1 > (int64_t)ny * nx)
+    return fail(ONMF_E_ARG, "patch_grid_accumulate: bad argument");
+  if (dtype != ONMF_F32 && dtype != ONMF_F64) return fail(ONMF_E_ARG, "patch_grid_accumulate: bad dtype");
+  // canvas rows of this range: those of its covering patches, gy(j0)*stride .. gy(j1-1)*stride + p, and the uncovered rows it
+  // owns: up to the next grid row's first row, or to the bottom of the canvas after the last grid row
+  const long long gy0 = j0 / nx, gy1 = (j1 - 1) / nx;
+  long long y0 = gy0 * stride, y1 = gy1 * stride + p;
+  const long long own_end = gy1 == ny - 1 ? (long long)H : (gy1 + 1) * stride;
+  if (y1 < own_end) y1 = own_end;
+  if (y1 > H) y1 = H;
+  if (y0 >= y1) return ONMF_OK;
+  cudaStream_t st = (cudaStream_t)stream;
+  const long long tot = (y1 - y0) * W * C;
+  unsigned grid = (unsigned)cdiv<long long>(tot, 256);
+  if (dtype == ONMF_F32)
+    patch_grid_accumulate_kernel<float><<<grid, 256, 0, st>>>((const float*)R, ldr, ny, nx, p, stride, C, W, j0, j1, (int)y0, tot,
+                                                               (float*)canvas, (float*)count);
+  else
+    patch_grid_accumulate_kernel<double><<<grid, 256, 0, st>>>((const double*)R, ldr, ny, nx, p, stride, C, W, j0, j1, (int)y0, tot,
+                                                                (double*)canvas, (double*)count);
+  ONMF_LAUNCH_CHECK("patch_grid_accumulate_kernel");
+  return ONMF_OK;
+}
+
 extern "C" int onmf_patch_grid_mean(int dtype, const void* R, int64_t ldr, int ny, int nx, int p, int stride, int C, int H, int W,
                                     void* canvas, void* count, void* stream) {
-  if (!R || !canvas || ny <= 0 || nx <= 0 || p <= 0 || stride <= 0 || C <= 0 || H <= 0 || W <= 0 || ldr < (int64_t)p * p * C)
-    return fail(ONMF_E_ARG, "patch_grid_mean: bad argument");
-  cudaStream_t st = (cudaStream_t)stream;
-  long long tot = (long long)H * W * C;
-  unsigned grid = (unsigned)cdiv<long long>(tot, 256);
-  if (dtype == ONMF_F32) patch_grid_mean_kernel<float><<<grid, 256, 0, st>>>((const float*)R, ldr, ny, nx, p, stride, C, H, W, (float*)canvas, (float*)count);
-  else if (dtype == ONMF_F64) patch_grid_mean_kernel<double><<<grid, 256, 0, st>>>((const double*)R, ldr, ny, nx, p, stride, C, H, W, (double*)canvas, (double*)count);
-  else return fail(ONMF_E_ARG, "patch_grid_mean: bad dtype");
-  ONMF_LAUNCH_CHECK("patch_grid_mean_kernel");
-  return ONMF_OK;
+  if (ny <= 0 || nx <= 0) return fail(ONMF_E_ARG, "patch_grid_mean: bad argument");
+  return onmf_patch_grid_accumulate(dtype, R, ldr, ny, nx, p, stride, C, H, W, 0, (int64_t)ny * nx, canvas, count, stream);
 }
 
 // ------------------------------------------------------------------------------------------------

@@ -277,12 +277,13 @@ class OnmfEngine:
             _lib.gather_rows(pool, idx, self._Xg[:n], stream=stream)
         return self._Xg[:n]
 
-    def _dense_patches(self, src, idx, n, stream):
+    def _dense_patches(self, pm, stream):
         """materialise a patch minibatch (engines without the fused kernels, track_C): K1 index gather (+ widening)"""
+        n = int(pm.n)
         if getattr(self, "_Xg", None) is None or self._Xg.shape[0] < n:
             self._Xg = torch.empty(max(n, 1), self.d, dtype=self.dtype, device=self.device)
         if n:
-            _lib.gather_patches_mb(src.minibatch(idx, n), self._Xg[:n], stream=stream)
+            _lib.gather_patches_mb(pm, self._Xg[:n], stream=stream)
         return self._Xg[:n]
 
     def sparse_code(self, Xt: torch.Tensor, W: Optional[torch.Tensor] = None, alpha=None, out=None):
@@ -295,23 +296,53 @@ class OnmfEngine:
             return Ht
         if W is None:
             self.flush()
-            W, G = self.W, self.G
-            Whi, Wlo = (self.Whi, self.Wlo) if self.use_tc else (None, None)
+            f = _Dictionary(self.W, self.G, getattr(self, "Whi", None), getattr(self, "Wlo", None), self._raw_W)
         else:
-            G = self._G_scratch
-            Whi, Wlo = (self._Whi_s, self._Wlo_s) if self.use_tc else (None, None)
-            self._derive(W, G, Whi, Wlo, torch.cuda.current_stream(self.device), use_ws=False)
-        self._cov_into(Xt, None, None, 1.0, n, W, Whi, Wlo, Ct, torch.cuda.current_stream(self.device))
-        a = self.alpha if alpha is None else alpha
-        wide = self.dtype == torch.float32 and (self._raw_W if G is self.G else
-                                                float(torch.diagonal(G).max().item()) > RAW_NORM ** 2)
-        if wide:
-            self._lars_wide(G, Ct, a, Ht, torch.cuda.current_stream(self.device))
-        else:
-            _lib.lasso_lars(G, Ct, self.d, a, Ht, self._ws_lars, max_iter=self.max_iter, stats=self._stats_ptr())
+            f = self.derive_foreign(W)
+        self._cov_into(Xt, None, None, 1.0, n, f.W, f.Whi, f.Wlo, Ct, torch.cuda.current_stream(self.device))
+        self._lars(f, Ct, alpha, Ht, -1)
         return Ht
 
-    def _lars_wide(self, G64, Ct, alpha, Ht, stream):
+    def derive_foreign(self, W: torch.Tensor):
+        """Everything the coder needs from a dictionary W (d x k, the engine's dtype) other than the engine's own: its FP64
+        Gram and, on the tensor-core path, its TF32 split, in the engine's scratch buffers; and whether it is raw (fp32
+        engine: coded in FP64, see set_state).  Returns the handle sparse_code_patches takes; it stays valid until the
+        next derive_foreign or sparse_code(Xt, W) call, which reuse the same buffers."""
+        G = self._G_scratch
+        Whi, Wlo = (self._Whi_s, self._Wlo_s) if self.use_tc else (None, None)
+        self._derive(W, G, Whi, Wlo, torch.cuda.current_stream(self.device), use_ws=False)
+        wide = self.dtype == torch.float32 and float(torch.diagonal(G).max().item()) > RAW_NORM ** 2
+        return _Dictionary(W, G, Whi, Wlo, wide)
+
+    def sparse_code_patches(self, pm, f, alpha=None, out=None, first_tier=-1):
+        """Ht (n x k) = positive lasso_lars codes of a patch minibatch BY REFERENCE (an onmf_patch_minibatch descriptor, see
+        _lib.make_patch_minibatch) against the dictionary of the handle f = derive_foreign(W).  Fused tensor-core engines
+        read the patches out of the image in the covariance kernel; every other engine gathers them into its dense buffer
+        first.  Same bits as sparse_code(<the gathered patches>, W).  first_tier: the coder's first active-set tier (0 / 1),
+        or -1 for the workspace's adaptive hint, which an earlier call may have moved."""
+        n = int(pm.n)
+        self._reserve(max(n, 1))
+        Ct = self.Ct[:n]
+        Ht = self.Ht[:n] if out is None else out
+        if n == 0:
+            return Ht
+        st = torch.cuda.current_stream(self.device)
+        if self.fused_tc:
+            self._cov_into(None, _Patches(pm), None, 1.0, n, f.W, f.Whi, f.Wlo, Ct, st)
+        else:
+            self._cov_into(self._dense_patches(pm, st), None, None, 1.0, n, f.W, f.Whi, f.Wlo, Ct, st)
+        self._lars(f, Ct, alpha, Ht, first_tier)
+        return Ht
+
+    def _lars(self, f, Ct, alpha, Ht, first_tier):
+        a = self.alpha if alpha is None else alpha
+        if f.wide:
+            self._lars_wide(f.G, Ct, a, Ht, torch.cuda.current_stream(self.device), first_tier)
+        else:
+            _lib.lasso_lars(f.G, Ct, self.d, a, Ht, self._ws_lars, max_iter=self.max_iter, stats=self._stats_ptr(),
+                            first_tier=first_tier)
+
+    def _lars_wide(self, G64, Ct, alpha, Ht, stream, first_tier=-1):
         """fp32 engine, raw dictionary: the coder in FP64 on the fp32 covariances (FP64 Gram as always), codes rounded to
         fp32.  Temporary FP64 copies of Ct / Ht live only for this call."""
         n = Ct.shape[0]
@@ -320,7 +351,8 @@ class OnmfEngine:
             Ht64 = torch.empty(n, self.k, dtype=torch.float64, device=self.device)
             ws = torch.zeros(_lib.lasso_lars_workspace(torch.float64, self.k, n), dtype=torch.uint8, device=self.device)
             _lib.convert(Ct, Ct64, stream=stream)
-            _lib.lasso_lars(G64, Ct64, self.d, alpha, Ht64, ws, max_iter=self.max_iter, stats=self._stats_ptr(), stream=stream)
+            _lib.lasso_lars(G64, Ct64, self.d, alpha, Ht64, ws, max_iter=self.max_iter, stats=self._stats_ptr(), stream=stream,
+                            first_tier=first_tier)
             _lib.convert(Ht64, Ht, stream=stream)
             for t_ in (Ct64, Ht64, ws):
                 t_.record_stream(stream)
@@ -356,7 +388,7 @@ class OnmfEngine:
         if src.engine_dtype != self.dtype:
             raise _lib.OnmfKernelError("step_patches: %s image for a %s engine" % (src.dtype, self.dtype))
         n = int(idx.shape[0]) if idx is not None else src.N
-        return self._step(None, _Patches(src, idx, n), t, codes, n)
+        return self._step(None, _Patches(src.minibatch(idx, n), idx), t, codes, n)
 
     def step(self, Xt: Optional[torch.Tensor], t: float, codes: Optional[torch.Tensor] = None, n: Optional[int] = None):
         """One minibatch: Xt (n_local x d) are THIS rank's columns of the minibatch, t the step index
@@ -385,7 +417,7 @@ class OnmfEngine:
         pool, idx, scale = (ref, ref.idx, 1.0) if patches else ref if ref is not None else (None, None, 1.0)
         by_ref = ref is not None and self.fused_tc and self.fused and not self.track_C      # kernels read the pool in place
         if ref is not None and not by_ref:
-            Xt = self._dense_patches(ref.src, idx, n, main) if patches else self._dense(pool, idx, scale, n, main)
+            Xt = self._dense_patches(ref.pm, main) if patches else self._dense(pool, idx, scale, n, main)
             ref = None
         if self._raw_W and codes is None:
             # first minibatch against a raw initial dictionary (fp32 engine): code it with the FP64 coder, then run the
@@ -623,8 +655,15 @@ class OnmfEngine:
 
 
 class _Patches:
-    """a patch minibatch by reference inside OnmfEngine._step: the ImagePatches, the index tensor and the C descriptor"""
+    """a patch minibatch by reference inside OnmfEngine: the C descriptor and the index tensor it points at"""
 
-    def __init__(self, src, idx, n):
-        self.src, self.idx = src, idx
-        self.pm = src.minibatch(idx, n)
+    def __init__(self, pm, idx=None):
+        self.pm, self.idx = pm, idx
+
+
+class _Dictionary:
+    """what the coder reads of one dictionary: W, its FP64 Gram G, the TF32 split (Whi, Wlo; None off the tensor-core
+    path) and whether the fp32 engine codes against it in FP64 (wide)"""
+
+    def __init__(self, W, G, Whi, Wlo, wide):
+        self.W, self.G, self.Whi, self.Wlo, self.wide = W, G, Whi, Wlo, bool(wide)

@@ -2,10 +2,11 @@
 
 The reference reconstructs an image by looping over a stride grid of patches in Python, coding ONE patch per call
 and painting a running-mean canvas pixel by pixel (image_reconstruction.py:358-406: `update_code_within_radius(patch,
-W, H0=None, r=None, alpha=1, sub_iter=10, stopping_diff=0.01)` at :384, running mean at :389-392).  Here the whole
-grid is one K1 gather, one Gram/covariance product, one batched coder launch (the same projected-gradient iteration
-with the reference's per-patch stopping test, or the positive LARS-lasso coder), one product Ht W^T and one
-overlap-mean kernel.  Results equal the reference loop's (same H0 stream) up to summation order.
+W, H0=None, r=None, alpha=1, sub_iter=10, stopping_diff=0.01)` at :384, running mean at :389-392).  Here the grid
+is processed in bands of patches, each one K1 gather (or a read by reference), one Gram/covariance product, one batched
+coder launch (the same projected-gradient iteration with the reference's per-patch stopping test, or the positive
+LARS-lasso coder), one product Ht W^T and one range of the overlap-mean kernel.  Results equal the reference loop's (same
+H0 stream) up to summation order, and do not depend on the band size.
 """
 from __future__ import annotations
 
@@ -22,65 +23,115 @@ def grid_shape(H, W, patch_size, recons_resolution):
     return len(range(0, H - k, s)), len(range(0, W - k, s))
 
 
+def _band_plan(n, max_band, floor):
+    """Consecutive bands [(j0, j1), ...] of near-equal size covering [0, n).  Every band holds at least `floor` columns (a
+    grid of fewer is one band): that keeps each coder call on the kernel variant the whole grid would take (see
+    _lib.coder_band_floor).  A max_band below the floor is raised to it; the floor takes precedence, so a band holds at most
+    max(max_band, 2 * floor - 1) columns."""
+    n, floor = int(n), max(int(floor), 1)
+    if n <= 0:
+        return []
+    mb = max(int(max_band), floor)
+    nb = max(1, min(-(-n // mb), n // floor))
+    base, rem = divmod(n, nb)
+    bands, j = [], 0
+    for b in range(nb):
+        m = base + (1 if b < rem else 0)
+        bands.append((j, j + m))
+        j += m
+    return bands
+
+
 def reconstruct_image(A, W, patch_size, recons_resolution=1, alpha=1, sub_iter=10, stopping_diff=0.01, coder="pgd",
-                      H0=None, precision=None, return_code=False):
-    """A: image (H x W) or (H x W x C); W: dictionary (patch_size^2 * C, r).
-    Returns (A_recons, overlap_count[, code (r x n_patches)]) as numpy float64.
+                      H0=None, precision=None, return_code=False, include_last=False, max_band=262144):
+    """A: image (H x W) or (H x W x C), or an ImagePatches (patches.py) whose resident image is used as stored (fp32, fp64,
+    or uint8 read as stored * scale; its corners are ignored, a one-channel image counts as grey); W: dictionary
+    (patch_size^2 * C, r).  Returns (A_recons, overlap_count[, code (r x n_patches)]) as numpy float64.
     coder="pgd": the reference's projected-gradient coder, one independent run per patch; H0 (r x n_patches) defaults to
     np.random.rand(r, 1) per patch in loop order, like the reference.  coder="lasso_lars": the positive lasso (the
-    commented-out alternative at image_reconstruction.py:380-383)."""
-    dev = _host.device()
-    dtype = _host.torch_dtype(precision)
-    A = np.asarray(A, dtype=np.float64)
-    squeeze = A.ndim == 2
-    A3 = A[:, :, None] if squeeze else A
-    Hh, Ww, C = A3.shape
-    k = int(patch_size)
+    commented-out alternative at image_reconstruction.py:380-383).
+    The patch grid is `range(0, H - k, stride)` per axis, the reference loop's; include_last=True takes every offset
+    0..H-k, sklearn's extract_patches_2d grid (with stride 1 and the lasso coder: the drivers' one-shot reconstruction).
+    The grid is processed in bands of at most max_band patches (gathered or read by reference, coded, multiplied by W^T and
+    added to the overlap mean band by band), so device memory is bounded by the band, not the image; the results are the
+    bits of one pass over the whole grid."""
+    if coder not in ("pgd", "lasso_lars"):
+        raise ValueError("coder must be 'pgd' or 'lasso_lars'")
+    k, s = int(patch_size), int(recons_resolution)
+    src = A if isinstance(A, patches.ImagePatches) else None
+    if src is not None:
+        if k != src.patch_size:
+            raise ValueError("patch_size %d differs from the ImagePatches' %d" % (k, src.patch_size))
+        if precision is not None and _host.torch_dtype(precision) != src.engine_dtype:
+            raise ValueError("precision %r differs from the ImagePatches' %s" % (precision, src.precision))
+        dtype = src.engine_dtype
+        Hh, Ww, C = src.H, src.W, src.C
+        squeeze = C == 1
+    else:
+        dtype = _host.torch_dtype(precision)
+        A = np.asarray(A, dtype=np.float64)
+        squeeze = A.ndim == 2
+        A3 = A[:, :, None] if squeeze else A
+        Hh, Ww, C = A3.shape
     W = np.asarray(W, dtype=np.float64)
     d, r = W.shape
     if d != k * k * C:
         raise ValueError("dictionary has %d rows, expected patch_size^2 * channels = %d" % (d, k * k * C))
-    ny, nx = grid_shape(Hh, Ww, k, recons_resolution)
+    ys = np.arange(0, Hh - k + (1 if include_last else 0), s)
+    xs = np.arange(0, Ww - k + (1 if include_last else 0), s)
+    ny, nx = len(ys), len(xs)
     n = ny * nx
-    canvas = torch.zeros(Hh, Ww, C, dtype=dtype, device=dev)
-    count = torch.zeros(Hh, Ww, dtype=dtype, device=dev)
+    if coder == "pgd" and H0 is not None:
+        H0 = np.asarray(H0, dtype=np.float64)
+        if H0.shape != (r, n):
+            raise ValueError("H0 must have shape (r, n_patches) = (%d, %d)" % (r, n))
+    dev = _host.device()
     if n == 0:
-        out = canvas.cpu().numpy().astype(np.float64)
-        return (out[:, :, 0] if squeeze else out), count.cpu().numpy().astype(np.float64)
-    gy, gx = np.meshgrid(np.arange(ny) * recons_resolution, np.arange(nx) * recons_resolution, indexing="ij")
-    coords = torch.from_numpy(np.stack([gy.reshape(-1), gx.reshape(-1)], 1).astype(np.int32)).to(dev)
-    img = _host.to_device(A3, dtype, dev)
-    Xt = torch.empty(n, d, dtype=dtype, device=dev)
-    _lib.gather_patches(img, coords, k, Xt)                                  # K1
+        out = np.zeros((Hh, Ww, C))
+        return (out[:, :, 0] if squeeze else out), np.zeros((Hh, Ww))
+    canvas = torch.empty(Hh, Ww, C, dtype=dtype, device=dev)      # every pixel is written once by its owning band
+    count = torch.empty(Hh, Ww, dtype=dtype, device=dev)
+    img, scale = (src.img, src.scale) if src is not None else (_host.to_device(A3, dtype, dev), 1.0)
     Wd = _host.to_device(W, dtype, dev)
-    if coder == "lasso_lars":
-        eng = OnmfEngine(d, r, alpha=alpha, dtype=dtype, device=dev)
-        Ht = eng.sparse_code(Xt, Wd, alpha=alpha).clone()                    # K2 + K3
-    elif coder == "pgd":
-        if H0 is None:
-            # same stream as n calls of np.random.rand(r, 1); already sample-major
-            Ht = _host.to_device(np.random.rand(n, r), dtype, dev)
-        else:
-            H0 = np.asarray(H0, dtype=np.float64)
-            if H0.shape != (r, n):
-                raise ValueError("H0 must have shape (r, n_patches) = (%d, %d)" % (r, n))
-            Ht = _host.to_sample_major(H0, dtype, dev)                        # uploaded as it is, transposed on the device
-        G = torch.empty(r, r, dtype=dtype, device=dev)
-        Ct = torch.empty(n, r, dtype=dtype, device=dev)
-        _lib.gram(Wd, G)
-        _lib.cov(Xt, Wd, Ct)
-        _lib.pgd_code_columns(G, Ct, alpha, sub_iter, stopping_diff, Ht)
-    else:
-        raise ValueError("coder must be 'pgd' or 'lasso_lars'")
     Wt = torch.empty(r, d, dtype=dtype, device=dev)
     _lib.transpose(Wd, Wt)
-    R = torch.empty(n, d, dtype=dtype, device=dev)
-    _lib.cov(Ht, Wt, R)                                                      # patch reconstructions (n x d) = Ht W^T
-    _lib.patch_grid_mean(R, ny, nx, k, recons_resolution, C, Hh, Ww, canvas, count)
+    bands = _band_plan(n, max_band, _lib.coder_band_floor(dev))
+    mmax = max(j1 - j0 for j0, j1 in bands)
+    if coder == "lasso_lars":
+        eng = OnmfEngine(d, r, alpha=alpha, dtype=dtype, device=dev)
+        f = eng.derive_foreign(Wd)                                           # Gram (+ TF32 split) once for all bands
+    else:
+        G = torch.empty(r, r, dtype=dtype, device=dev)
+        _lib.gram(Wd, G)
+        Xt = torch.empty(mmax, d, dtype=dtype, device=dev)
+        Ct = torch.empty(mmax, r, dtype=dtype, device=dev)
+    R = torch.empty(mmax, d, dtype=dtype, device=dev)
+    code = np.empty((r, n)) if return_code else None
+    for j0, j1 in bands:
+        m = j1 - j0
+        jj = np.arange(j0, j1)
+        corners = torch.from_numpy(np.stack([ys[jj // nx], xs[jj % nx]], 1).astype(np.int32)).to(dev)
+        pm = _lib.make_patch_minibatch(img, k, corners, None, m, scale)
+        if coder == "lasso_lars":
+            # first tier 0 in every band: the tier hint an earlier band leaves in the workspace must not steer this one
+            Ht = eng.sparse_code_patches(pm, f, alpha=alpha, first_tier=0)  # K1 (or by reference) + K2 + K3
+        else:
+            if H0 is None:
+                # rand(m, r) band after band is the stream of n calls of np.random.rand(r, 1); already sample-major
+                Ht = _host.to_device(np.random.rand(m, r), dtype, dev)
+            else:
+                Ht = _host.to_sample_major(H0[:, j0:j1], dtype, dev)
+            _lib.gather_patches_mb(pm, Xt[:m])                               # K1
+            _lib.cov(Xt[:m], Wd, Ct[:m])
+            _lib.pgd_code_columns(G, Ct[:m], alpha, sub_iter, stopping_diff, Ht)
+        _lib.cov(Ht, Wt, R[:m])                                              # patch reconstructions (m x d) = Ht W^T
+        _lib.patch_grid_accumulate(R[:m], j0, j1, ny, nx, k, s, C, Hh, Ww, canvas, count)
+        if return_code:
+            code[:, j0:j1] = _host.from_sample_major(Ht)
     out = canvas.cpu().numpy().astype(np.float64)
     res = (out[:, :, 0] if squeeze else out, count.cpu().numpy().astype(np.float64))
     if return_code:
-        res = res + (_host.from_sample_major(Ht),)
+        res = res + (code,)
     return res
 
 
