@@ -341,7 +341,7 @@ int onmf_patch_grid_accumulate(int dtype, const void* R, int64_t ldr, int ny, in
 
 /* NDL motif-adjacency patches (SURVEY.md §8f.4): Xt[j, q*kk + r] = has_edge(emb[j, q], emb[j, r]) for a CSR graph with
  * sorted neighbour lists -- replaces the k*k python has_edge loop network_reconstruction_nx.py:302-305 for a batch of
- * MCMC states (the walk itself stays on the host). */
+ * MCMC states (onmf_motif_chain below produces them on the device). */
 int onmf_motif_patches(int dtype, const int64_t* rowptr, const int32_t* colidx, int n_nodes, const int32_t* emb,
                        int64_t n, int kk, void* Xt, void* stream);
 
@@ -354,6 +354,32 @@ int onmf_motif_patches(int dtype, const int64_t* rowptr, const int32_t* colidx, 
 int onmf_edge_scatter_add(int dtype, const void* R, int64_t ldr, const int32_t* emb, int64_t n, int kk,
                           unsigned long long* keys, double* sums, unsigned int* counts, int64_t capacity,
                           unsigned int* failed, void* stream);
+
+/* NDL motif embeddings (the MCMC of network_reconstruction_nx.py: tree_sample, get_single_patch_glauber): n_chains independent
+ * Glauber chains of homomorphisms x of the path 0 - 1 - ... - kk-1 into a graph (x[q] ~ x[q+1]), 2 <= kk <= 32.  The graph is
+ * a CSR adjacency (rowptr n_nodes + 1 int64, colidx int32) with ascending rows, self-loops allowed; it must be symmetric.
+ * state (n_chains x kk int32) holds node positions; chain c is the global chain chain0 + c (chain0 + n_chains <= 2^32).
+ * Randomness: Philox4x32-10 (multipliers 0xD2511F53, 0xCD9E8D57, key increments 0x9E3779B9, 0xBB67AE85), key = seed (lo, hi);
+ * mulhi32(u, m) = floor(u m / 2^32), a bias of at most m / 2^32 against the uniform draw from m items.
+ *   init, draw q of chain c, counter (q, 0, c, 1):  x[0] = node mulhi32(word0, n_nodes), redrawn from counter (0, a, c, 1),
+ *         a = 1, 2, ..., while it has no neighbour; x[q] = N(x[q-1])[mulhi32(word0, deg)] for q >= 1.
+ *   Glauber step t of chain c, counter (t_lo, t_hi, c, 0):  site i = mulhi32(word0, kk); x[i] <- S[mulhi32(word1, |S|)] with
+ *         S = N(x[i-1]) & N(x[i+1]) for 0 < i < kk-1, N(x[1]) for i = 0, N(x[kk-2]) for i = kk-1, in ascending order.  S holds
+ *         the current x[i], so a step may leave the state unchanged.
+ * A trajectory is a function of (seed, chain0 + c, t) only: launch shape, n_chains, steps_per_sample and the split of a run into
+ * calls do not change it (oracle/motif_chain.py restates both entry points in numpy).
+ * onmf_motif_chain_init writes state; it reads rowptr[n_nodes] and synchronises the stream once (ONMF_E_ARG for a graph
+ * without an edge).
+ * onmf_motif_chain runs the steps step0 + 1 ... step0 + n_samples * steps_per_sample and writes out[s, c, :] (n_samples x n_chains
+ * x kk int32, row-major) = the state after step step0 + (s+1) * steps_per_sample; the final state is left in state.  It first
+ * checks every state with one small kernel and synchronises the stream to read the result: ONMF_E_ARG, before any step, for
+ * a node outside [0, n_nodes) or a consecutive pair that is not an edge.  Neither call can be captured in a CUDA graph.
+ * ONMF_E_ARG: kk < 2, a non-positive count, n_nodes > INT32_MAX; ONMF_E_UNSUPPORTED: kk > 32. */
+int onmf_motif_chain_init(const int64_t* rowptr, const int32_t* colidx, int64_t n_nodes, int kk, int64_t n_chains, int64_t chain0,
+                          uint64_t seed, int32_t* state, void* stream);
+int onmf_motif_chain(const int64_t* rowptr, const int32_t* colidx, int64_t n_nodes, int kk, int64_t n_chains, int64_t chain0,
+                     uint64_t seed, uint64_t step0, int64_t n_samples, int64_t steps_per_sample, int32_t* state, int32_t* out,
+                     void* stream);
 
 /* ---------------------------------------------------------------------------------------------
  * The fused online step: ONE host call per minibatch

@@ -30,6 +30,7 @@ class LarsStats(ctypes.Structure):
 STATS_FIELDS = [f[0] for f in LarsStats._fields_]
 
 _vp, _i, _i64, _dbl, _sz = ctypes.c_void_p, ctypes.c_int, ctypes.c_int64, ctypes.c_double, ctypes.c_size_t
+_u64 = ctypes.c_uint64
 
 # name -> (restype, argtypes); must list every symbol include/onmf_b200.h declares
 SIGNATURES = {
@@ -84,6 +85,8 @@ SIGNATURES = {
     "onmf_patch_grid_accumulate": (_i, [_i, _vp, _i64, _i, _i, _i, _i, _i, _i, _i, _i64, _i64, _vp, _vp, _vp]),
     "onmf_motif_patches": (_i, [_i, _vp, _vp, _i, _vp, _i64, _i, _vp, _vp]),
     "onmf_edge_scatter_add": (_i, [_i, _vp, _i64, _vp, _i64, _i, _vp, _vp, _vp, _i64, _vp, _vp]),
+    "onmf_motif_chain_init": (_i, [_vp, _vp, _i64, _i, _i64, _i64, _u64, _vp, _vp]),
+    "onmf_motif_chain": (_i, [_vp, _vp, _i64, _i, _i64, _i64, _u64, _u64, _i64, _i64, _vp, _vp, _vp]),
     "onmf_step_plan_create": (_i, [ctypes.POINTER(_vp), _i]),
     "onmf_step_plan_destroy": (_i, [_vp]),
     "onmf_step_plan_mark_state": (_i, [_vp, _vp]),
@@ -649,6 +652,33 @@ def edge_scatter_add(R, emb, keys, sums, counts, failed, stream=None):
     _check(load().onmf_edge_scatter_add(dt(R), _ptr(R), R.stride(0) if n else kk * kk, _ptr(emb), n, kk, _ptr(keys),
                                         _ptr(sums), _ptr(counts), keys.numel(), _ptr(failed), _stream(stream)),
            "onmf_edge_scatter_add")
+
+
+def _csr_args(rowptr, colidx, state):
+    _req(rowptr, "rowptr", torch.int64); _req(colidx, "colidx", torch.int32); _req(state, "state", torch.int32)
+    if state.dim() != 2:
+        raise OnmfKernelError("state must be (n_chains x kk)")
+    return _ptr(rowptr), _ptr(colidx), rowptr.shape[0] - 1, state.shape[1], state.shape[0]
+
+
+def motif_chain_init(rowptr, colidx, state, chain0, seed, stream=None):
+    """state (n_chains x kk int32) <- the initial path homomorphisms of chains chain0 .. chain0 + n_chains - 1"""
+    rp, ci, n_nodes, kk, n_chains = _csr_args(rowptr, colidx, state)
+    _check(load().onmf_motif_chain_init(rp, ci, n_nodes, kk, n_chains, int(chain0), int(seed), _ptr(state), _stream(stream)),
+           "onmf_motif_chain_init")
+    return state
+
+
+def motif_chain(rowptr, colidx, state, chain0, seed, step0, steps_per_sample, out, stream=None):
+    """out (n_samples x n_chains x kk int32) <- the states after steps step0 + (s+1) * steps_per_sample; state advanced in place"""
+    rp, ci, n_nodes, kk, n_chains = _csr_args(rowptr, colidx, state)
+    _req(out, "out", torch.int32)
+    if out.numel() % max(n_chains * kk, 1):
+        raise OnmfKernelError("out must hold n_samples x n_chains x kk entries")
+    _check(load().onmf_motif_chain(rp, ci, n_nodes, kk, n_chains, int(chain0), int(seed), int(step0),
+                                   out.numel() // (n_chains * kk), int(steps_per_sample), _ptr(state), _ptr(out), _stream(stream)),
+           "onmf_motif_chain")
+    return out
 
 
 # ---- fused step (csrc/step.cu) ---------------------------------------------------------------------

@@ -33,7 +33,8 @@ keep_code (False: no (r x N) `code` matrix is kept or copied back; the code slot
 
 X may also be a patches.ImagePatches: the patches of one resident image by reference (lasso_lars coder only).  train_dict
 then trains on the patches at the drawn indices without ever writing the (d x N) matrix out, with the same results, bit for
-bit, and the same draws from the global RNG as on X = ImagePatches.to_matrix().
+bit, and the same draws from the global RNG as on X = ImagePatches.to_matrix().  X may also be a patches.SamplePool: a data
+matrix already on the device in the sample-major layout, trained on in place with the results of the host matrix.
 """
 from __future__ import annotations
 
@@ -42,7 +43,7 @@ import torch
 
 from . import _host, _lib
 from .engine import OnmfEngine
-from .patches import ImagePatches
+from .patches import ImagePatches, SamplePool
 from .parallel import default_group, shard_range
 
 DEBUG = False
@@ -101,6 +102,11 @@ class Online_NMF():
                 precision = X.precision
             elif _host.torch_dtype(precision) != X.engine_dtype:
                 raise ValueError("precision %r differs from the ImagePatches' %r" % (precision, X.precision))
+        if isinstance(X, SamplePool):
+            if precision is None:
+                precision = X.precision
+            elif _host.torch_dtype(precision) != X.Xt.dtype:
+                raise ValueError("precision %r differs from the SamplePool's %r" % (precision, X.precision))
         self.precision = precision
         self._dtype = _host.torch_dtype(precision)
         self.track_C = track_C
@@ -177,7 +183,8 @@ class Online_NMF():
     def train_dict(self, full_code=False):
         dev = _host.device()
         patches = isinstance(self.X, ImagePatches)
-        X = self.X if patches else np.asarray(self.X)
+        resident = isinstance(self.X, SamplePool)
+        X = self.X if patches or resident else np.asarray(self.X)
         d, n = X.shape
         r = self.n_components
         code = self.code
@@ -195,7 +202,10 @@ class Online_NMF():
             C0 = agg0[2] if (agg0 is not None and len(agg0) == 3) else None
         t0 = self.history
 
-        pool = None if patches else _host.to_sample_major(X, self._dtype, dev)        # (n x d)
+        if resident:
+            pool = X.Xt if X.Xt.device == dev else X.Xt.to(dev)                        # (n x d), already sample-major
+        else:
+            pool = None if patches else _host.to_sample_major(X, self._dtype, dev)    # (n x d)
         group, world, rank = default_group(self.process_group)
         if world > 1:
             if self.coder != "lasso_lars" or self.compat == "shipped_onmf":

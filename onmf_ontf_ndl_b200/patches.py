@@ -168,6 +168,112 @@ def graph_to_csr(G):
     return rowptr, np.asarray(cols, dtype=np.int32), nodes
 
 
+class SamplePool:
+    """The data matrix X (d x N) held on the device in the sample-major layout: `Xt` (N x d, float32 or float64) is X^T.
+    Pass it as `X` to Online_NMF to train on device-resident columns (for instance MotifChains.patches) without a host copy;
+    the results are those of the same call on the host matrix X."""
+
+    def __init__(self, Xt):
+        if not isinstance(Xt, torch.Tensor) or not Xt.is_cuda or Xt.dim() != 2 or Xt.dtype not in (torch.float32, torch.float64):
+            raise ValueError("Xt must be an (N x d) float32 / float64 CUDA tensor")
+        self.Xt = Xt.contiguous()
+        self.precision = "fp64" if Xt.dtype == torch.float64 else "fp32"
+
+    @property
+    def shape(self):
+        return (self.Xt.shape[1], self.Xt.shape[0])
+
+
+def _symmetric_csr(G):
+    """graph_to_csr of a networkx graph or scipy adjacency, or a (rowptr, colidx[, nodes]) tuple; ValueError unless rows are
+    ascending, in range and the adjacency is symmetric (M = M^T)."""
+    if isinstance(G, tuple):
+        rowptr, colidx = np.asarray(G[0], dtype=np.int64), np.asarray(G[1], dtype=np.int32)
+        nodes = list(G[2]) if len(G) > 2 else list(range(len(rowptr) - 1))
+    else:
+        if hasattr(G, "is_directed") and G.is_directed():
+            raise ValueError("motif chains need an undirected graph (got a directed one)")
+        rowptr, colidx, nodes = graph_to_csr(G)
+    n = len(rowptr) - 1
+    if n <= 0 or len(nodes) != n or rowptr[0] != 0 or rowptr[-1] != len(colidx) or np.any(np.diff(rowptr) < 0):
+        raise ValueError("malformed CSR")
+    if n > np.iinfo(np.int32).max:
+        raise ValueError("more than 2^31 - 1 nodes")
+    rows = np.repeat(np.arange(n, dtype=np.int64), np.diff(rowptr))
+    c64 = colidx.astype(np.int64)
+    if len(c64) and (c64.min() < 0 or c64.max() >= n):
+        raise ValueError("a neighbour index is outside the graph")
+    if len(c64) > 1 and np.any((np.diff(c64) <= 0) & (rows[1:] == rows[:-1])):
+        raise ValueError("CSR rows must be strictly ascending")
+    if not np.array_equal(np.sort(rows * n + c64), np.sort(c64 * n + rows)):
+        raise ValueError("the adjacency is not symmetric (directed graphs are not supported)")
+    return rowptr, colidx, nodes
+
+
+class MotifChains:
+    """n_chains independent Glauber chains of homomorphisms of the path 0 - 1 - ... - kk-1 into an undirected graph, kept on the
+    device: the motif MCMC of the NDL drivers (network_reconstruction_nx.py tree_sample / get_single_patch_glauber) without a
+    host walk.  Every chain samples the same law; chain c's trajectory depends on (seed, c, step) only (include/onmf_b200.h,
+    onmf_motif_chain), so two sample() calls give the bits of one longer call.
+
+    G_or_csr: networkx graph, scipy sparse adjacency or a graph_to_csr tuple; it must be symmetric (ValueError otherwise).
+    state: optional (n_chains x kk) initial states in node labels; by default each chain starts from a tree sample (a root
+    uniform over the nodes with a neighbour, then uniform neighbours).  2 <= kk <= 32."""
+
+    def __init__(self, G_or_csr, kk, n_chains, seed, state=None):
+        rowptr, colidx, nodes = _symmetric_csr(G_or_csr)
+        self.kk, self.n_chains = int(kk), int(n_chains)
+        self.seed = int(seed)
+        if not 0 <= self.seed < 2 ** 64:
+            raise ValueError("seed must be in [0, 2^64)")
+        self.nodes = nodes
+        self.n_nodes = len(nodes)
+        dev = _host.device()
+        self.rowptr = torch.from_numpy(rowptr).to(dev)
+        self.colidx = torch.from_numpy(np.ascontiguousarray(colidx)).to(dev)
+        self.step = 0                                   # global Glauber steps run so far
+        if state is None:
+            self.state = torch.empty(self.n_chains, self.kk, dtype=torch.int32, device=dev)
+            _lib.motif_chain_init(self.rowptr, self.colidx, self.state, 0, self.seed)
+        else:
+            pos = {u: i for i, u in enumerate(nodes)}
+            st = np.asarray(state, dtype=object) if not isinstance(state, np.ndarray) else state
+            if st.shape != (self.n_chains, self.kk):
+                raise ValueError("state must have shape (n_chains, kk) = (%d, %d)" % (self.n_chains, self.kk))
+            try:
+                ix = np.asarray([[pos[u] for u in row] for row in st.tolist()], dtype=np.int32)
+            except (KeyError, TypeError):
+                raise ValueError("state names a node that is not in the graph")
+            self.state = torch.from_numpy(ix.reshape(self.n_chains, self.kk)).to(dev)
+        self._labels = None
+
+    def sample(self, n_samples, steps_per_sample=1):
+        """int32 device tensor (n_samples * n_chains x kk) of node positions: row s * n_chains + c is chain c after
+        steps_per_sample * (s + 1) more steps.  Advances the chains and the step counter."""
+        n_samples, sps = int(n_samples), int(steps_per_sample)
+        out = torch.empty(n_samples * self.n_chains, self.kk, dtype=torch.int32, device=self.state.device)
+        _lib.motif_chain(self.rowptr, self.colidx, self.state, 0, self.seed, self.step, sps, out)
+        self.step += n_samples * sps
+        return out
+
+    def patches(self, n_samples, steps_per_sample=1, precision=None):
+        """the sample-major (n_samples * n_chains x kk^2) motif-adjacency patches of sample(): row j, column q*kk + r =
+        has_edge(x_j[q], x_j[r])"""
+        emb = self.sample(n_samples, steps_per_sample)
+        out = torch.empty(emb.shape[0], self.kk * self.kk, dtype=_host.torch_dtype(precision), device=emb.device)
+        _lib.motif_patches(self.rowptr, self.colidx, emb, out)
+        return out
+
+    def labels(self, emb):
+        """node labels (host object array, same shape) of node positions emb (device tensor or array)"""
+        if self._labels is None:
+            self._labels = np.empty(self.n_nodes, dtype=object)
+            for i, u in enumerate(self.nodes):
+                self._labels[i] = u
+        e = emb.cpu().numpy() if isinstance(emb, torch.Tensor) else np.asarray(emb)
+        return self._labels[e]
+
+
 def motif_patches(csr, emb, precision=None, device=False):
     """emb (N x kk) node positions (indices into the CSR) of N motif embeddings -> X (kk*kk, N) with
     X[q*kk + r, j] = has_edge(emb[j, q], emb[j, r])   (network_reconstruction_nx.py:302-305, 315-329)."""

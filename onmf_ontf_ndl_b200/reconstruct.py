@@ -186,28 +186,42 @@ def reconstruct_network(G, W, embs, alpha=0, precision=None):
     The reference walks the motif MCMC and, per step, builds ONE k x k adjacency patch (`get_single_patch_glauber`,
     :331-340), codes it with `SparseCoder(transform_alpha=0, 'lasso_lars', positive_code=True)` (:466-473), forms
     patch_recons = W code (:474-475) and folds every entry into a running-mean weight of the directed edge
-    (emb[q], emb[r]) (:477-491).  The walk is sequential and stays with the caller; given its states `embs`
+    (emb[q], emb[r]) (:477-491).  The walk is the caller's (or patches.MotifChains on the device); given its states `embs`
     (recons_iter x k node labels, the embedding AFTER each update, i.e. what get_single_patch_glauber returns), this
     runs all steps at once: K1 motif patches -> K2 Gram/covariances -> K3 positive LARS at alpha -> Ht W^T -> one
     scatter kernel accumulating sum / count per directed pair.
 
-    G: networkx graph (or scipy sparse adjacency, node labels = indices); W: (k*k, r) dictionary.
+    G: networkx graph (or scipy sparse adjacency, node labels = indices); W: (k*k, r) dictionary.  embs may also be an
+    (n x k) int32 CUDA tensor of node positions (indices into G.nodes), e.g. from patches.MotifChains.sample; the patches,
+    codes and reconstructions are those of the same states given as labels, and so are the pairs and counts (the sums are
+    accumulated with FP64 atomics, whose order sets their last bits in either form).
     Returns (pairs (E x 2 node labels), weight (E,), count (E,)) sorted by (a, b) position in G.nodes -- the content
     of the reference's G_recons / G_overlap_count DiGraphs."""
     dev = _host.device()
     dtype = _host.torch_dtype(precision)
     W = np.asarray(W, dtype=np.float64)
     d, r = W.shape
-    embs = np.asarray(embs)
+    positions = isinstance(embs, torch.Tensor)
+    if positions:
+        if not embs.is_cuda or embs.dtype != torch.int32 or embs.dim() != 2:
+            raise ValueError("embs as a tensor must be an (n x k) int32 CUDA tensor of node positions")
+    else:
+        embs = np.asarray(embs)
     n, kk = embs.shape
     if kk * kk != d:
         raise ValueError("dictionary has %d rows, expected k^2 = %d" % (d, kk * kk))
     if n == 0:
         return np.empty((0, 2), dtype=object), np.empty(0), np.empty(0, dtype=np.int64)
     rowptr, colidx, nodes = patches.graph_to_csr(G)
-    pos = {u: i for i, u in enumerate(nodes)}
-    emb_i = np.asarray([[pos[u] for u in row] for row in embs.tolist()], dtype=np.int32).reshape(n, kk)
-    e = torch.from_numpy(emb_i).to(dev)
+    if positions:
+        # node positions (indices into G.nodes), e.g. MotifChains.sample: no per-entry label mapping on the host
+        e = embs.to(dev).contiguous()
+        if int(e.min()) < 0 or int(e.max()) >= len(nodes):
+            raise ValueError("embs holds a node position outside [0, %d)" % len(nodes))
+    else:
+        pos = {u: i for i, u in enumerate(nodes)}
+        emb_i = np.asarray([[pos[u] for u in row] for row in embs.tolist()], dtype=np.int32).reshape(n, kk)
+        e = torch.from_numpy(emb_i).to(dev)
     Xt = torch.empty(n, d, dtype=dtype, device=dev)
     if n:
         _lib.motif_patches(torch.from_numpy(np.asarray(rowptr, dtype=np.int64)).to(dev),
@@ -223,7 +237,9 @@ def reconstruct_network(G, W, embs, alpha=0, precision=None):
     # Table size: a table of 2 * n * k^2 slots always suffices (every entry a distinct pair), but consecutive states of the
     # Glauber walk differ in one node, so a trajectory visits about n * (2k - 1) distinct directed pairs: start there (20 bytes
     # per slot -- the worst-case table of a 10^6-state trajectory at k = 21 would be 20 GB) and grow on the kernel's
-    # "table full" report.
+    # "table full" report.  The rows of MotifChains.sample are time slices of independent chains, not one walk: each chain adds
+    # up to k^2 pairs for its first state, so few samples per chain can need up to the worst case.  The start is not restated
+    # for that ordering; the x4 growth below reaches the needed size in a few retries (log4 of k^2 / 8k, one retry at k = 21).
     worst = 2 * max(n * d, 1) + 2
     cap = 1024
     while cap < min(worst, 2 * n * 4 * kk + 2):
