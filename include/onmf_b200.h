@@ -381,6 +381,40 @@ int onmf_motif_chain(const int64_t* rowptr, const int32_t* colidx, int64_t n_nod
                      uint64_t seed, uint64_t step0, int64_t n_samples, int64_t steps_per_sample, int32_t* state, int32_t* out,
                      void* stream);
 
+/* Ising lattices (the trajectory of the Ising driver, ising_simulator.ising_update): n_chains independent checkerboard
+ * heat-bath chains of P(sigma) ~ exp(beta sum_<ij> sigma_i sigma_j) on an H x W torus (J = 1, no field); H and W even and
+ * >= 4 (a bipartite torus on which no neighbour repeats), H*W < 2^31.  state (n_chains x H x W int8, row-major) holds +-1;
+ * chain c is the global chain chain0 + c (chain0 + n_chains <= 2^32).  colour(y, x) = (y + x) & 1; the sites of one colour
+ * are numbered m = 0, 1, ... in row-major order.
+ *   sweep t (t = 1, 2, ... counts sweeps globally): colour 0, then colour 1.  Site m of colour k draws word (m & 3) of
+ *         Philox4x32-10 (the constants of onmf_motif_chain) at counter (t_lo, t_hi, chain0 + c, 2 (m >> 2) + k), key = seed
+ *         (lo, hi), and becomes +1 iff that word < thr[(s + 4) / 2], s in {-4, -2, 0, 2, 4} the sum of its four neighbours.
+ *   init: sweep t = 0 with every threshold 2^31 (independent uniform +-1).
+ * A trajectory is a function of (seed, chain0 + c, t) only: the form the plan picks, the launch shape, n_chains,
+ * sweeps_per_sample and the split of a run into calls do not change it (oracle/ising_chain.py restates both calls in numpy).
+ * onmf_ising_chain runs the sweeps sweep0 + 1 ... sweep0 + n_samples * sweeps_per_sample and writes out[s, c, :, :]
+ * (n_samples x n_chains x H x W, out_dtype ONMF_F32 or ONMF_F64, row-major) = +-1, the state after sweep
+ * sweep0 + (s+1) * sweeps_per_sample; the final state is left in state.  No address depends on a spin value, so a state
+ * that is not +-1 is not checked (its sites become +-1 as they are updated).
+ * ONMF_E_ARG, before any launch: odd or too small sides, a non-positive count, chain0 out of range, a non-finite beta,
+ * another out_dtype, or a last sweep beyond 2^64 - 1. */
+int onmf_ising_chain_init(int H, int W, int64_t n_chains, int64_t chain0, uint64_t seed, int8_t* state, void* stream);
+int onmf_ising_chain(int H, int W, int64_t n_chains, int64_t chain0, uint64_t seed, double beta, uint64_t sweep0, int64_t n_samples,
+                     int64_t sweeps_per_sample, int8_t* state, void* out, int out_dtype, void* stream);
+/* The heat-bath table thr[j] = min(floor(2^32 / (1 + exp(-2 beta (2j - 4)))), 2^32 - 1), j = 0..4: 2^32 P(+1 | s = 2j - 4);
+ * thr[2] = 2^31.  Host only.  ONMF_E_ARG for a non-finite beta. */
+int onmf_ising_thresholds(double beta, uint32_t thr[5]);
+/* The form onmf_ising_chain uses for an H x W lattice, the same decision the launcher makes.  Host only: launches nothing and
+ * needs no GPU (without one it assumes the B200's 227 KB of opt-in shared memory).  ONMF_E_ARG for a shape the chain refuses. */
+#define ONMF_ISING_FORM_SMEM 0    /* one CTA per chain (grid-striding), the lattice in shared memory for every sweep of a call */
+#define ONMF_ISING_FORM_GLOBAL 1  /* lattices above the opt-in shared memory: one launch per half-sweep over all chains */
+typedef struct {
+  int form;              /* ONMF_ISING_FORM_* */
+  int threads;           /* threads per CTA (of the sweep kernel) */
+  size_t smem;           /* dynamic shared memory per CTA, bytes (H * W for SMEM, 0 for GLOBAL) */
+} onmf_ising_plan;
+int onmf_ising_chain_plan(int H, int W, onmf_ising_plan* out);
+
 /* ---------------------------------------------------------------------------------------------
  * The fused online step: ONE host call per minibatch
  * replaces: Online_NTF.step / Online_NMF.step  (src/ontf.py:117-154, src/onmf.py:119-167) -- sparse_code, the A/B

@@ -87,6 +87,10 @@ SIGNATURES = {
     "onmf_edge_scatter_add": (_i, [_i, _vp, _i64, _vp, _i64, _i, _vp, _vp, _vp, _i64, _vp, _vp]),
     "onmf_motif_chain_init": (_i, [_vp, _vp, _i64, _i, _i64, _i64, _u64, _vp, _vp]),
     "onmf_motif_chain": (_i, [_vp, _vp, _i64, _i, _i64, _i64, _u64, _u64, _i64, _i64, _vp, _vp, _vp]),
+    "onmf_ising_chain_init": (_i, [_i, _i, _i64, _i64, _u64, _vp, _vp]),
+    "onmf_ising_chain": (_i, [_i, _i, _i64, _i64, _u64, _dbl, _u64, _i64, _i64, _vp, _vp, _i, _vp]),
+    "onmf_ising_thresholds": (_i, [_dbl, ctypes.POINTER(ctypes.c_uint32)]),
+    "onmf_ising_chain_plan": (_i, [_i, _i, _vp]),
     "onmf_step_plan_create": (_i, [ctypes.POINTER(_vp), _i]),
     "onmf_step_plan_destroy": (_i, [_vp]),
     "onmf_step_plan_mark_state": (_i, [_vp, _vp]),
@@ -678,6 +682,55 @@ def motif_chain(rowptr, colidx, state, chain0, seed, step0, steps_per_sample, ou
     _check(load().onmf_motif_chain(rp, ci, n_nodes, kk, n_chains, int(chain0), int(seed), int(step0),
                                    out.numel() // (n_chains * kk), int(steps_per_sample), _ptr(state), _ptr(out), _stream(stream)),
            "onmf_motif_chain")
+    return out
+
+
+def ising_thresholds(beta):
+    """the heat-bath table thr[0..4] (list of ints) of onmf_ising_chain at inverse temperature beta; host only"""
+    thr = (ctypes.c_uint32 * 5)()
+    _check(load().onmf_ising_thresholds(float(beta), thr), "onmf_ising_thresholds")
+    return [int(v) for v in thr]
+
+
+class IsingPlan(ctypes.Structure):
+    """onmf_ising_plan (include/onmf_b200.h): the form onmf_ising_chain uses for one lattice shape."""
+    _fields_ = [("form", _i), ("threads", _i), ("smem", _sz)]
+
+
+ISING_FORMS = ("smem", "global")
+
+
+def ising_chain_plan(H, W):
+    """what onmf_ising_chain launches for an H x W lattice, as a dict (form: "smem" / "global"); host only"""
+    p = IsingPlan()
+    _check(load().onmf_ising_chain_plan(int(H), int(W), ctypes.byref(p)), "onmf_ising_chain_plan")
+    return dict(form=ISING_FORMS[p.form], threads=int(p.threads), smem=int(p.smem))
+
+
+def _lattice_args(state):
+    _req(state, "state", torch.int8)
+    if state.dim() != 3:
+        raise OnmfKernelError("state must be (n_chains x H x W)")
+    return state.shape[0], state.shape[1], state.shape[2]
+
+
+def ising_chain_init(state, chain0, seed, stream=None):
+    """state (n_chains x H x W int8) <- the uniform +-1 initial lattices of chains chain0 .. chain0 + n_chains - 1"""
+    C, H, W = _lattice_args(state)
+    _check(load().onmf_ising_chain_init(H, W, C, int(chain0), int(seed), _ptr(state), _stream(stream)), "onmf_ising_chain_init")
+    return state
+
+
+def ising_chain(state, chain0, seed, beta, sweep0, sweeps_per_sample, out, stream=None):
+    """out (n_samples x n_chains x H x W, float32 / float64) <- the lattices after sweeps sweep0 + (s+1) * sweeps_per_sample;
+    state advanced in place"""
+    C, H, W = _lattice_args(state)
+    _req(out, "out")
+    if out.numel() % max(C * H * W, 1):
+        raise OnmfKernelError("out must hold n_samples x n_chains x H x W entries")
+    _check(load().onmf_ising_chain(H, W, C, int(chain0), int(seed), float(beta), int(sweep0), out.numel() // (C * H * W),
+                                   int(sweeps_per_sample), _ptr(state), _ptr(out), dt(out), _stream(stream)),
+           "onmf_ising_chain")
     return out
 
 

@@ -59,6 +59,22 @@ inline int max_smem_optin() {
   return n;
 }
 
+// Philox4x32-10 (Salmon et al., SC'11; the Random123 constants), the counter-based generator of the device chains
+// (motif_chain.cu, ising_chain.cu); oracle/motif_chain.py restates it.
+__device__ __forceinline__ uint4 philox4x32_10(uint4 c, uint2 k) {
+#pragma unroll
+  for (int r = 0; r < 10; ++r) {
+    if (r) { k.x += 0x9E3779B9u; k.y += 0xBB67AE85u; }
+    const unsigned lo0 = 0xD2511F53u * c.x, hi0 = __umulhi(0xD2511F53u, c.x);
+    const unsigned lo1 = 0xCD9E8D57u * c.z, hi1 = __umulhi(0xCD9E8D57u, c.z);
+    c = make_uint4(hi1 ^ c.y ^ k.x, lo1, hi0 ^ c.w ^ k.y, lo0);
+  }
+  return c;
+}
+
+// the Philox key of a 64-bit seed
+inline uint2 seed_key(uint64_t seed) { return make_uint2((unsigned)seed, (unsigned)(seed >> 32)); }
+
 template <typename T>
 __host__ __device__ inline T cdiv(T a, T b) { return (a + b - 1) / b; }
 

@@ -4,7 +4,7 @@
 // get_single_patch_glauber) run as thousands of independent chains instead of one host walk.  The chain's law depends
 // only on the graph, so every chain samples the same distribution; one warp advances one chain (lane q holds x[q]).
 //
-// Randomness is counter-based (Philox4x32-10, written here; no cuRAND), keyed by the seed and addressed by (global step,
+// Randomness is counter-based (Philox4x32-10, common.cuh; no cuRAND), keyed by the seed and addressed by (global step,
 // global chain index), so a chain's trajectory does not depend on the launch shape, on n_chains, or on how a run is split
 // into calls.  oracle/motif_chain.py restates both kernels in numpy bit for bit.
 // ------------------------------------------------------------------------------------------------
@@ -13,17 +13,6 @@
 #include "common.cuh"
 
 namespace onmf {
-
-__device__ __forceinline__ uint4 philox4x32_10(uint4 c, uint2 k) {
-#pragma unroll
-  for (int r = 0; r < 10; ++r) {
-    if (r) { k.x += 0x9E3779B9u; k.y += 0xBB67AE85u; }
-    const unsigned lo0 = 0xD2511F53u * c.x, hi0 = __umulhi(0xD2511F53u, c.x);
-    const unsigned lo1 = 0xCD9E8D57u * c.z, hi1 = __umulhi(0xCD9E8D57u, c.z);
-    c = make_uint4(hi1 ^ c.y ^ k.x, lo1, hi0 ^ c.w ^ k.y, lo0);
-  }
-  return c;
-}
 
 // tree_sample of a path, one thread per chain: root uniform over the nodes with a neighbour (redrawn from counter
 // (0, a, c, 1), a = 1, 2, ... while it has none), then x[q] uniform in N(x[q-1]) from counter (q, 0, c, 1).
@@ -144,8 +133,6 @@ __global__ void __launch_bounds__(256) motif_chain_kernel(const long long* __res
 
 __device__ unsigned g_motif_bad;     // validation flag of onmf_motif_chain (one per device; calls are serialised by a host lock)
 static std::mutex g_motif_lock;
-
-static inline uint2 seed_key(uint64_t seed) { return make_uint2((unsigned)seed, (unsigned)(seed >> 32)); }
 
 static int chain_args(const int64_t* rowptr, const int32_t* colidx, int64_t n_nodes, int kk, int64_t n_chains, int64_t chain0,
                const int32_t* state, const char* what) {

@@ -179,6 +179,13 @@ class Online_NMF():
         Ht = self._code_device(eng, Xt, eng.W)
         return eng.step_with_codes(Xt, Ht, t)
 
+    def surrogate_error(self):
+        """tr(W A W^T) - 2 tr(W B) + tr(C) of the state the last train_dict left on the device, read there (the surrogate loss
+        the Ising and network drivers plot, ising_reconstruction.py:133,164; tr(C) is 0 when C was not tracked)"""
+        if getattr(self, "_trained", None) is None:
+            raise RuntimeError("surrogate_error() reads the state of train_dict(); call train_dict() first")
+        return self._trained.surrogate_error()
+
     # -- training loop ---------------------------------------------------------------------------
     def train_dict(self, full_code=False):
         dev = _host.device()
@@ -269,6 +276,7 @@ class Online_NMF():
                 code[:, idx[lo:hi]] += _host.from_sample_major(Ht)    # src/onmf.py:221 (this rank's columns)
         Wd, Ad, Bd, Cd = eng.state()
         self.lars_stats = eng.read_stats()
+        self._trained = eng
         Wn, An, Bn = _host.to_numpy(Wd), _host.to_numpy(Ad), _host.to_numpy(Bd)
         Cn = _host.to_numpy(Cd) if want_C else None
         if self._shipped_return:

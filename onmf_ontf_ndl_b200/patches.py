@@ -274,6 +274,64 @@ class MotifChains:
         return self._labels[e]
 
 
+def frame_patch_coords(n_frames, shape, patch_size, num_patches):
+    """Corners of num_patches patches in each of n_frames frames (H x W) stacked as one (n_frames * H x W) image: frame f, in
+    order, draws sample_patch_coords(shape, patch_size, num_patches) and its rows are offset by f * H.  With one frame this
+    is the drivers' draw.  ImagePatches(frames.reshape(n_frames * H, W), patch_size, coords) then stands for the patches of
+    every frame by reference (no patch straddles two frames)."""
+    H = int(shape[0])
+    out = [sample_patch_coords(shape, patch_size, num_patches) for _ in range(int(n_frames))]
+    for f, co in enumerate(out):
+        co[:, 0] += f * H
+    return np.concatenate(out) if out else np.empty((0, 2), dtype=np.int32)
+
+
+class IsingChains:
+    """n_chains independent checkerboard heat-bath chains of the Ising model (J = 1, no field) on an H x W torus, kept on the
+    device: the lattice trajectory of the Ising driver (ising_simulator.ising_update / init_lattice) without a host loop.
+    Every chain samples the Gibbs law P(sigma) ~ exp(beta sum_<ij> sigma_i sigma_j); chain c's trajectory depends on (seed, c,
+    sweep) only (include/onmf_b200.h, onmf_ising_chain), so two sample() calls give the bits of one longer call.
+
+    shape: (H, W), both even and >= 4.  state: optional (n_chains x H x W) +-1 initial lattices; by default each chain
+    starts from independent uniform spins."""
+
+    def __init__(self, shape, beta, n_chains, seed, state=None):
+        if len(shape) != 2:
+            raise ValueError("shape must be (H, W)")
+        self.H, self.W = int(shape[0]), int(shape[1])
+        if self.H < 4 or self.W < 4 or self.H % 2 or self.W % 2 or self.H * self.W >= 2 ** 31:
+            raise ValueError("the lattice sides must be even and at least 4 (got %s)" % ((self.H, self.W),))
+        self.beta = float(beta)
+        if not np.isfinite(self.beta):
+            raise ValueError("beta must be finite")
+        self.n_chains = int(n_chains)
+        if not 0 < self.n_chains <= 2 ** 32:
+            raise ValueError("n_chains must be in [1, 2^32]")
+        self.seed = int(seed)
+        if not 0 <= self.seed < 2 ** 64:
+            raise ValueError("seed must be in [0, 2^64)")
+        self.sweep = 0                                  # global sweeps run so far
+        if state is None:
+            self.state = torch.empty(self.n_chains, self.H, self.W, dtype=torch.int8, device=_host.device())
+            _lib.ising_chain_init(self.state, 0, self.seed)
+        else:
+            st = state.detach() if isinstance(state, torch.Tensor) else torch.from_numpy(np.asarray(state))
+            if tuple(st.shape) != (self.n_chains, self.H, self.W):
+                raise ValueError("state must have shape (n_chains, H, W) = %s" % ((self.n_chains, self.H, self.W),))
+            if st.is_complex() or not bool(((st == 1) | (st == -1)).all()):
+                raise ValueError("state must hold +-1 spins")
+            self.state = st.to(_host.device(), torch.int8).contiguous()
+
+    def sample(self, n_samples, sweeps_per_sample=1, precision=None):
+        """device tensor (n_samples * n_chains x H x W) of +-1 in `precision` (fp32 default): row s * n_chains + c is chain c
+        after sweeps_per_sample * (s + 1) more sweeps.  Advances the chains and the sweep counter."""
+        n_samples, sps = int(n_samples), int(sweeps_per_sample)
+        out = torch.empty(n_samples * self.n_chains, self.H, self.W, dtype=_host.torch_dtype(precision), device=self.state.device)
+        _lib.ising_chain(self.state, 0, self.seed, self.beta, self.sweep, sps, out)
+        self.sweep += n_samples * sps
+        return out
+
+
 def motif_patches(csr, emb, precision=None, device=False):
     """emb (N x kk) node positions (indices into the CSR) of N motif embeddings -> X (kk*kk, N) with
     X[q*kk + r, j] = has_edge(emb[j, q], emb[j, r])   (network_reconstruction_nx.py:302-305, 315-329)."""
