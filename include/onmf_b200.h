@@ -380,6 +380,23 @@ int onmf_motif_chain_init(const int64_t* rowptr, const int32_t* colidx, int64_t 
 int onmf_motif_chain(const int64_t* rowptr, const int32_t* colidx, int64_t n_nodes, int kk, int64_t n_chains, int64_t chain0,
                      uint64_t seed, uint64_t step0, int64_t n_samples, int64_t steps_per_sample, int32_t* state, int32_t* out,
                      void* stream);
+/* The pivot chain of the NDL drivers (network_reconstruction_nx.py:265-278, is_glauber_dict / is_glauber_recons = False) on
+ * the same states, with the arguments, output, return codes, validation and determinism of onmf_motif_chain; its states come
+ * from onmf_motif_chain_init.  x[0] is the pivot; deg(v) = rowptr[v+1] - rowptr[v] (a self-loop counts once).  It samples the
+ * uniform law on Hom(P_kk, G), the law of the Glauber chain, and moves the whole path at once, so it mixes much faster on
+ * sparse graphs, where an interior Glauber site rarely has a second candidate.
+ *   pivot step t of chain c: word j (j = 0 ... kk) is word (j & 3) of Philox4x32-10 at counter (t_lo, t_hi, c, 2 + (j >> 2)),
+ *         key = seed (lo, hi).
+ *     proposal: y[0] = N(x[0])[mulhi32(word 0, deg x[0])]; y[q] = N(y[q-1])[mulhi32(word q, deg y[q-1])], q = 1 ... kk-1.
+ *     acceptance: num = prod_{q=1}^{kk-2} deg(y[q]), den = prod_{q=1}^{kk-2} deg(x[q]), fp64 products in that order with
+ *         round-to-nearest (1.0 for kk = 2); x <- y iff ldexp(double(word kk), -32) * den < num, otherwise x stays.  The
+ *         proposal has probability deg(x[0])^-1 prod_{q=0}^{kk-2} deg(y[q])^-1; the pivot's degrees cancel in the ratio of
+ *         the two directions, so this is the exact Metropolis-Hastings rule for the uniform law.  A proposal that reaches a
+ *         y[q], q <= kk-2, without a neighbour (only a non-symmetric graph has one) is refused.
+ * Counter words 0 (Glauber) and 1 (init) are not used, so a pivot run never shares a draw with either. */
+int onmf_motif_pivot_chain(const int64_t* rowptr, const int32_t* colidx, int64_t n_nodes, int kk, int64_t n_chains, int64_t chain0,
+                           uint64_t seed, uint64_t step0, int64_t n_samples, int64_t steps_per_sample, int32_t* state,
+                           int32_t* out, void* stream);
 
 /* Ising lattices (the trajectory of the Ising driver, ising_simulator.ising_update): n_chains independent checkerboard
  * heat-bath chains of P(sigma) ~ exp(beta sum_<ij> sigma_i sigma_j) on an H x W torus (J = 1, no field); H and W even and

@@ -87,6 +87,7 @@ SIGNATURES = {
     "onmf_edge_scatter_add": (_i, [_i, _vp, _i64, _vp, _i64, _i, _vp, _vp, _vp, _i64, _vp, _vp]),
     "onmf_motif_chain_init": (_i, [_vp, _vp, _i64, _i, _i64, _i64, _u64, _vp, _vp]),
     "onmf_motif_chain": (_i, [_vp, _vp, _i64, _i, _i64, _i64, _u64, _u64, _i64, _i64, _vp, _vp, _vp]),
+    "onmf_motif_pivot_chain": (_i, [_vp, _vp, _i64, _i, _i64, _i64, _u64, _u64, _i64, _i64, _vp, _vp, _vp]),
     "onmf_ising_chain_init": (_i, [_i, _i, _i64, _i64, _u64, _vp, _vp]),
     "onmf_ising_chain": (_i, [_i, _i, _i64, _i64, _u64, _dbl, _u64, _i64, _i64, _vp, _vp, _i, _vp]),
     "onmf_ising_thresholds": (_i, [_dbl, ctypes.POINTER(ctypes.c_uint32)]),
@@ -682,6 +683,19 @@ def motif_chain(rowptr, colidx, state, chain0, seed, step0, steps_per_sample, ou
     _check(load().onmf_motif_chain(rp, ci, n_nodes, kk, n_chains, int(chain0), int(seed), int(step0),
                                    out.numel() // (n_chains * kk), int(steps_per_sample), _ptr(state), _ptr(out), _stream(stream)),
            "onmf_motif_chain")
+    return out
+
+
+def motif_pivot_chain(rowptr, colidx, state, chain0, seed, step0, steps_per_sample, out, stream=None):
+    """motif_chain with pivot steps (onmf_motif_pivot_chain): out (n_samples x n_chains x kk int32) <- the states after pivot
+    steps step0 + (s+1) * steps_per_sample; state advanced in place"""
+    rp, ci, n_nodes, kk, n_chains = _csr_args(rowptr, colidx, state)
+    _req(out, "out", torch.int32)
+    if out.numel() % max(n_chains * kk, 1):
+        raise OnmfKernelError("out must hold n_samples x n_chains x kk entries")
+    _check(load().onmf_motif_pivot_chain(rp, ci, n_nodes, kk, n_chains, int(chain0), int(seed), int(step0),
+                                         out.numel() // (n_chains * kk), int(steps_per_sample), _ptr(state), _ptr(out),
+                                         _stream(stream)), "onmf_motif_pivot_chain")
     return out
 
 

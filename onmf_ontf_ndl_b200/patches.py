@@ -210,17 +210,27 @@ def _symmetric_csr(G):
     return rowptr, colidx, nodes
 
 
+_MOTIF_STEPS = {"glauber": _lib.motif_chain, "pivot": _lib.motif_pivot_chain}
+
+
 class MotifChains:
-    """n_chains independent Glauber chains of homomorphisms of the path 0 - 1 - ... - kk-1 into an undirected graph, kept on the
-    device: the motif MCMC of the NDL drivers (network_reconstruction_nx.py tree_sample / get_single_patch_glauber) without a
-    host walk.  Every chain samples the same law; chain c's trajectory depends on (seed, c, step) only (include/onmf_b200.h,
-    onmf_motif_chain), so two sample() calls give the bits of one longer call.
+    """n_chains independent chains of homomorphisms of the path 0 - 1 - ... - kk-1 into an undirected graph, kept on the
+    device: the motif MCMC of the NDL drivers (network_reconstruction_nx.py tree_sample / get_single_patch_glauber, or the
+    pivot chain) without a host walk.  Every chain samples the same law, the uniform law on the homomorphisms; chain c's
+    trajectory depends on (seed, c, step) only (include/onmf_b200.h, onmf_motif_chain / onmf_motif_pivot_chain), so two
+    sample() calls give the bits of one longer call.
 
     G_or_csr: networkx graph, scipy sparse adjacency or a graph_to_csr tuple; it must be symmetric (ValueError otherwise).
     state: optional (n_chains x kk) initial states in node labels; by default each chain starts from a tree sample (a root
-    uniform over the nodes with a neighbour, then uniform neighbours).  2 <= kk <= 32."""
+    uniform over the nodes with a neighbour, then uniform neighbours).  2 <= kk <= 32.
+    mcmc: "glauber" (one site redrawn per step; the drivers' is_glauber_dict / is_glauber_recons = True) or "pivot" (x[0]
+    takes a random-walk step and the rest of the path is redrawn from it, under a Metropolis-Hastings rule; = False).  The
+    pivot chain mixes much faster on sparse graphs, where an interior Glauber site rarely has a second candidate."""
 
-    def __init__(self, G_or_csr, kk, n_chains, seed, state=None):
+    def __init__(self, G_or_csr, kk, n_chains, seed, state=None, mcmc="glauber"):
+        if mcmc not in _MOTIF_STEPS:
+            raise ValueError("mcmc must be 'glauber' or 'pivot' (got %r)" % (mcmc,))
+        self.mcmc = mcmc
         rowptr, colidx, nodes = _symmetric_csr(G_or_csr)
         self.kk, self.n_chains = int(kk), int(n_chains)
         self.seed = int(seed)
@@ -231,7 +241,7 @@ class MotifChains:
         dev = _host.device()
         self.rowptr = torch.from_numpy(rowptr).to(dev)
         self.colidx = torch.from_numpy(np.ascontiguousarray(colidx)).to(dev)
-        self.step = 0                                   # global Glauber steps run so far
+        self.step = 0                                   # global steps of this chain (Glauber or pivot) run so far
         if state is None:
             self.state = torch.empty(self.n_chains, self.kk, dtype=torch.int32, device=dev)
             _lib.motif_chain_init(self.rowptr, self.colidx, self.state, 0, self.seed)
@@ -252,7 +262,7 @@ class MotifChains:
         steps_per_sample * (s + 1) more steps.  Advances the chains and the step counter."""
         n_samples, sps = int(n_samples), int(steps_per_sample)
         out = torch.empty(n_samples * self.n_chains, self.kk, dtype=torch.int32, device=self.state.device)
-        _lib.motif_chain(self.rowptr, self.colidx, self.state, 0, self.seed, self.step, sps, out)
+        _MOTIF_STEPS[self.mcmc](self.rowptr, self.colidx, self.state, 0, self.seed, self.step, sps, out)
         self.step += n_samples * sps
         return out
 
