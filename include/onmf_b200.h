@@ -98,11 +98,6 @@ int onmf_transpose(int dtype_in, int dtype_out, const void* src, int64_t rows, i
  *           from src/ontf.py:86) and A = W.T @ W, B = W.T @ X (src/onmf.py:242-243)
  * ------------------------------------------------------------------------------------------- */
 int onmf_gram(int dtype, const void* W, int d, int k, void* G /* k x k */, void* stream);
-/* same product with a workspace: the sum over d is split into up to 16 slices (fixed-order reduction) so the small
- * k x k output still fills the GPU */
-size_t onmf_gram_workspace(int dtype, int d, int k);
-int onmf_gram_ws(int dtype, const void* W, int d, int k, void* G, void* workspace, size_t workspace_bytes,
-                 void* stream);
 int onmf_cov(int dtype, const void* Xt, int64_t n, int d, const void* W, int k,
              void* Ct /* n x k */, void* stream);
 /* FP64-accumulated Gram of an fp32 (dtype_in = ONMF_F32) or fp64 dictionary: G64 (k x k doubles), optional fp32 copy G32
@@ -201,9 +196,6 @@ int onmf_surrogate_error(int dtype, const void* W, const double* G64, const void
  * ------------------------------------------------------------------------------------------- */
 int onmf_tc_supported(int k, int d);
 int onmf_split_tf32(const void* src, void* hi, void* lo, int64_t count, void* stream);
-/* fused minibatch gather + split: (hi, lo)[j, :] = split(pool[idx[j], :]) */
-int onmf_gather_rows_split(const void* pool, int64_t n_pool, int d, const int64_t* idx, int64_t n, void* hi,
-                           void* lo, void* stream);
 int onmf_cov_tc(const void* Xt_hi, const void* Xt_lo, int64_t n, int d, const void* W_hi, const void* W_lo,
                 int k, void* Ct, void* stream);
 size_t onmf_surrogate_tc_workspace(int64_t n, int k, int d);
@@ -442,7 +434,7 @@ int onmf_ising_chain_plan(int H, int W, onmf_ising_plan* out);
  *   multi GPU  : onmf_step_launch(...);  all-reduce(sum) P[cur] (and P2) on side_stream;  onmf_step_finish(..., w, cur)
  * `cur` (0/1) selects the current dictionary W[cur] (with G[cur], Whi/Wlo[cur]) and the partial-sum buffer P[cur]; the
  * step writes the new dictionary to index cur^1 and the caller flips cur afterwards.  w = t^-beta.
- * Xt (n x d) are this rank's columns; Xt = NULL (tensor-core path): Xhi/Xlo already hold the split minibatch.
+ * Xt (n x d) are this rank's columns; Xt may be NULL only when n == 0.
  * codes != NULL: externally computed codes (n x k) are aggregated instead of running the coder.
  * ------------------------------------------------------------------------------------------- */
 typedef struct onmf_step_plan onmf_step_plan;

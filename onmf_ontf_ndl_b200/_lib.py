@@ -44,8 +44,6 @@ SIGNATURES = {
     "onmf_convert": (_i, [_i, _i, _vp, _i64, _vp, _vp]),
     "onmf_widen": (_i, [_i, _vp, _i64, _dbl, _vp, _vp, _vp]),
     "onmf_gram": (_i, [_i, _vp, _i, _i, _vp, _vp]),
-    "onmf_gram_workspace": (_sz, [_i, _i, _i]),
-    "onmf_gram_ws": (_i, [_i, _vp, _i, _i, _vp, _vp, _sz, _vp]),
     "onmf_set_option": (_i, [_i, _i]),
     "onmf_get_option": (_i, [_i, ctypes.POINTER(_i)]),
     "onmf_gram_f64_workspace": (_sz, [_i, _i]),
@@ -65,7 +63,6 @@ SIGNATURES = {
     "onmf_axpby": (_i, [_i, _i64, _dbl, _vp, _dbl, _vp, _vp]),
     "onmf_tc_supported": (_i, [_i, _i]),
     "onmf_split_tf32": (_i, [_vp, _vp, _vp, _i64, _vp]),
-    "onmf_gather_rows_split": (_i, [_vp, _i64, _i, _vp, _i64, _vp, _vp, _vp]),
     "onmf_cov_tc": (_i, [_vp, _vp, _i64, _i, _vp, _vp, _i, _vp, _vp]),
     "onmf_surrogate_tc_workspace": (_sz, [_i64, _i, _i]),
     "onmf_surrogate_partial_tc": (_i, [_vp, _vp, _vp, _vp, _i64, _i, _i, _vp, _vp, _sz, _vp]),
@@ -302,19 +299,10 @@ def get_option(key):
     return int(v.value)
 
 
-def gram_workspace(dtype, d, k):
-    return int(load().onmf_gram_workspace(F64 if dtype == torch.float64 else F32, d, k))
-
-
-def gram(W, G, stream=None, workspace=None):
+def gram(W, G, stream=None):
     _req(W, "W"); _req(G, "G", W.dtype)
     d, k = W.shape
-    if workspace is not None:
-        _req(workspace, "workspace", torch.uint8)
-        _check(load().onmf_gram_ws(dt(W), _ptr(W), d, k, _ptr(G), _ptr(workspace), workspace.numel(), _stream(stream)),
-               "onmf_gram_ws")
-    else:
-        _check(load().onmf_gram(dt(W), _ptr(W), d, k, _ptr(G), _stream(stream)), "onmf_gram")
+    _check(load().onmf_gram(dt(W), _ptr(W), d, k, _ptr(G), _stream(stream)), "onmf_gram")
     return G
 
 
@@ -478,14 +466,6 @@ def tc_supported(k, d):
 def split_tf32(src, hi, lo, stream=None):
     _req(src, "src", torch.float32); _req(hi, "hi", torch.float32); _req(lo, "lo", torch.float32)
     _check(load().onmf_split_tf32(_ptr(src), _ptr(hi), _ptr(lo), src.numel(), _stream(stream)), "onmf_split_tf32")
-
-
-def gather_rows_split(pool, idx, hi, lo, stream=None):
-    _req(pool, "pool", torch.float32); _req(idx, "idx", torch.int64); _req(hi, "hi", torch.float32); _req(lo, "lo", torch.float32)
-    if idx.shape[0] == 0:
-        return
-    _check(load().onmf_gather_rows_split(_ptr(pool), pool.shape[0], pool.shape[1], _ptr(idx), idx.shape[0], _ptr(hi), _ptr(lo),
-                                         _stream(stream)), "onmf_gather_rows_split")
 
 
 def cov_tc(Xhi, Xlo, Whi, Wlo, Ct, stream=None):

@@ -343,34 +343,6 @@ extern "C" int onmf_gram(int dtype, const void* W, int d, int k, void* G, void* 
   return fail(ONMF_E_ARG, "gram: bad dtype");
 }
 
-extern "C" size_t onmf_gram_workspace(int dtype, int d, int k) {
-  if (d <= 0 || k <= 0) return 0;
-  return (size_t)16 * k * k * (dtype == ONMF_F64 ? 8 : 4) + 256;
-}
-
-// same product, split over d into up to 16 slices reduced in fixed order: fills the GPU when k x k alone is 4 tiles
-extern "C" int onmf_gram_ws(int dtype, const void* W, int d, int k, void* G, void* workspace, size_t workspace_bytes, void* stream) {
-  if (!W || !G || d <= 0 || k <= 0) return fail(ONMF_E_ARG, "gram: bad argument");
-  int splits = d / 64;
-  if (splits > 16) splits = 16;
-  if (splits < 2 || !workspace || workspace_bytes < onmf_gram_workspace(dtype, d, k)) return onmf_gram(dtype, W, d, k, G, stream);
-  cudaStream_t st = (cudaStream_t)stream;
-  const long long stride = (long long)k * k;
-  int rc;
-  if (dtype == ONMF_F32) {
-    rc = launch_gemm<float, true>((const float*)W, k, (const float*)W, k, (float*)workspace, k, k, k, d, splits, stride, st);
-    if (!rc) split_reduce_kernel<float><<<(unsigned)cdiv<long long>(stride, 256), 256, 0, st>>>((const float*)workspace, splits, stride, stride, (float*)G);
-  } else if (dtype == ONMF_F64) {
-    rc = launch_gemm<double, true>((const double*)W, k, (const double*)W, k, (double*)workspace, k, k, k, d, splits, stride, st);
-    if (!rc) split_reduce_kernel<double><<<(unsigned)cdiv<long long>(stride, 256), 256, 0, st>>>((const double*)workspace, splits, stride, stride, (double*)G);
-  } else {
-    return fail(ONMF_E_ARG, "gram: bad dtype");
-  }
-  if (rc) return rc;
-  ONMF_LAUNCH_CHECK("gram split reduce");
-  return ONMF_OK;
-}
-
 extern "C" size_t onmf_gram_f64_workspace(int d, int k) {
   if (d <= 0 || k <= 0) return 0;
   return (size_t)onmf::gram64_splits(d) * k * k * sizeof(double) + 256;

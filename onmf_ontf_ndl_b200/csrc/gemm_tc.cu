@@ -277,36 +277,6 @@ __global__ void split_tf32_kernel(const float* __restrict__ src, float* __restri
   }
 }
 
-// fused minibatch gather + split: (hi, lo)[j, :] = split(pool[idx[j], :])   (d % 4 == 0)
-__global__ void gather_rows_split_kernel(const float* __restrict__ pool, long long n_pool, int d4, const long long* __restrict__ idx,
-                                         long long n, float* __restrict__ hi, float* __restrict__ lo) {
-  const int lane = threadIdx.x & 31;
-  const long long wid = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
-  const long long nw = ((long long)gridDim.x * blockDim.x) >> 5;
-  for (long long j = wid; j < n; j += nw) {
-    const long long i = idx[j];
-    float4* h4 = reinterpret_cast<float4*>(hi) + (size_t)j * d4;
-    float4* l4 = reinterpret_cast<float4*>(lo) + (size_t)j * d4;
-    if (i < 0 || i >= n_pool) {                               // bad index: NaN row instead of an out-of-bounds read
-      const float q = __int_as_float(0x7fc00000);
-      for (int e = lane; e < d4; e += 32) { h4[e] = make_float4(q, q, q, q); l4[e] = make_float4(0.f, 0.f, 0.f, 0.f); }
-      continue;
-    }
-    const float4* src = reinterpret_cast<const float4*>(pool) + (size_t)i * d4;
-    for (int e = lane; e < d4; e += 32) {
-      float4 x = src[e];
-      float4 h, l;
-      uint32_t t;
-      asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(t) : "f"(x.x)); h.x = __uint_as_float(t); l.x = x.x - h.x;
-      asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(t) : "f"(x.y)); h.y = __uint_as_float(t); l.y = x.y - h.y;
-      asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(t) : "f"(x.z)); h.z = __uint_as_float(t); l.z = x.z - h.z;
-      asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(t) : "f"(x.w)); h.w = __uint_as_float(t); l.w = x.w - h.w;
-      h4[e] = h;
-      l4[e] = l;
-    }
-  }
-}
-
 // out[r, c] (leading dim ldo) = sum_z part[z][r][c] in fixed order
 __global__ void split_reduce2d_kernel(const float* __restrict__ part, int splits, int rows, int cols, float* __restrict__ out,
                                       long long ldo) {
@@ -446,17 +416,6 @@ extern "C" int onmf_split_tf32(const void* src, void* hi, void* lo, int64_t coun
   int grid = (int)std::min<long long>(cdiv<long long>(c4, 256), 16LL * num_sms());
   tc::split_tf32_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>((const float*)src, (float*)hi, (float*)lo, c4);
   ONMF_LAUNCH_CHECK("split_tf32_kernel");
-  return ONMF_OK;
-}
-
-extern "C" int onmf_gather_rows_split(const void* pool, int64_t n_pool, int d, const int64_t* idx, int64_t n, void* hi, void* lo,
-                                      void* stream) {
-  if (!pool || !idx || !hi || !lo || d <= 0 || d % 4 || n < 0 || n_pool <= 0) return fail(ONMF_E_ARG, "gather_rows_split: bad argument");
-  if (n == 0) return ONMF_OK;
-  int grid = (int)std::min<long long>(cdiv<long long>(n * 32, 256), 8LL * num_sms());
-  tc::gather_rows_split_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>((const float*)pool, n_pool, d / 4, (const long long*)idx, n, (float*)hi,
-                                                                       (float*)lo);
-  ONMF_LAUNCH_CHECK("gather_rows_split_kernel");
   return ONMF_OK;
 }
 

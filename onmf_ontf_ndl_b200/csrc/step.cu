@@ -142,8 +142,8 @@ static int check_buffers(const onmf_step_buffers* b, bool need_code_bufs) {
   return ONMF_OK;
 }
 
-// what one step consumes: a dense minibatch, a pool descriptor or a patch minibatch (at most one of Xt / mb / pm; none on
-// the pre-split path)
+// what one step consumes: a dense minibatch, a pool descriptor or a patch minibatch (exactly one of Xt / mb / pm when n > 0;
+// all may be null when n == 0)
 struct StepIn {
   const void* Xt;              // dense (n x d) in the engine dtype, or nullptr
   const onmf_minibatch* mb;    // descriptor (fused tensor-core path), or nullptr
@@ -187,7 +187,6 @@ static int enqueue_step(onmf_step_plan* p, const onmf_step_buffers* b, const Ste
   const size_t esz = dt == ONMF_F64 ? 8 : 4;
   const long long n = in.n;
   const bool fused = mb_fused(b, in);
-  const bool presplit = (in.Xt == nullptr && in.mb == nullptr && in.pm == nullptr);
   int rc;
   const long long l0 = g_launches;
   *blended = false;
@@ -213,7 +212,7 @@ static int enqueue_step(onmf_step_plan* p, const onmf_step_buffers* b, const Ste
   const bool fuse_blend = fused && bl.mode != 0 && !b->track_C;
   if (n > 0) {
     const void* Hcodes = in.codes ? in.codes : b->Ht;
-    if (b->use_tc && !fused && !presplit) {
+    if (b->use_tc && !fused) {
       if ((rc = onmf_split_tf32(in.Xt, b->Xhi, b->Xlo, n * d, main))) return rc;
     }
     if (!in.codes) {
@@ -288,9 +287,7 @@ static int check_step_in(const onmf_step_buffers* b, const StepIn& in, int cur, 
     if (!mb_fused(b, in)) return fail(ONMF_E_UNSUPPORTED, "step: a patch minibatch needs the fused tensor-core path (fp32, onmf_fused_tc_supported); gather it with onmf_gather_patches_mb otherwise");
     if (b->track_C) return fail(ONMF_E_UNSUPPORTED, "step: track_C needs a dense minibatch");
   }
-  const bool presplit = (in.Xt == nullptr && in.mb == nullptr && in.pm == nullptr);
-  if (in.n > 0 && presplit && !b->use_tc) return fail(ONMF_E_ARG, "step: Xt = NULL needs the tensor-core path");
-  if (in.n > 0 && presplit && b->track_C) return fail(ONMF_E_ARG, "step: track_C needs the unsplit minibatch");
+  if (in.n > 0 && !in.Xt && !in.mb && !in.pm) return fail(ONMF_E_ARG, "step: no minibatch");
   return ONMF_OK;
 }
 

@@ -358,17 +358,6 @@ class OnmfEngine:
                 t_.record_stream(stream)
 
     # ------------------------------------------------------------------ one online step
-    def step_with_codes(self, Xt, Ht, t):
-        """Same as step() but with externally computed codes Ht (n x k), e.g. from the PGD coder."""
-        return self.step(Xt, t, codes=Ht)
-
-    def split_buffers(self, n):
-        """(Xhi, Xlo) views of the engine-owned pre-split minibatch buffers (pre-split tensor-core kernels): a producer such
-        as _lib.gather_rows_split can write the minibatch straight into them and then call step(None, t, n=n)."""
-        self._reserve(max(n, 1))
-        self._need_split_buffers()
-        return self.Xhi[:n], self.Xlo[:n]
-
     def step_pool(self, pool: torch.Tensor, idx: Optional[torch.Tensor], t: float, n: Optional[int] = None, scale: float = 1.0,
                   codes: Optional[torch.Tensor] = None):
         """One minibatch BY REFERENCE: rows idx (int64, device; None = rows 0..n-1) of a resident sample-major pool, which
@@ -390,14 +379,13 @@ class OnmfEngine:
         n = int(idx.shape[0]) if idx is not None else src.N
         return self._step(None, _Patches(src.minibatch(idx, n), idx), t, codes, n)
 
-    def step(self, Xt: Optional[torch.Tensor], t: float, codes: Optional[torch.Tensor] = None, n: Optional[int] = None):
+    def step(self, Xt: torch.Tensor, t: float, codes: Optional[torch.Tensor] = None):
         """One minibatch: Xt (n_local x d) are THIS rank's columns of the minibatch, t the step index
-        (w = t^-beta).  Returns the local codes Ht (view, valid until the next call).
-        Xt=None (pre-split tensor-core kernels only): the minibatch is already in split_buffers(n)."""
-        if Xt is None and not self.use_tc:
-            raise _lib.OnmfKernelError("step(None, ...) needs the tensor-core path")
-        n = Xt.shape[0] if Xt is not None else int(n)
-        return self._step(Xt, None, t, codes, n)
+        (w = t^-beta).  codes: externally computed codes (n_local x k), e.g. from the PGD coder, aggregated instead of
+        running the coder.  Returns the local codes Ht (view, valid until the next call)."""
+        if Xt is None:
+            raise _lib.OnmfKernelError("step: no minibatch")
+        return self._step(Xt, None, t, codes, Xt.shape[0])
 
     def _step(self, Xt, ref, t, codes, n):
         main, side = self.main, self.side
@@ -409,7 +397,6 @@ class OnmfEngine:
             if ev is not None:
                 side.wait_event(ev)
                 main.wait_event(ev)
-        presplit = Xt is None and ref is None
         self._reserve(max(n, 1))
         w = float(t) ** (-self.beta)
         cur = self._cur
@@ -425,10 +412,7 @@ class OnmfEngine:
             self._raw_W = os.environ.get("ONMF_B200_WIDE_ALWAYS") == "1"      # (analysis switch: FP64 coder at every step)
             if n > 0:
                 Ct, Ht = self.Ct[:n], self.Ht[:n]
-                if presplit:
-                    _lib.cov_tc(self.Xhi[:n], self.Xlo[:n], self.Whi, self.Wlo, Ct, stream=main)
-                else:
-                    self._cov_into(Xt, pool, idx, scale, n, self.W, getattr(self, "Whi", None), getattr(self, "Wlo", None), Ct, main)
+                self._cov_into(Xt, pool, idx, scale, n, self.W, getattr(self, "Whi", None), getattr(self, "Wlo", None), Ct, main)
                 self._lars_wide(self.G, Ct, self.alpha, Ht, main)
                 codes = Ht
         if os.environ.get("ONMF_B200_WIDE_ALWAYS") != "1":
@@ -453,8 +437,7 @@ class OnmfEngine:
         if n > 0:
             if self.use_tc:
                 Xhi, Xlo = self.Xhi[:n], self.Xlo[:n]
-                if not presplit:
-                    _lib.split_tf32(Xt, Xhi, Xlo, stream=main)
+                _lib.split_tf32(Xt, Xhi, Xlo, stream=main)
             if codes is None:
                 Ct = self.Ct[:n]
                 if self.use_tc:
@@ -482,8 +465,6 @@ class OnmfEngine:
             else:
                 _lib.surrogate_partial(Ht, Xt, self.P[cur], self._ws_sur, stream=main)
             if self.track_C:
-                if presplit:
-                    raise _lib.OnmfKernelError("track_C needs the unsplit minibatch")
                 _lib.xxt_partial(Xt, self.P2, self._ws_sur, stream=main)
         else:
             with torch.cuda.stream(main):

@@ -177,7 +177,7 @@ class Online_NMF():
         if self.coder == "lasso_lars":
             return eng.step(Xt, t)
         Ht = self._code_device(eng, Xt, eng.W)
-        return eng.step_with_codes(Xt, Ht, t)
+        return eng.step(Xt, t, codes=Ht)
 
     def surrogate_error(self):
         """tr(W A W^T) - 2 tr(W B) + tr(C) of the state the last train_dict left on the device, read there (the surrogate loss

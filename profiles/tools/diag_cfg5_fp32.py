@@ -54,7 +54,7 @@ for i in range(int(g["iters"])):
     idx = torch.from_numpy(g["idx"][i].astype(np.int64)).to(dev)
     _lib.gather_rows(pool64, idx, x64); _lib.gather_rows(pool32, idx, x32)
     H64 = e64.step(x64, float(i + 1)).clone()
-    e32.step_with_codes(x32, H64.float().contiguous(), float(i + 1))
+    e32.step(x32, float(i + 1), codes=H64.float().contiguous())
     W6, A6, B6, _ = e64.state(); W3, A3, B3, _ = e32.state()
     torch.cuda.synchronize()
     err = ((W3.double() - W6).norm(dim=0) / W6.norm(dim=0))

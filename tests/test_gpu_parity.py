@@ -339,6 +339,13 @@ def test_empty_minibatch_and_loud_failures():
     W, A, B, _ = eng.state()
     assert float(A.abs().max()) == 0.0
     with pytest.raises(_lib.OnmfKernelError):
+        eng.step(None, 2.0)
+    before = [x.clone() for x in eng.state()[:3]]
+    with pytest.raises(_lib.OnmfKernelError):
+        eng._plan.step(eng._sb, None, None, 5, 0.5, eng._cur)       # n > 0 with no minibatch: refused before any launch
+    torch.cuda.synchronize()
+    assert all(torch.equal(x, y) for x, y in zip(eng.state()[:3], before))
+    with pytest.raises(_lib.OnmfKernelError):
         _lib.gram(torch.rand(4, 3), torch.empty(3, 3))               # CPU tensors are refused, not silently handled
     with pytest.raises(_lib.OnmfKernelError):
         OnmfEngine(10, 600, device=dev()).sparse_code(torch.rand(4, 10, device=dev()))   # k > 512 unsupported
@@ -600,7 +607,7 @@ def test_fused_step_equals_python_composed_schedule(monkeypatch):
                 H = None
                 for t in (1, 2, 3, 4):
                     H = eng.step(Xt, float(t)).clone()
-                eng.step_with_codes(Xt, H, 5.0)                      # aggregate externally supplied codes
+                eng.step(Xt, 5.0, codes=H)                          # aggregate externally supplied codes
                 eng.step(Xt[:0], 6.0)                                # empty shard
                 W, A, B, C = eng.state()
                 torch.cuda.synchronize()
@@ -755,9 +762,6 @@ def test_gather_index_checks_and_large_dictionary_fallbacks():
     _lib.gather_rows(pool, idx, out)
     assert torch.equal(out[0], pool[0]) and torch.equal(out[1], pool[9]) and torch.equal(out[4], pool[3])
     assert torch.isnan(out[2]).all() and torch.isnan(out[3]).all()                 # bad indices: NaN rows, no wild reads
-    hi, lo = torch.zeros(5, 8, device=dev()), torch.zeros(5, 8, device=dev())
-    _lib.gather_rows_split(pool, idx, hi, lo)
-    assert torch.isnan(hi[2]).all() and torch.equal(hi[1] + lo[1], pool[9])
     img = torch.rand(12, 9, device=dev())
     co = torch.tensor([[0, 0], [8, 5], [9, 0], [0, 6], [-1, 2]], dtype=torch.int32, device=dev())
     P = torch.zeros(5, 16, device=dev())
