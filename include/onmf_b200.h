@@ -347,6 +347,25 @@ int onmf_edge_scatter_add(int dtype, const void* R, int64_t ldr, const int32_t* 
                           unsigned long long* keys, double* sums, unsigned int* counts, int64_t capacity,
                           unsigned int* failed, void* stream);
 
+/* onmf_edge_scatter_add into a table kept across calls (a streamed reconstruction adds one band of states per call).  Same
+ * arguments, table layout and fill values; in addition *claimed (device uint64, accumulated into, never reset) += the slots
+ * this call newly took, i.e. the number of new distinct pairs.  The caller reads it to keep the load <= 1/2: before a call
+ * of n states it makes sure capacity >= 2 (claimed + n kk^2), growing the table with onmf_edge_table_grow.  claimed must
+ * not be NULL. */
+int onmf_edge_table_add(int dtype, const void* R, int64_t ldr, const int32_t* emb, int64_t n, int kk,
+                        unsigned long long* keys, double* sums, unsigned int* counts, int64_t capacity,
+                        unsigned long long* claimed, unsigned int* failed, void* stream);
+
+/* Move every occupied slot (key != ~0) of an edge table (keys, sums, counts; capacity slots) into an empty table of
+ * new_capacity slots (keys filled with 0xFF bytes, sums / counts zeroed by the caller), at the slot the new capacity's
+ * probe sequence gives it.  One thread per old slot; keys are unique, so each (key, sum, count) triple is moved, not
+ * re-added, and is bit-identical afterwards.  The old table is not modified.  Both capacities must be powers of two and
+ * new_capacity > capacity; otherwise, or for a NULL pointer, ONMF_E_ARG before any launch.  *failed (device uint32,
+ * accumulated into) counts keys that found no free slot, which cannot happen while the old table's load is <= 1/2. */
+int onmf_edge_table_grow(const unsigned long long* keys, const double* sums, const unsigned int* counts, int64_t capacity,
+                         unsigned long long* new_keys, double* new_sums, unsigned int* new_counts, int64_t new_capacity,
+                         unsigned int* failed, void* stream);
+
 /* NDL motif embeddings (the MCMC of network_reconstruction_nx.py: tree_sample, get_single_patch_glauber): n_chains independent
  * Glauber chains of homomorphisms x of the path 0 - 1 - ... - kk-1 into a graph (x[q] ~ x[q+1]), 2 <= kk <= 32.  The graph is
  * a CSR adjacency (rowptr n_nodes + 1 int64, colidx int32) with ascending rows, self-loops allowed; it must be symmetric.

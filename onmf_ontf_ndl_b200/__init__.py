@@ -9,7 +9,8 @@ include/onmf_b200.h).  There is no CPU fallback.
 from .onmf import Online_NMF, update_code_within_radius  # noqa: F401
 from .ontf import Online_NTF  # noqa: F401
 from .engine import OnmfEngine  # noqa: F401
-from .reconstruct import reconstruct_from_patches_2d, reconstruct_image, reconstruct_network  # noqa: F401
+from .reconstruct import reconstruct_from_patches_2d, reconstruct_image, reconstruct_network, \
+    reconstruct_network_chains  # noqa: F401
 
 __all__ = ["Online_NMF", "Online_NTF", "update_code_within_radius", "OnmfEngine", "reconstruct_image",
-           "reconstruct_network", "reconstruct_from_patches_2d"]
+           "reconstruct_network", "reconstruct_network_chains", "reconstruct_from_patches_2d"]

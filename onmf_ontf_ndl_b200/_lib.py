@@ -82,6 +82,8 @@ SIGNATURES = {
     "onmf_patch_grid_accumulate": (_i, [_i, _vp, _i64, _i, _i, _i, _i, _i, _i, _i, _i64, _i64, _vp, _vp, _vp]),
     "onmf_motif_patches": (_i, [_i, _vp, _vp, _i, _vp, _i64, _i, _vp, _vp]),
     "onmf_edge_scatter_add": (_i, [_i, _vp, _i64, _vp, _i64, _i, _vp, _vp, _vp, _i64, _vp, _vp]),
+    "onmf_edge_table_add": (_i, [_i, _vp, _i64, _vp, _i64, _i, _vp, _vp, _vp, _i64, _vp, _vp, _vp]),
+    "onmf_edge_table_grow": (_i, [_vp, _vp, _vp, _i64, _vp, _vp, _vp, _i64, _vp, _vp]),
     "onmf_motif_chain_init": (_i, [_vp, _vp, _i64, _i, _i64, _i64, _u64, _vp, _vp]),
     "onmf_motif_chain": (_i, [_vp, _vp, _i64, _i, _i64, _i64, _u64, _u64, _i64, _i64, _vp, _vp, _vp]),
     "onmf_motif_pivot_chain": (_i, [_vp, _vp, _i64, _i, _i64, _i64, _u64, _u64, _i64, _i64, _vp, _vp, _vp]),
@@ -637,6 +639,30 @@ def edge_scatter_add(R, emb, keys, sums, counts, failed, stream=None):
     _check(load().onmf_edge_scatter_add(dt(R), _ptr(R), R.stride(0) if n else kk * kk, _ptr(emb), n, kk, _ptr(keys),
                                         _ptr(sums), _ptr(counts), keys.numel(), _ptr(failed), _stream(stream)),
            "onmf_edge_scatter_add")
+
+
+def edge_table_add(R, emb, keys, sums, counts, claimed, failed, stream=None):
+    """edge_scatter_add into a table that is kept across calls; claimed (int64, 1) += the slots this call newly took"""
+    _req(R, "R"); _req(emb, "emb", torch.int32); _req(keys, "keys", torch.int64); _req(sums, "sums", torch.float64)
+    _req(counts, "counts", torch.int32); _req(claimed, "claimed", torch.int64); _req(failed, "failed", torch.int32)
+    n, kk = emb.shape
+    _check(load().onmf_edge_table_add(dt(R), _ptr(R), R.stride(0) if n else kk * kk, _ptr(emb), n, kk, _ptr(keys),
+                                      _ptr(sums), _ptr(counts), keys.numel(), _ptr(claimed), _ptr(failed), _stream(stream)),
+           "onmf_edge_table_add")
+
+
+def edge_table_grow(keys, sums, counts, new_keys, new_sums, new_counts, failed, stream=None):
+    """move every occupied slot of (keys, sums, counts) into the larger, empty table (new_keys, new_sums, new_counts)"""
+    for t, name, dt_ in ((keys, "keys", torch.int64), (sums, "sums", torch.float64), (counts, "counts", torch.int32),
+                         (new_keys, "new_keys", torch.int64), (new_sums, "new_sums", torch.float64),
+                         (new_counts, "new_counts", torch.int32), (failed, "failed", torch.int32)):
+        _req(t, name, dt_)
+    if sums.numel() != keys.numel() or counts.numel() != keys.numel() or new_sums.numel() != new_keys.numel() \
+            or new_counts.numel() != new_keys.numel():
+        raise OnmfKernelError("a table's keys, sums and counts must have the same length")
+    _check(load().onmf_edge_table_grow(_ptr(keys), _ptr(sums), _ptr(counts), keys.numel(), _ptr(new_keys), _ptr(new_sums),
+                                       _ptr(new_counts), new_keys.numel(), _ptr(failed), _stream(stream)),
+           "onmf_edge_table_grow")
 
 
 def _csr_args(rowptr, colidx, state):

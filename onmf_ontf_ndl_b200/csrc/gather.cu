@@ -843,7 +843,10 @@ extern "C" int onmf_motif_patches(int dtype, const int64_t* rowptr, const int32_
 // result is sum / count per distinct (a, b): one thread per (state, q, r) entry adds into an open-addressing hash table
 // keyed by (a << 32 | b) -- FP64 sums, integer counts.  The caller sizes the table (power of two, > 2x the entries is
 // always enough), fills the keys with 0xFF bytes and zeroes sums / counts.
+// A streamed reconstruction keeps one table across many calls (onmf_edge_table_add): the kernel then also counts the slots
+// it claims, so that the caller knows the load and can move the table into a larger one (onmf_edge_table_grow) in time.
 // ------------------------------------------------------------------------------------------------
+#include <cooperative_groups.h>
 namespace onmf {
 __device__ __forceinline__ unsigned long long mix64(unsigned long long x) {    // splitmix64 finaliser
   x ^= x >> 30; x *= 0xbf58476d1ce4e5b9ULL;
@@ -855,7 +858,8 @@ __device__ __forceinline__ unsigned long long mix64(unsigned long long x) {    /
 template <typename T>
 __global__ void edge_scatter_kernel(const T* __restrict__ R, long long ldr, const int* __restrict__ emb, long long n, int kk,
                                     unsigned long long* __restrict__ keys, double* __restrict__ sums,
-                                    unsigned int* __restrict__ cnts, unsigned long long mask, unsigned int* __restrict__ failed) {
+                                    unsigned int* __restrict__ cnts, unsigned long long mask, unsigned int* __restrict__ failed,
+                                    unsigned long long* __restrict__ claimed) {
   const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   const long long per = (long long)kk * kk;
   if (idx >= n * per) return;
@@ -872,29 +876,96 @@ __global__ void edge_scatter_kernel(const T* __restrict__ R, long long ldr, cons
     if (prev == ~0ULL || prev == key) {
       atomicAdd(&sums[h], val);
       atomicAdd(&cnts[h], 1u);
+      if (claimed != nullptr && prev == ~0ULL) {        // a new pair: one atomic per group of lanes that claimed together
+        const cooperative_groups::coalesced_group g = cooperative_groups::coalesced_threads();
+        if (g.thread_rank() == 0) atomicAdd(claimed, (unsigned long long)g.size());
+      }
       return;
     }
     h = (h + 1) & mask;
   }
   atomicAdd(failed, 1u);                      // table full (caller sized it too small)
 }
+
+// One thread per old slot.  Keys are unique, so an occupied slot is moved whole into the first free slot of its probe
+// sequence in the new table: the CAS that wins an empty key owns that slot, and its sum and count are stored, not added.
+__global__ void edge_table_grow_kernel(const unsigned long long* __restrict__ keys, const double* __restrict__ sums,
+                                       const unsigned int* __restrict__ cnts, long long capacity,
+                                       unsigned long long* __restrict__ new_keys, double* __restrict__ new_sums,
+                                       unsigned int* __restrict__ new_cnts, unsigned long long new_mask,
+                                       unsigned int* __restrict__ failed) {
+  const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= capacity) return;
+  const unsigned long long key = keys[i];
+  if (key == ~0ULL) return;
+  unsigned long long h = mix64(key) & new_mask;
+  for (unsigned long long probe = 0; probe <= new_mask; ++probe) {
+    if (atomicCAS(&new_keys[h], ~0ULL, key) == ~0ULL) {
+      new_sums[h] = sums[i];
+      new_cnts[h] = cnts[i];
+      return;
+    }
+    h = (h + 1) & new_mask;
+  }
+  atomicAdd(failed, 1u);                      // new table full (load above 1/2 is never asked for)
+}
 }  // namespace onmf
 
-extern "C" int onmf_edge_scatter_add(int dtype, const void* R, int64_t ldr, const int32_t* emb, int64_t n, int kk,
-                                     unsigned long long* keys, double* sums, unsigned int* counts, int64_t capacity,
-                                     unsigned int* failed, void* stream) {
-  if (!R || !emb || !keys || !sums || !counts || !failed || n < 0 || kk <= 0 || ldr < (int64_t)kk * kk)
-    return fail(ONMF_E_ARG, "edge_scatter_add: bad argument");
-  if (capacity <= 0 || (capacity & (capacity - 1))) return fail(ONMF_E_ARG, "edge_scatter_add: capacity must be a power of two");
+static int edge_scatter(const char* name, int dtype, const void* R, int64_t ldr, const int32_t* emb, int64_t n, int kk,
+                        unsigned long long* keys, double* sums, unsigned int* counts, int64_t capacity, unsigned int* failed,
+                        unsigned long long* claimed, void* stream) {
+  char msg[96];
+  if (!R || !emb || !keys || !sums || !counts || !failed || n < 0 || kk <= 0 || ldr < (int64_t)kk * kk) {
+    snprintf(msg, sizeof(msg), "%s: bad argument", name);
+    return fail(ONMF_E_ARG, msg);
+  }
+  if (capacity <= 0 || (capacity & (capacity - 1))) {
+    snprintf(msg, sizeof(msg), "%s: capacity must be a power of two", name);
+    return fail(ONMF_E_ARG, msg);
+  }
   if (n == 0) return ONMF_OK;
+  if (dtype != ONMF_F32 && dtype != ONMF_F64) {
+    snprintf(msg, sizeof(msg), "%s: bad dtype", name);
+    return fail(ONMF_E_ARG, msg);
+  }
   cudaStream_t st = (cudaStream_t)stream;
   const long long tot = n * (long long)kk * kk;
   const unsigned grid = (unsigned)cdiv<long long>(tot, 256);
   const unsigned long long mask = (unsigned long long)capacity - 1;
-  if (dtype == ONMF_F32) edge_scatter_kernel<float><<<grid, 256, 0, st>>>((const float*)R, ldr, emb, n, kk, keys, sums, counts, mask, failed);
-  else if (dtype == ONMF_F64) edge_scatter_kernel<double><<<grid, 256, 0, st>>>((const double*)R, ldr, emb, n, kk, keys, sums, counts, mask, failed);
-  else return fail(ONMF_E_ARG, "edge_scatter_add: bad dtype");
+  if (dtype == ONMF_F32)
+    edge_scatter_kernel<float><<<grid, 256, 0, st>>>((const float*)R, ldr, emb, n, kk, keys, sums, counts, mask, failed, claimed);
+  else
+    edge_scatter_kernel<double><<<grid, 256, 0, st>>>((const double*)R, ldr, emb, n, kk, keys, sums, counts, mask, failed, claimed);
   ONMF_LAUNCH_CHECK("edge_scatter_kernel");
+  return ONMF_OK;
+}
+
+extern "C" int onmf_edge_scatter_add(int dtype, const void* R, int64_t ldr, const int32_t* emb, int64_t n, int kk,
+                                     unsigned long long* keys, double* sums, unsigned int* counts, int64_t capacity,
+                                     unsigned int* failed, void* stream) {
+  return edge_scatter("edge_scatter_add", dtype, R, ldr, emb, n, kk, keys, sums, counts, capacity, failed, nullptr, stream);
+}
+
+extern "C" int onmf_edge_table_add(int dtype, const void* R, int64_t ldr, const int32_t* emb, int64_t n, int kk,
+                                   unsigned long long* keys, double* sums, unsigned int* counts, int64_t capacity,
+                                   unsigned long long* claimed, unsigned int* failed, void* stream) {
+  if (!claimed) return fail(ONMF_E_ARG, "edge_table_add: bad argument");
+  return edge_scatter("edge_table_add", dtype, R, ldr, emb, n, kk, keys, sums, counts, capacity, failed, claimed, stream);
+}
+
+extern "C" int onmf_edge_table_grow(const unsigned long long* keys, const double* sums, const unsigned int* counts,
+                                    int64_t capacity, unsigned long long* new_keys, double* new_sums, unsigned int* new_counts,
+                                    int64_t new_capacity, unsigned int* failed, void* stream) {
+  if (!keys || !sums || !counts || !new_keys || !new_sums || !new_counts || !failed)
+    return fail(ONMF_E_ARG, "edge_table_grow: bad argument");
+  if (capacity <= 0 || (capacity & (capacity - 1)) || new_capacity <= 0 || (new_capacity & (new_capacity - 1)))
+    return fail(ONMF_E_ARG, "edge_table_grow: capacities must be powers of two");
+  if (new_capacity <= capacity) return fail(ONMF_E_ARG, "edge_table_grow: the new capacity must be larger than the old one");
+  cudaStream_t st = (cudaStream_t)stream;
+  const unsigned grid = (unsigned)cdiv<long long>(capacity, 256);
+  edge_table_grow_kernel<<<grid, 256, 0, st>>>(keys, sums, counts, capacity, new_keys, new_sums, new_counts,
+                                               (unsigned long long)new_capacity - 1, failed);
+  ONMF_LAUNCH_CHECK("edge_table_grow_kernel");
   return ONMF_OK;
 }
 

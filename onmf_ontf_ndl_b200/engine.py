@@ -286,8 +286,10 @@ class OnmfEngine:
             _lib.gather_patches_mb(pm, self._Xg[:n], stream=stream)
         return self._Xg[:n]
 
-    def sparse_code(self, Xt: torch.Tensor, W: Optional[torch.Tensor] = None, alpha=None, out=None):
-        """Ht (n x k) = positive lasso_lars codes of the rows of Xt (n x d) against W (default: current)."""
+    def sparse_code(self, Xt: torch.Tensor, W=None, alpha=None, out=None, first_tier=-1):
+        """Ht (n x k) = positive lasso_lars codes of the rows of Xt (n x d) against W (default: current).  W may also be
+        the handle of derive_foreign(W), so that many calls against one dictionary derive it once.  first_tier: as in
+        sparse_code_patches."""
         n = Xt.shape[0]
         self._reserve(max(n, 1))
         Ct = self.Ct[:n]
@@ -297,10 +299,12 @@ class OnmfEngine:
         if W is None:
             self.flush()
             f = _Dictionary(self.W, self.G, getattr(self, "Whi", None), getattr(self, "Wlo", None), self._raw_W)
+        elif isinstance(W, _Dictionary):
+            f = W
         else:
             f = self.derive_foreign(W)
         self._cov_into(Xt, None, None, 1.0, n, f.W, f.Whi, f.Wlo, Ct, torch.cuda.current_stream(self.device))
-        self._lars(f, Ct, alpha, Ht, -1)
+        self._lars(f, Ct, alpha, Ht, first_tier)
         return Ht
 
     def derive_foreign(self, W: torch.Tensor):

@@ -257,6 +257,11 @@ def reconstruct_network(G, W, embs, alpha=0, precision=None):
             raise _lib.OnmfKernelError("edge_scatter_add could not place %d entries" % nf)
         del keys, sums, cnts
         cap *= 4
+    return _table_result(keys, sums, cnts, nodes)
+
+
+def _table_result(keys, sums, cnts, nodes):
+    """(pairs, weight, count) of the occupied slots of an edge table, sorted by (a, b) position in nodes"""
     used = torch.nonzero(cnts > 0).flatten()
     kz = keys[used].cpu().numpy().astype(np.uint64)
     sm = sums[used].cpu().numpy()
@@ -267,6 +272,98 @@ def reconstruct_network(G, W, embs, alpha=0, precision=None):
     lab = np.asarray(nodes, dtype=object)
     pairs = np.stack([lab[a], lab[b]], axis=1) if len(kz) else np.empty((0, 2), dtype=object)
     return pairs, sm / np.maximum(ct, 1), ct
+
+
+# First capacity of the streamed pair table (20 bytes per slot: 20 MB); it grows by doubling as pairs arrive.
+_TABLE_START = 1 << 20
+# Entries per scatter of the streamed form.  Before a scatter the table is grown to twice the slots in use plus the entries
+# about to be added, so this sets the table's headroom (at most 2^24 slots, 320 MB: less than one full band's Xt at
+# k = 21); it is large enough that the one host read of the slot count per scatter is a small part of the scatter.
+_SCATTER_ENTRIES = 1 << 23
+
+
+def _empty_table(cap, dev):
+    return (torch.full((cap,), -1, dtype=torch.int64, device=dev), torch.zeros(cap, dtype=torch.float64, device=dev),
+            torch.zeros(cap, dtype=torch.int32, device=dev))
+
+
+def reconstruct_network_chains(chains, W, n_samples, steps_per_sample=1, alpha=0, precision=None, max_band=262144):
+    """reconstruct_network(G, W, chains.sample(n_samples, steps_per_sample), alpha, precision) in device memory bounded by
+    a band of states and the pair table, not by the trajectory: the streamed form of the drivers' reconstruct_network(
+    recons_iter, is_glauber_recons) for long runs of patches.MotifChains.
+
+    The n_chains x n_samples states are taken in bands: a chain range [c0, c1) times a run of consecutive samples, each at
+    least _lib.coder_band_floor() states (unless the whole run is smaller) and at most about max_band, by _band_plan's rule.
+    A band advances chains c0 .. c1-1 only (a trajectory depends on (seed, chain, step), so these are the states of one
+    sample() call), forms its motif patches, codes them (first tier 0 in every band: an earlier band's tier hint must not
+    steer this one), forms R = Ht W^T and adds R to one pair table with onmf_edge_table_add.  The table starts small and is
+    moved into a larger one (onmf_edge_table_grow) whenever the next scatter could take its load above 1/2; no entry is
+    ever rescattered.  Its final size is set by the distinct directed pairs visited, 20 bytes per slot at load <= 1/2.
+
+    Returns (pairs, weight, count) as reconstruct_network: the same pairs and counts, the same codes and reconstructions,
+    weights equal up to the order of the FP64 atomic sums.  chains.state and chains.step end where that sample() call
+    leaves them.  A chain state that is not a homomorphism raises (OnmfKernelError) when its chain range is reached."""
+    if not isinstance(chains, patches.MotifChains):
+        raise ValueError("chains must be a patches.MotifChains")
+    W = np.asarray(W, dtype=np.float64)
+    if W.ndim != 2:
+        raise ValueError("W must be a (k^2 x r) dictionary")
+    d, r = W.shape
+    kk = chains.kk
+    if d != kk * kk:
+        raise ValueError("dictionary has %d rows, expected k^2 = %d" % (d, kk * kk))
+    n_samples, sps = int(n_samples), int(steps_per_sample)
+    if n_samples < 0:
+        raise ValueError("n_samples must be >= 0")
+    if sps < 1:
+        raise ValueError("steps_per_sample must be >= 1")
+    dtype = _host.torch_dtype(precision)
+    N = chains.n_chains
+    if n_samples == 0 or N == 0:
+        return np.empty((0, 2), dtype=object), np.empty(0), np.empty(0, dtype=np.int64)
+    dev = chains.state.device
+    floor = _lib.coder_band_floor(dev)
+    plan = [(c0, c1, _band_plan(n_samples, max(max_band // (c1 - c0), 1), -(-floor // (c1 - c0))))
+            for c0, c1 in _band_plan(N, max_band, floor)]
+    mmax = max((c1 - c0) * (s1 - s0) for c0, c1, sb in plan for s0, s1 in sb)
+    run = patches._MOTIF_STEPS[chains.mcmc]
+    Wd = _host.to_device(W, dtype, dev)
+    eng = OnmfEngine(d, r, alpha=alpha, dtype=dtype, device=dev)
+    f = eng.derive_foreign(Wd)
+    Wt = torch.empty(r, d, dtype=dtype, device=dev)
+    _lib.transpose(Wd, Wt)
+    emb = torch.empty(mmax, kk, dtype=torch.int32, device=dev)
+    Xt = torch.empty(mmax, d, dtype=dtype, device=dev)
+    R = torch.empty(mmax, d, dtype=dtype, device=dev)
+    keys, sums, cnts = _empty_table(_TABLE_START, dev)
+    claimed = torch.zeros(1, dtype=torch.int64, device=dev)
+    failed = torch.zeros(1, dtype=torch.int32, device=dev)
+    chunk = max(1, _SCATTER_ENTRIES // d)
+    for c0, c1, sbands in plan:
+        state = chains.state[c0:c1]
+        for s0, s1 in sbands:
+            m = (c1 - c0) * (s1 - s0)
+            e = emb[:m]
+            run(chains.rowptr, chains.colidx, state, c0, chains.seed, chains.step + s0 * sps, sps, e)
+            _lib.motif_patches(chains.rowptr, chains.colidx, e, Xt[:m])                             # K1
+            Ht = eng.sparse_code(Xt[:m], f, alpha=alpha, first_tier=0)                               # K2 + K3
+            _lib.cov(Ht, Wt, R[:m])                                                                  # patch_recons rows
+            for j0 in range(0, m, chunk):
+                j1 = min(m, j0 + chunk)
+                need = 2 * (int(claimed.item()) + (j1 - j0) * d)
+                if need > keys.numel():
+                    cap = keys.numel()
+                    while cap < need:
+                        cap *= 2
+                    grown = _empty_table(cap, dev)
+                    _lib.edge_table_grow(keys, sums, cnts, *grown, failed)
+                    keys, sums, cnts = grown
+                _lib.edge_table_add(R[j0:j1], e[j0:j1], keys, sums, cnts, claimed, failed)
+    chains.step += n_samples * sps
+    nf = int(failed.item())
+    if nf:
+        raise _lib.OnmfKernelError("edge_table_add / edge_table_grow could not place %d entries" % nf)
+    return _table_result(keys, sums, cnts, chains.nodes)
 
 
 def simple_graph_edges(pairs, weight):
