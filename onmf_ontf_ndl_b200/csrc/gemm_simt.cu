@@ -373,10 +373,15 @@ extern "C" int onmf_gram_f64(int dtype_in, const void* W, int d, int k, double* 
 // projected-gradient coder takes two of them per outer iteration (np.linalg.norm(., 2), src/onmf.py:265).
 // M^T M comes from the FP64 Gram kernels above; lambda_max of the k x k matrix by repeated squaring in one CTA:
 // B_0 = G / tr G, B_{m+1} = B_m^2 / tr(B_m^2) -- the dominant eigenspace takes over quadratically -- then the Rayleigh
-// quotient of G at the column of B with the largest diagonal entry.  With SQ squarings the relative error is at most
-// ~eps^2 (1 - lambda_2/lambda_1) with eps = (lambda_2/lambda_1)^(2^SQ): < 1e-5 for every spectrum at SQ = 16.
+// quotient of G at the column of B with the largest diagonal entry.  With SQ squarings, x = 1 - lambda_2/lambda_1,
+// eps = (1 - x)^(2^SQ) and m eigenvalues at lambda_2 (m up to k - 1), the relative error of sqrt(lambda) is about
+// (x / 2) m eps^2 / (1 + m eps^2) when the top eigenvector is flat: largest, ~ln k / 2^(SQ+3), at x ~ ln k / 2^(SQ+1).
+// At SQ = 16 that reaches 1.3e-5 for k = 256 and 1.5e-5 for k = 512; SQ = 17 keeps every spectrum below 1e-5 for k <= 512
+// (tests/test_pgd_coder_variants.py restates this kernel in numpy and runs those spectra on both).  The 17th squaring
+// costs one more k^3 product: onmf_spectral_norm of a 4096 x k matrix 2.42 -> 2.57 ms at k = 64, 148 -> 157 ms at
+// k = 256, 1184 -> 1258 ms at k = 512 (+6 %; B200, 1000 W power limit, CUDA events over 20-50 calls).
 namespace onmf {
-constexpr int LMAX_SQUARINGS = 16;
+constexpr int LMAX_SQUARINGS = 17;
 __global__ void __launch_bounds__(1024) lambda_max_kernel(const double* __restrict__ G, int k, double* __restrict__ b0,
                                                           double* __restrict__ b1, int squarings, double* __restrict__ out) {
   __shared__ double red[32];

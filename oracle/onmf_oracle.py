@@ -12,6 +12,7 @@ It is a numpy restatement (float64, like the reference) of
   * `Online_NTF.step`                       reference src/ontf.py:117-154
   * `Online_NTF.train_dict_single` loop     reference src/ontf.py:156-244
   * `update_code_within_radius`             reference src/onmf.py:233-271
+    (and its G / C form per sweep and per sample, `pgd_sweep_gc` / `pgd_columns_gc`)
   * tensor matricization (`tl_unfold`)      reference src/ontf.py:203-208
   * the drivers' patch gathers              reference image_reconstruction.py:173-206,
                                             image_reconstruction_tensor.py:87-124,
@@ -297,6 +298,48 @@ def update_code_within_radius(X, W, H0, r=None, alpha=0, sub_iter=10, stopping_d
         dist = np.linalg.norm(H - H_old, 2) / np.linalg.norm(H_old, 2)
         it += 1
     return H
+
+
+def pgd_sweep_gc(G, Ct, Ht, alpha, it, q0=0, q1=None):
+    """One outer iteration of the coder above in the kernels' G / C form (onmf_pgd_sweep_rows): for q0 <= q < q1, Gauss-Seidel
+    in q, h_q <- max(h_q - (G[q, :] h - c_q + alpha) / (sqrt(it + 10) (G_qq + 1)), 0), independently per sample.
+    G (k x k) is used as given (row q), so it need not be symmetric; Ct, Ht (n x k) are sample-major.  Returns the new Ht."""
+    G = np.asarray(G, dtype=np.float64)
+    Ct = np.asarray(Ct, dtype=np.float64)
+    H = np.array(Ht, dtype=np.float64, copy=True)
+    k = G.shape[0]
+    q1 = k if q1 is None else q1
+    scale = np.sqrt(it + 10.0)
+    for q in range(q0, q1):
+        grad = H @ G[q, :] - Ct[:, q] + alpha
+        H[:, q] = np.maximum(H[:, q] - grad / (scale * (G[q, q] + 1.0)), 0.0)
+    return H
+
+
+def pgd_columns_gc(G, Ct, Ht, alpha, sub_iter, stopping_diff):
+    """The whole coder per sample in the G / C form (onmf_pgd_code_columns): sweeps it = 0, 1, ... while it < sub_iter and
+    dist > stopping_diff, dist = ||h - h_old|| / ||h_old|| of that sample alone (x / 0 = inf keeps going, 0 / 0 = NaN stops,
+    like the reference's numpy division).  Returns (Ht, sweeps (n,), trail (n x sub_iter)): trail[j, i] is the dist after
+    sweep i of sample j, valid for i < sweeps[j] (NaN beyond)."""
+    G = np.asarray(G, dtype=np.float64)
+    H = np.array(Ht, dtype=np.float64, copy=True)
+    Ct = np.asarray(Ct, dtype=np.float64)
+    n = H.shape[0]
+    sweeps = np.zeros(n, dtype=np.int64)
+    trail = np.full((n, max(int(sub_iter), 0)), np.nan)
+    dist = np.ones(n)
+    for it in range(int(sub_iter)):
+        act = np.nonzero(dist > stopping_diff)[0]
+        if act.size == 0:
+            break
+        h_old = H[act]
+        h = pgd_sweep_gc(G, Ct[act], h_old, alpha, it)
+        with np.errstate(divide="ignore", invalid="ignore"):
+            dist[act] = np.linalg.norm(h - h_old, axis=1) / np.linalg.norm(h_old, axis=1)
+        H[act] = h
+        trail[act, it] = dist[act]
+        sweeps[act] += 1
+    return H, sweeps, trail
 
 
 # --------------------------------------------------------------------------------------

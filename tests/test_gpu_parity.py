@@ -4,6 +4,7 @@ reference's golden fixtures.  Tolerances (BASELINE.json north_star):
               (measured ~1e-11; asserted at 1e-8 to catch regressions)
   fp32 mode : final dictionary per atom within 1e-3; reconstruction error within 0.5 %.
 """
+import math
 import os
 import warnings
 
@@ -1040,7 +1041,9 @@ def test_fast_tier_small_dictionaries():
 
 def test_spectral_norm_kernel():
     """onmf_spectral_norm (FP64 Gram + largest eigenvalue by repeated squaring) against numpy's SVD: generic, rank-one,
-    repeated and nearly repeated top singular values, a zero matrix, one column; fp32 and fp64 inputs."""
+    repeated and nearly repeated top singular values, a zero matrix, one column; fp32 and fp64 inputs; and n in {1024, 1040,
+    5000, 1e5} x k in {1, 2, 64, 65, 256, 512}, where the FP64 Gram takes its 16-way split over n with a partial last chunk.
+    Every case within the header's 1e-5 of the norm of the dtype-rounded matrix."""
     rng = np.random.default_rng(55)
     cases = []
     cases.append(rng.random((700, 25)))
@@ -1052,17 +1055,22 @@ def test_spectral_norm_kernel():
     cases.append(np.zeros((50, 7)))
     cases.append(rng.random((1000, 1)))
     cases.append(rng.random((3, 238)) * 1e-3)
-    for M in cases:
-        n, k = M.shape
-        ref = np.linalg.norm(M, 2)
+    shapes = [(n, k) for n in (1024, 1040, 5000, 100000) for k in (1, 2, 64, 65, 256, 512)]
+    for M in cases + shapes:
         for dt_ in (torch.float64, torch.float32):
-            Md = tt(M, dt_)
+            if isinstance(M, tuple):
+                n, k = M
+                Mr = rng.random((n, k)) - 0.3 * (k > 1) * rng.random(k)                 # tilted: a dominant but not lone top
+            else:
+                n, k = M.shape
+                Mr = M
+            Mr = Mr.astype(np.float32 if dt_ == torch.float32 else np.float64).astype(np.float64)
+            ref = math.sqrt(max(np.linalg.eigvalsh(Mr.T @ Mr)[-1], 0.0)) if n > 4 * k else np.linalg.norm(Mr, 2)
             out = torch.full((1,), float("nan"), dtype=torch.float64, device=dev())
             ws = torch.empty(_lib.spectral_norm_workspace(n, k), dtype=torch.uint8, device=dev())
-            _lib.spectral_norm(Md, out, ws)
+            _lib.spectral_norm(tt(Mr, dt_), out, ws)
             got = float(out[0])
-            tol = 2e-5 if dt_ == torch.float64 else 1e-4
-            assert abs(got - ref) <= tol * max(ref, 1e-300) + (0 if ref > 0 else 1e-300), (n, k, dt_, got, ref)
+            assert abs(got - ref) <= 1e-5 * ref or got == ref == 0.0, (n, k, dt_, got, ref)
 
 
 # ---------------------------------------------------------------------------------------------- K1 vector forms, batched PGD
