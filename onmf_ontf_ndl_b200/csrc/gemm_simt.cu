@@ -522,7 +522,9 @@ extern "C" int onmf_xxt_partial(int dtype, const void* Xt, int64_t n, int d, voi
   int splits = (int)(want < cap ? want : cap);
   if (splits < 1) splits = 1;
   long long stride = (long long)d * d;
-  if (splits > 1 && (!workspace || workspace_bytes < (size_t)splits * stride * tsz)) splits = 1;
+  // as many splits as the workspace holds: one split is one CTA per tile summing every sample in sequence
+  const long long fit = workspace ? (long long)(workspace_bytes / ((size_t)stride * tsz)) : 0;
+  if (splits > fit) splits = fit > 1 ? (int)fit : 1;
   int rc;
   if (dtype == ONMF_F32) {
     float* dst = splits == 1 ? (float*)P2 : (float*)workspace;

@@ -257,6 +257,29 @@ def step(X, A, B, W, t, alpha, beta=None, coder="lars"):
     return H, A1, B1, W1
 
 
+def step_given_codes(X, H, W, A, B, C, t, beta=None):
+    """`step` with the codes H (k x n) given: the coder drops out and the step is the update with the OLD aggregates and
+    the blends.  C (d x d) or None follows C1 = (1-w) C + w X X^T (reference src/onmf.py:157-158).  Returns (W1, A1, B1, C1)."""
+    X = np.asarray(X, dtype=np.float64)
+    H = np.asarray(H, dtype=np.float64)
+    W1 = update_dict(W, A, B)
+    A1, B1 = aggregate(A, B, H, X, t, beta)
+    C1 = None
+    if C is not None:
+        w = float(t) ** (-(1.0 if beta is None else beta))
+        C1 = (1.0 - w) * C + w * (X @ X.T)
+    return W1, A1, B1, C1
+
+
+def run_given_codes(Xs, Hs, W0, A0, B0, ts, beta=None, C0=None):
+    """step_given_codes over a sequence of minibatches Xs[i] (d x n_i) with codes Hs[i] (k x n_i) at steps ts[i].
+    Returns the final (W, A, B, C)."""
+    W, A, B, C = W0, A0, B0, C0
+    for X, H, t in zip(Xs, Hs, ts):
+        W, A, B, C = step_given_codes(X, H, W, A, B, C, t, beta)
+    return W, A, B, C
+
+
 def train(X, k, idx_seq, W0, A0=None, B0=None, history=0, alpha=1, beta=None, coder="lars",
           record=False):
     """reference src/ontf.py:224-236 with the minibatch indices given explicitly
