@@ -148,8 +148,14 @@ int onmf_lasso_lars(int dtype, const void* G, const void* Ct, int64_t n, int k, 
  * start by the next (larger, lower-occupancy) tier.  first_tier = 0 / 1 starts every column in that tier;
  * first_tier = -1 (what onmf_lasso_lars uses) is adaptive: a device-side flag kept in the first 64 bytes of the
  * workspace remembers whether more than 1/16 of the previous call's columns needed the larger tier.  The workspace
- * must therefore be zero-filled once before its first use and may be reused across calls.  Results are identical
- * for every setting. */
+ * must therefore be zero-filled once before its first use and may be reused across calls.  first_tier = t and the
+ * adaptive call under hint t run the same kernels and give the same bits, so the adaptive call's codes depend on the
+ * hint left by earlier calls on the workspace.  first_tier 0 and 1 give the same bits at k <= 32 (one tier) and on the
+ * fp32 small-minibatch route (FP64 Gram, fast tier on, k <= 64 and n <= 24 / 48 x SMs at k <= 32 / 64), which runs
+ * whatever first_tier says and neither reads nor updates the hint.  Elsewhere a column that fits the first tier is
+ * finished by a different kernel instance under 0 and 1 and may differ in the last bits: measured in fp64 at every
+ * class k > 32 (0 to 10 columns of 40 to 80, up to 1e-4 of the fp64 code bar); the source of the difference is not
+ * isolated.  tests/test_lars_coder_variants.py checks each of these statements. */
 int onmf_lasso_lars_ex(int dtype, const void* G, const void* Ct, int64_t n, int k, int d, double alpha,
                        int max_iter, void* Ht, void* workspace, size_t workspace_bytes,
                        onmf_lars_stats* stats, int first_tier, void* stream);

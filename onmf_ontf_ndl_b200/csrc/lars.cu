@@ -1182,8 +1182,11 @@ static int launch_class(const T* G, const double* G64, const T* Ct, long long n,
   };
   int rc = ONMF_OK;
   if constexpr (std::is_same<T, float>::value && KP <= 64 && S0 == 32 && !GL) {
-    if (G64 != nullptr && g_lars_fast && first_tier <= 0 && n <= (k <= 32 ? 1LL : 2LL) * num_sms() * FAST_SMALL_WARPS && k <= 64) {
-      // fast tier over all columns, then the general kernel (the larger of its tiers) over the columns it handed on
+    if (G64 != nullptr && g_lars_fast && n <= (k <= 32 ? 1LL : 2LL) * num_sms() * FAST_SMALL_WARPS && k <= 64) {
+      // fast tier over all columns, then the general kernel (the larger of its tiers) over the columns it handed on.
+      // Taken for every first_tier: the fast kernel and the general kernel sum a join's FP64 terms in different orders, so
+      // a first_tier that picked the general kernel here would change the codes in the last bits.  The hint is neither
+      // read nor updated on this route.
       rc = launch_fast_small(tier_params(0, 0, false, true, false), n, st);
       if (rc) return rc;
       constexpr int NEXT = S1 > 0 ? S1 : S0;

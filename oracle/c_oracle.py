@@ -31,6 +31,10 @@ def load():
         _lib.oracle_update_dict.argtypes = [dp, dp, dp, ctypes.c_int, ctypes.c_int]
         _lib.oracle_aggregate.restype = None
         _lib.oracle_aggregate.argtypes = [dp, dp, dp, dp, ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_double]
+        ip = ctypes.POINTER(ctypes.c_int)
+        _lib.oracle_lars_positive.restype = ctypes.c_int
+        _lib.oracle_lars_positive.argtypes = [dp, dp, ctypes.c_int, ctypes.c_int, ctypes.c_double, ctypes.c_int, dp, ip, dp, ip,
+                                              dp]
     return _lib
 
 
@@ -47,6 +51,36 @@ def sparse_code(X, W, alpha, max_iter=1000):
     H = np.zeros((k, n))
     load().oracle_sparse_code(_p(X), _p(W), d, n, k, float(alpha), int(max_iter), _p(H))
     return H
+
+
+def lars_columns(G, Ct, alpha, d, max_iter=1000):
+    """Positive lasso_lars codes of the rows of Ct (n x k covariances W^T x) against the Gram G (k x k), one
+    oracle_lars_positive path per row.  Returns H (n x k) and a dict of per-row arrays: n_iter (knots), max_active,
+    drops (drop steps), status (bits 1 degenerate pivot, 2 "alpha increasing" bail-out, 4 max_iter), min_gap (the
+    smallest relative gap between the joining covariance and the runner-up, or between a drop and the step it competes
+    with: a near-tie) and min_pivot (the smallest pivot^2 / G_jj of an accepted join)."""
+    G = np.ascontiguousarray(G, dtype=np.float64)
+    Ct = np.ascontiguousarray(Ct, dtype=np.float64)
+    n, k = Ct.shape
+    lib = load()
+    H = np.zeros((n, k))
+    info = np.zeros((n, 4), dtype=np.int32)
+    gaps = np.zeros((n, 2))
+    gap = np.zeros(2)
+    work = np.empty((k + 1) * (k + 1) + 6 * k)
+    iwork = np.empty(2 * k, dtype=np.int32)
+    one = np.zeros(3, dtype=np.int32)
+    h = np.empty(k)
+    ip = ctypes.POINTER(ctypes.c_int)
+    for j in range(n):
+        c = Ct[j]
+        info[j, 3] = lib.oracle_lars_positive(_p(G), _p(c), k, int(d), float(alpha), int(max_iter), _p(h),
+                                              one.ctypes.data_as(ip), _p(work), iwork.ctypes.data_as(ip), _p(gap))
+        gaps[j] = gap
+        info[j, :3] = one
+        H[j] = h
+    return H, dict(n_iter=info[:, 0].copy(), max_active=info[:, 1].copy(), drops=info[:, 2].copy(), status=info[:, 3].copy(),
+                 min_gap=gaps[:, 0].copy(), min_pivot=gaps[:, 1].copy())
 
 
 def update_dict(W, A, B):

@@ -73,11 +73,18 @@ static void chol_delete(double* L, int ld, int s, int out) {
   }
 }
 
+/* relative gap of the two smallest of a, b (a <= b) */
+static double rel_gap(double a, double b) { return (b - a) / (fabs(b) > 0.0 ? fabs(b) : 1.0); }
+
 /* One column.  G (k x k), c (k) -> coef (k).  Returns status bits (1 degenerate, 2 alpha-increase, 4 max_iter);
- * info[0]=n_iter, info[1]=max_active, info[2]=drops if info != NULL.  work: caller scratch of
+ * info[0]=n_iter, info[1]=max_active, info[2]=drops if info != NULL.  min_gap (if not NULL): min_gap[0] = the smallest
+ * relative gap, over the knots, between the joining covariance and the runner-up, and between the shortest drop step and
+ * the join / full step or the next drop -- a near-tie, where rounding may change the path; min_gap[1] = the smallest
+ * pivot^2 / G_jj of an accepted join (a nearly dependent atom: whether it passes the 1e-7 pivot rule is up to rounding
+ * when this is small).  work: caller scratch of
  * (k+1)*(k+1) + 6*k doubles and 2*k ints. */
 int oracle_lars_positive(const double* G, const double* c, int k, int d, double reg, int max_iter, double* coef,
-                         int* info, double* work, int* iwork) {
+                         int* info, double* work, int* iwork, double* min_gap) {
   const int ld = k + 1;
   double* L = work;
   double* cov = L + (size_t)ld * ld;
@@ -90,6 +97,7 @@ int oracle_lars_positive(const double* G, const double* c, int k, int d, double 
   int n_act = 0, n_in = k, n_iter = 0, drop = 0, status = 0, max_act = 0, drops = 0;
   double a_cur = 0.0, a_prev = 0.0;
   const double amin = reg / d;
+  double gap = INFINITY, minsig = INFINITY;
   memcpy(cov, c, sizeof(double) * k);
   for (int i = 0; i < k; ++i) { cur[i] = 0.0; prev[i] = 0.0; inact[i] = i; }
   for (;;) {
@@ -100,6 +108,9 @@ int oracle_lars_positive(const double* G, const double* c, int k, int d, double 
       C = cov[inact[0]];
       for (int i = 1; i < n_in; ++i)
         if (cov[inact[i]] > C) { C = cov[inact[i]]; pos = i; }
+      if (!drop && C / d > amin + EPS32)
+        for (int i = 0; i < n_in; ++i)
+          if (i != pos) { double g = rel_gap(cov[inact[i]], C); if (g < gap) gap = g; }
     }
     a_cur = C / d;
     if (a_cur <= amin + EPS32) {
@@ -123,6 +134,7 @@ int oracle_lars_positive(const double* G, const double* c, int k, int d, double 
         status |= 1;
         continue;
       }
+      if (piv * piv / G[(size_t)j * k + j] < minsig) minsig = piv * piv / G[(size_t)j * k + j];
       memmove(inact, inact + 1, sizeof(int) * (n_in - 1));
       --n_in;
       act[n_act++] = j;
@@ -146,11 +158,17 @@ int oracle_lars_positive(const double* G, const double* c, int k, int d, double 
     }
     double gamma = C / AA;
     if (g1 < gamma) gamma = g1;
-    double zpos = min_pos_init();
+    double zpos = min_pos_init(), z2 = min_pos_init();
     int zi = -1;
     for (int q = 0; q < n_act; ++q) {
       double z = -cur[act[q]] / (w[q] + TINY32);
-      if (z > 0.0 && z < zpos) { zpos = z; zi = q; }
+      if (z > 0.0 && z < zpos) { z2 = zpos; zpos = z; zi = q; } else if (z > 0.0 && z < z2) z2 = z;
+    }
+    /* a drop against the join / full step, or against a second drop, decides the knot and drop counts */
+    if (zpos < min_pos_init()) {
+      double g = zpos < gamma ? rel_gap(zpos, gamma) : rel_gap(gamma, zpos);
+      if (z2 < min_pos_init() && rel_gap(zpos, z2) < g) g = rel_gap(zpos, z2);
+      if (g < gap) gap = g;
     }
     drop = 0;
     if (zpos < gamma) { gamma = zpos; drop = 1; }
@@ -177,6 +195,7 @@ int oracle_lars_positive(const double* G, const double* c, int k, int d, double 
   }
   memcpy(coef, cur, sizeof(double) * k);
   if (info) { info[0] = n_iter; info[1] = max_act; info[2] = drops; }
+  if (min_gap) { min_gap[0] = gap; min_gap[1] = minsig; }
   return status;
 }
 
@@ -200,7 +219,7 @@ int oracle_sparse_code(const double* X, const double* W, int d, int n, int k, do
       for (int f = 0; f < d; ++f) s += W[(size_t)f * k + a] * X[(size_t)f * n + j];
       cv[a] = s;
     }
-    status |= oracle_lars_positive(G, cv, k, d, reg, max_iter, h, NULL, work, iwork);
+    status |= oracle_lars_positive(G, cv, k, d, reg, max_iter, h, NULL, work, iwork, NULL);
     for (int a = 0; a < k; ++a) H[(size_t)a * n + j] = h[a];
   }
   free(G); free(cv); free(h); free(work); free(iwork);

@@ -100,8 +100,39 @@ def _chol_delete(L, s, out):
             L[q, i + 1] = c * y - sn * x
 
 
+def _chol_append_blas(L, s, g_row, g_diag):
+    """_chol_append with one triangular solve (same result to rounding; the float32 emulation's factor)"""
+    from scipy.linalg import solve_triangular
+    w = solve_triangular(L[:s, :s], g_row, lower=True, check_finite=False) if s else np.zeros(0)
+    L[s, :s] = w
+    piv = max(np.sqrt(abs(g_diag - w @ w)), _EPS64)
+    L[s, s] = piv
+    return piv
+
+
+def _chol_solve_blas(L, s, b):
+    from scipy.linalg import solve_triangular
+    y = solve_triangular(L[:s, :s], b, lower=True, check_finite=False)
+    return solve_triangular(L[:s, :s].T, y, lower=False, check_finite=False)
+
+
+def _chol_delete_blas(L, s, out):
+    """_chol_delete with each rotation applied to the rows below as one vector operation"""
+    for i in range(out, s - 1):
+        L[i, :i + 2] = L[i + 1, :i + 2]
+    for i in range(out, s - 1):
+        a, b = L[i, i], L[i, i + 1]
+        r = np.hypot(a, b)
+        c, sn = (1.0, 0.0) if r == 0.0 else (a / r, b / r)
+        L[i, i] = r
+        L[i, i + 1] = 0.0
+        x, y = L[i + 1:s - 1, i].copy(), L[i + 1:s - 1, i + 1].copy()
+        L[i + 1:s - 1, i] = c * x + sn * y
+        L[i + 1:s - 1, i + 1] = c * y - sn * x
+
+
 def lars_lasso_positive(G, c, reg, n_features, max_iter=1000, return_info=False,
-                        round_decimals=15):
+                        round_decimals=15, work_dtype=np.float64, gram32=False, mutant=None):
     """argmin_{h>=0} 0.5*||x - W h||^2 + reg * sum(h) the way sklearn's positive lasso_lars does it.
 
     G = W^T W (k x k), c = W^T x (k,), n_features = d (sklearn scales alpha by 1/d,
@@ -111,14 +142,42 @@ def lars_lasso_positive(G, c, reg, n_features, max_iter=1000, return_info=False,
     eps) and linearly interpolates the last segment (_least_angle.py:651-663) -- which on
     the final (unregularised least-squares) segment lands at a slightly shifted alpha
     (SURVEY.md §B.2); that behaviour is reproduced here by construction.
+
+    work_dtype=np.float32 emulates the fp32 coder of csrc/lars.cu: covariances, correlations, C, AA, step lengths,
+    coefficients and the interpolation are rounded to float32 (the correlation pass and the recomputed covariance of a
+    dropped atom read a float32 copy of G), the factor and the unnormalised weights G_AA^-1 1 stay float64 (kept with
+    BLAS triangular solves: the same factor to rounding, fast enough to emulate every column of a case); alpha and
+    the eps32 tolerance are kept in covariance units; a step-length candidate whose numerator is an exact tie counts as
+    a zero-length step (denominator > 0 decides); the atom dropped by the last drop step may not be the joiner of the
+    next join knot while another candidate exists; a dropped atom's coefficient is exactly 0.  gram32=True adds the
+    rule of the fp32-Gram form (onmf_lasso_lars_ex): a pivot G_jj - |t|^2 <= 4 eps32 G_jj is degenerate.  With the
+    default float64 the function is the restatement above, bit for bit.
+
+    mutant: one deliberate bug (tests only, to show that their bars tell a broken coder from rounding): 'tie_high' (join
+    ties go to the last candidate), 'no_interp' (no last-segment interpolation), 'no_drop_recompute' (a dropped atom keeps
+    its stale covariance), 'join_after_drop', 'alpha_unscaled' (alpha not divided by d), 'max_iter_plus1', 'no_eps_stop'.
     """
+    f32 = np.dtype(work_dtype) == np.float32
+    t = np.float32 if f32 else np.float64
+    append, solve, delete = (_chol_append_blas, _chol_solve_blas, _chol_delete_blas) if f32 else \
+        (_chol_append, _chol_solve, _chol_delete)
     G = np.asarray(G, dtype=np.float64)
-    cov = np.array(c, dtype=np.float64)
+    Gw = G.astype(t)
+    cov = np.array(c, dtype=t)
+    c = np.asarray(c, dtype=t)
     k = cov.shape[0]
-    alpha_min = float(reg) / n_features
-    coef = np.zeros(k)
-    prev_coef = np.zeros(k)
-    alpha_cur, alpha_prev = 0.0, 0.0
+    if f32:
+        dT = t(n_features)
+        alpha_min = t(t(reg) / dT) * dT
+        eps = t(_EPS32) * dT
+    else:
+        alpha_min = float(reg) / (1 if mutant == "alpha_unscaled" else n_features)
+        eps = _EPS32
+    stop_eps = 0.0 if mutant == "no_eps_stop" else eps
+    banned = -1
+    coef = np.zeros(k, dtype=t)
+    prev_coef = np.zeros(k, dtype=t)
+    alpha_cur, alpha_prev = t(0.0), t(0.0)
     active = []                 # ordered like the Cholesky factor
     inact = list(range(k))      # ordered like sklearn's shortened Cov (tie-breaking only)
     L = np.zeros((min(max_iter, k) + 1, min(max_iter, k) + 1))
@@ -130,25 +189,31 @@ def lars_lasso_positive(G, c, reg, n_features, max_iter=1000, return_info=False,
     while True:
         if inact:
             vals = cov[inact]
-            pos = int(np.argmax(vals))
-            C = float(vals[pos])
+            pos = int(np.argmax(vals)) if mutant != "tie_high" else len(vals) - 1 - int(np.argmax(vals[::-1]))
+            if f32 and banned >= 0 and not drop and inact[pos] == banned and len(inact) > 1:
+                others = vals.copy()
+                others[pos] = -np.inf
+                pos = int(np.argmax(others))
+            C = t(vals[pos])
         else:
-            pos, C = -1, 0.0
-        alpha_cur = C / n_features
-        if alpha_cur <= alpha_min + _EPS32:
-            if abs(alpha_cur - alpha_min) > _EPS32 and n_iter > 0:
-                ss = (alpha_prev - alpha_min) / (alpha_prev - alpha_cur)
-                coef = prev_coef + ss * (coef - prev_coef)
+            pos, C = -1, t(0.0)
+        if f32 and not drop:
+            banned = -1
+        alpha_cur = C if f32 else C / n_features
+        if alpha_cur <= alpha_min + (eps if f32 else stop_eps):
+            if abs(alpha_cur - alpha_min) > eps and n_iter > 0 and mutant != "no_interp":
+                ss = t((alpha_prev - alpha_min) / (alpha_prev - alpha_cur))
+                coef = (prev_coef + ss * (coef - prev_coef)).astype(t)
             break
-        if n_iter >= max_iter or len(active) >= k:
+        if n_iter >= max_iter + (mutant == "max_iter_plus1") or len(active) >= k:
             status = 3 if n_iter >= max_iter else status
             break
-        if not drop:
+        if not drop or mutant == "join_after_drop":
             s = len(active)
             inact[pos], inact[0] = inact[0], inact[pos]
             j = inact[0]
-            piv = _chol_append(L, s, G[j, active], G[j, j])
-            if piv < 1e-7:
+            piv = append(L, s, G[j, active], G[j, j])
+            if piv < 1e-7 or (gram32 and not G[j, j] - L[s, :s] @ L[s, :s] > 4 * _EPS32 * G[j, j]):
                 # degenerate regressor: sklearn zeroes its covariance and retries
                 # (_least_angle.py:723-742); it stays inactive.
                 cov[j] = 0.0
@@ -162,16 +227,28 @@ def lars_lasso_positive(G, c, reg, n_features, max_iter=1000, return_info=False,
             status = 2          # "alpha increasing" early stop (_least_angle.py:752-765)
             break
         s = len(active)
-        w = _chol_solve(L, s, np.ones(s))
+        w = solve(L, s, np.ones(s))
         AA = 1.0 / np.sqrt(w.sum())
         w = w * AA
-        corr = G[np.ix_(inact, active)] @ w if inact else np.zeros(0)
-        if round_decimals is not None:
+        if f32:
+            AA, w = t(AA), w.astype(t)
+        corr = Gw[np.ix_(inact, active)] @ w if inact else np.zeros(0, dtype=t)
+        if round_decimals is not None and not f32:
             corr = np.around(corr, decimals=round_decimals)
-        g1 = _min_pos((C - cov[inact]) / (AA - corr + _TINY32)) if inact else np.finfo(np.float64).max
-        gamma = min(g1, C / AA)
-        z = -coef[active] / (w + _TINY32)
-        z_pos = _min_pos(z)
+        if f32:
+            big = t(np.finfo(np.float32).max)
+            den = AA - corr + t(_TINY32)
+            v = np.maximum(C - cov[inact], t(0)) / den
+            g1 = t(v[den > 0].min()) if (den > 0).any() else big
+            g1 = min(g1, big)
+            gamma = min(g1, t(C / AA))
+            z = -coef[active] / (w + t(_TINY32))
+            z_pos = t(min(_min_pos(z), float(big)))
+        else:
+            g1 = _min_pos((C - cov[inact]) / (AA - corr + _TINY32)) if inact else np.finfo(np.float64).max
+            gamma = min(g1, C / AA)
+            z = -coef[active] / (w + _TINY32)
+            z_pos = _min_pos(z)
         drop = False
         drop_pos = []
         if z_pos < gamma:
@@ -181,17 +258,24 @@ def lars_lasso_positive(G, c, reg, n_features, max_iter=1000, return_info=False,
         n_iter += 1
         prev_coef = coef
         alpha_prev = alpha_cur
-        coef = np.zeros(k)
+        coef = np.zeros(k, dtype=t)
         coef[active] = prev_coef[active] + gamma * w
         cov[inact] -= gamma * corr
         if drop:
             n_drops += len(drop_pos)
             for p in drop_pos:
-                _chol_delete(L, len(active), p)
+                delete(L, len(active), p)
                 jd = active.pop(p)
-                # exact covariance of the dropped variable (_least_angle.py:891)
-                cov[jd] = c[jd] - G[jd] @ coef
+                if f32:
+                    coef[jd] = 0
+                    cov[jd] = c[jd] - Gw[jd, active] @ coef[active]
+                    banned = jd
+                else:
+                    # exact covariance of the dropped variable (_least_angle.py:891)
+                    if mutant != "no_drop_recompute":
+                        cov[jd] = c[jd] - G[jd] @ coef
                 inact.insert(0, jd)
+    coef = coef.astype(np.float64)
     if return_info:
         return coef, dict(n_iter=n_iter, max_active=max_active, n_drops=n_drops, status=status)
     return coef
